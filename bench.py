@@ -8,6 +8,7 @@ d=256, codebook K=8192, bf16 latents, Euclidean, EMA decay 0.8; config 2 is "sea
 config 3), so threshold_ema_dead_code=0 there -- stated in the JSON line -- in both arms.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs C3,C4,C5|none]
+                    [--dump-outputs DIR]
 
 N>1 is launched by the driver through torch.distributed.run (one rank per GPU, NCCL): data parallel, every rank
 quantises its own 1M latents ("weak" scaling) and the EMA statistics are summed with one packed all_reduce.
@@ -21,6 +22,8 @@ synthetic latents of each named shape is reported at 1, 2, 4 and 8 GPUs"):
 `--impl reference` times the UNMODIFIED reference (baseline/_ref, installed by baseline/install_ref.sh) on the host
 CPU on a bounded sample of the headline workload, on rank 0 only; if baseline/_ref is missing it falls back to the
 oracle port (oracle/ restates the reference op for op) and says so in `cpu_baseline.kind`.
+`--dump-outputs DIR` writes what the last timed step of the headline computed (rank 0) as .npy files, so that two
+builds can be compared output for output on identical seeded inputs: see dump_outputs().
 Prints ONE JSON line.
 """
 import argparse
@@ -42,6 +45,22 @@ SHAPE = (1024, 1024, DIM)               # (batch, tokens, d) -> N = 2^20 latents
 CPU_SAMPLE_ROWS = 16384                 # bounded sample for the CPU legs (N x K fp32 must fit the host)
 WORKLOAD = "C2: EuclideanCodebook search+EMA, N=1048576 latents x d=256, K=8192, bf16 latents"
 REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+DUMP_QUANTIZE_ROWS = 16384              # --dump-outputs: seeded sample of the 2^20 quantize rows (16 MiB of 1 GiB)
+
+
+def dump_outputs(path, out, cb):
+    """Writes one headline step's results to `path` as .npy: quantize (a fixed seeded sample of its rows, fp32),
+    indices and loss (fp64, exact), and the codebook state the step's EMA update left (embeddings, embed_avg,
+    cluster_size, fp32).  About 40 MB in all."""
+    import numpy as np
+    q, ind, loss = out
+    rows = torch.randperm(N_ROWS, generator=torch.Generator().manual_seed(0))[:DUMP_QUANTIZE_ROWS].sort().values
+    arrays = {"quantize": q.reshape(N_ROWS, DIM)[rows.to(q.device)].float(), "indices": ind.double(),
+              "loss": loss.double(), "embeddings": cb.embeddings.float(), "embed_avg": cb.embed_avg.float(),
+              "cluster_size": cb.cluster_size.float()}
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().cpu().numpy())
 
 
 def ncu_traffic_bytes():
@@ -449,7 +468,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--configs", default="C3,C4,C5", help="other named shapes to time after the headline ('none' to skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed headline step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -488,10 +511,16 @@ def main():
     gx = torch.Generator(device=dev).manual_seed(1234 + rank)
     n_bufs = 2                                                          # 512 MiB each, > 126 MB L2: never L2-hot
     xs = [torch.randn(SHAPE, generator=gx, device=dev, dtype=torch.float32).bfloat16() for _ in range(n_bufs)]
+    keep_last = args.dump_outputs is not None and rank == 0
+    last = []                             # --dump-outputs: the outputs of the latest step
 
     def step(i):
+        last.clear()                      # the previous outputs are freed before the next step, as without the flag
         with torch.no_grad():
-            return vq(xs[i % n_bufs])
+            out = vq(xs[i % n_bufs])
+        if keep_last:
+            last.append(out)
+        return out
 
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -503,6 +532,9 @@ def main():
     t_end = time.time()
     clocks = sampler.stop(t_warm, t_end) if rank == 0 else None
     stats = ops.search_stats(cb.last_search_ws)
+    if keep_last:
+        dump_outputs(args.dump_outputs, last[0], cb)
+        last.clear()
 
     # ---- the bandwidth-bound part of the step on its own: gather + straight-through + loss + EMA sums in one pass over
     #      the latents (counting sort included), against its ALGORITHMIC bytes (DESIGN 4.2: sz(x) d + 12 read,

@@ -18,14 +18,14 @@ def _cpu_draw(num_rows, m, device):
 @pytest.fixture()
 def cpu_ops(monkeypatch):
     from vqb200 import _lib, codebook, ops
-    saved = {n: getattr(ops, n) for n in cpu_kernels.REPLACED}
-    saved_guard = _lib.require_device
+    # the real entry points are recorded with the test's own monkeypatch before anything replaces them, so they are
+    # what is restored last: a test that patches one of them again (tests/f4_util.py) cannot leave a plain-torch
+    # statement in place of a kernel for the tests that follow
+    for n in cpu_kernels.REPLACED:
+        monkeypatch.setattr(ops, n, getattr(ops, n))
+    monkeypatch.setattr(_lib, "require_device", _lib.require_device)
     cpu_kernels.install(ops, _lib)
     monkeypatch.setattr(codebook.Codebook, "_draw_rows", staticmethod(_cpu_draw))
-    yield
-    for n, f in saved.items():
-        setattr(ops, n, f)
-    _lib.require_device = saved_guard
 
 
 @pytest.fixture()
