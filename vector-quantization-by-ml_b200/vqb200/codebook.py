@@ -164,7 +164,9 @@ class Codebook(nn.Module):
         return self._cache
 
     def invalidate_cache(self) -> None:
-        self._dirty = True
+        """Call after an in-place edit of `embeddings`: the search operands and, on a sharded codebook, the all-gathered
+        replica the gather reads are rebuilt on next use."""
+        self._dirty = self._replica_dirty = True
 
     # ------------------------------------------------------------------ helpers
     def _all_reduce(self, t: torch.Tensor) -> None:

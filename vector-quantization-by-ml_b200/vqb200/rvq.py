@@ -51,7 +51,9 @@ class ResidualVQ(nn.Module):
 
     @property
     def codebooks(self):
-        return torch.stack([layer._codebook.embeddings[0] for layer in self.layers], dim=0)
+        # full (K,d) codebooks: a sharded codebook is all-gathered (a collective when a shard changed since the last call)
+        return torch.stack([layer._codebook.full_codebook()[0] if layer._codebook.sharded
+                            else layer._codebook.embeddings[0] for layer in self.layers], dim=0)
 
     def get_codes_from_indices(self, indices):
         q_dim = indices.shape[-1]
@@ -75,6 +77,8 @@ class ResidualVQ(nn.Module):
     def _can_fuse(self, x, dropout_active) -> bool:
         if not self.use_fused_levels or dropout_active or not x.is_cuda or x.ndim != 3:
             return False
+        if any(l._codebook.sharded for l in self.layers):
+            return False        # the level kernels search and update one whole codebook; shards need `_run_sharded`
         if torch.is_grad_enabled() and x.requires_grad and not self._can_fuse_autograd(x):
             return False
         l0 = self.layers[0]

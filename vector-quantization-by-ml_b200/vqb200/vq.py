@@ -96,18 +96,24 @@ class VectorQuantize(nn.Module):
         self.register_buffer("zero", torch.tensor(0.0), persistent=False)
 
     # reference :140-176 reads `_codebook.embed`, which does not exist there; implemented on `embeddings`
+    # A sharded codebook (Codebook.sharded) reads and writes the full (K, d) codebook here: the getter all-gathers the
+    # shards (a collective every rank must join when a shard changed since the last call), the setter keeps this
+    # rank's rows of what it is given.
     @property
     def codebook(self):
-        cb = self._codebook.embeddings
+        cb = self._codebook.full_codebook() if self._codebook.sharded else self._codebook.embeddings
         return cb if self.separate_codebook_per_head else cb[0]
 
     @codebook.setter
     def codebook(self, codes):
         if not self.separate_codebook_per_head:
             codes = codes[None]
+        cb = self._codebook
+        if cb.sharded:
+            codes = codes[:, cb.shard_offset:cb.shard_offset + cb.shard_size]
         with torch.no_grad():
-            self._codebook.embeddings.copy_(codes)
-        self._codebook.invalidate_cache()
+            cb.embeddings.copy_(codes)
+        cb.invalidate_cache()
 
     def get_codes_from_indices(self, indices):
         cb = self.codebook
