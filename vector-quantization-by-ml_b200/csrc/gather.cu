@@ -244,10 +244,8 @@ rvq_level_kernel(const float* res_in, float* res_out, const float* __restrict__ 
 #pragma unroll
     for (int t = 0; t < 4; ++t) keep[t] = make_float4(0.f, 0.f, 0.f, 0.f);
     if (vec) {
-#pragma unroll
-      for (int t = 0; t < 16; ++t) {
-        const int j = lane * 4 + 128 * t;
-        if (j >= d) break;
+      // one float4 group of columns j..j+3; returns the new residual
+      auto step = [&](int j) {
         const float4 r = *reinterpret_cast<const float4*>(rr + j);
         const float4 c = __ldg(reinterpret_cast<const float4*>(cr + j));
         const float4 df = make_float4(__fsub_rn(c.x, r.x), __fsub_rn(c.y, r.y), __fsub_rn(c.z, r.z), __fsub_rn(c.w, r.w));
@@ -269,9 +267,18 @@ rvq_level_kernel(const float* res_in, float* res_out, const float* __restrict__ 
         *reinterpret_cast<float4*>(ro + j) = rn;
         if (qout) *reinterpret_cast<float4*>(qout + row * (int64_t)d + j) = qv;
         sq = fmaf(df.x, df.x, sq); sq = fmaf(df.y, df.y, sq); sq = fmaf(df.z, df.z, sq); sq = fmaf(df.w, df.w, sq);
-        if (t < 4) keep[t] = rn;
         m = fmaxf(fmaxf(fmaxf(m, fabsf(rn.x)), fmaxf(fabsf(rn.y), fabsf(rn.z))), fabsf(rn.w));
+        return rn;
+      };
+#pragma unroll
+      for (int t = 0; t < 16; ++t) {
+        const int j = lane * 4 + 128 * t;
+        if (j >= d) break;
+        const float4 rn = step(j);
+        if (t < 4) keep[t] = rn;
       }
+#pragma unroll 1
+      for (int j = lane * 4 + 2048; j < d; j += 128) step(j);   // rows wider than 2048 (no next operand there)
     } else {
       for (int j = lane; j < d; j += 32) {
         const float r = rr[j], c = cr[j];

@@ -132,6 +132,12 @@ def aligned(t: torch.Tensor) -> torch.Tensor:
     return t
 
 
+def require_aligned(t, name: str) -> None:
+    """A buffer the kernels write in place cannot be swapped for an aligned copy: it must be 16-byte aligned already."""
+    if t is not None and t.data_ptr() % 16:
+        raise ValueError(f"vqb200: `{name}` must be 16-byte aligned (the kernels use 128-bit stores)")
+
+
 def ptr(t) -> int:
     return 0 if t is None else t.data_ptr()
 

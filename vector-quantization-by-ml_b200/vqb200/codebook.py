@@ -419,8 +419,8 @@ class Codebook(nn.Module):
         replica = self.full_codebook()
         training = self.training
         update = training and self.ema_update and not freeze_codebook
-        if update and torch.is_grad_enabled() and flat.requires_grad:
-            replica = replica.clone()          # backward reads the PRE-update codes (see _run)
+        if torch.is_grad_enabled() and flat.requires_grad:
+            replica = replica.clone()          # backward reads the codes of this forward (see _run)
         lo_r = self.shard_rank * n_local if gathered else 0
         gidx = gidx_all[:, lo_r:lo_r + n_local] if gathered else gidx_all
         commit = None
@@ -579,8 +579,8 @@ class Codebook(nn.Module):
         else:
             emb_eff = base
         emb_val = emb_eff.detach().contiguous()
-        if update and emb_val.data_ptr() == self.embeddings.data_ptr() and (keep_dense or (grad_on and flat.requires_grad)):
-            emb_val = emb_val.clone()          # backward reads the PRE-update codes (see _run)
+        if emb_val.data_ptr() == self.embeddings.data_ptr() and (keep_dense or (grad_on and flat.requires_grad)):
+            emb_val = emb_val.clone()          # backward reads the codes of this forward (see _run)
         if keep_dense:
             self.dense_ctx = ops._DenseCtx(flat, emb_val, emb_val if self.use_affine else self.embeddings,
                                            self.use_cosine_sim)
@@ -678,9 +678,10 @@ class Codebook(nn.Module):
 
         emb = self.embeddings.detach()
         update = self.training and self.ema_update and not freeze_codebook
-        if update and (keep_dense or (torch.is_grad_enabled() and flat.requires_grad)):
-            # this forward's EMA step overwrites `embeddings` in place before backward runs; the reference's
-            # commitment loss holds the gathered PRE-update codes (vector_quantize_pytorch.py:262-268, a tensor
+        if keep_dense or (torch.is_grad_enabled() and flat.requires_grad):
+            # the EMA step of this forward, or of a later training forward before backward runs (gradient
+            # accumulation; this one may be frozen), overwrites `embeddings` in place; the reference's commitment
+            # loss holds the gathered codes of THIS forward (vector_quantize_pytorch.py:262-268, a tensor
             # materialised at codebooks.py:395 before :425), so everything saved for backward reads a snapshot
             emb = emb.clone()
         if keep_dense:

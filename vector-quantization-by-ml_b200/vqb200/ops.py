@@ -391,11 +391,14 @@ def rvq_level(residual: torch.Tensor, residual_next: torch.Tensor, embeddings: t
               next_cache: Optional[torch.Tensor], q_out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Reads `residual` (N,d fp32), writes `residual_next` and updates `quantized_out` in place;
     returns loss_buf [mean sq err, rows used].  `next_cache`: codebook cache of the level that searches
-    `residual_next` next (its operands are prepared in the same pass), or None."""
+    `residual_next` next (its operands are prepared in the same pass; same number of codes as `embeddings`), or None."""
     prepare_next = next_cache is not None
     L.require_cuda(residual, "residual")
     L.require_cuda(residual_next, "residual_next")
     assert residual.dtype == torch.float32 and residual.ndim == 2 and residual_next.shape == residual.shape
+    residual, embeddings = L.aligned(residual), L.aligned(embeddings)
+    for t, n in ((residual_next, "residual_next"), (quantized_out, "quantized_out"), (q_out, "q_out")):
+        L.require_aligned(t, n)
     N, d = residual.shape
     K = embeddings.shape[-2]
     dev = residual.device
@@ -421,14 +424,16 @@ def rvq_replay_out(x: torch.Tensor, codebooks, idxs, training, mask_u8: Optional
     import ctypes as C
     L.require_cuda(x, "x")
     assert x.dtype == torch.float32 and x.ndim == 2
+    x = L.aligned(x)
     N, d = x.shape
     Q = len(codebooks)
-    keep = [c.contiguous() for c in codebooks] + [i.contiguous() for i in idxs]
+    keep = [L.aligned(c) for c in codebooks] + [i.contiguous() for i in idxs]
     cbp = (C.c_void_p * Q)(*[L.ptr(c) for c in keep[:Q]])
     ixp = (C.c_void_p * Q)(*[L.ptr(i) for i in keep[Q:]])
     trp = (C.c_int * Q)(*[int(bool(t)) for t in training])
     if out is None:
         out = torch.empty((N, d), dtype=torch.float32, device=x.device)
+    L.require_aligned(out, "out")
     L.check(L.lib().vqb_rvq_replay_out(L.ptr(x), C.cast(cbp, C.c_void_p), C.cast(ixp, C.c_void_p),
                                        C.cast(trp, C.c_void_p), Q, L.ptr(mask_u8), L.ptr(out), N, d,
                                        L.stream_ptr(x.device)), "vqb_rvq_replay_out")
@@ -442,14 +447,17 @@ def rvq_backward(x: torch.Tensor, codebooks, idxs, training, coef: torch.Tensor,
     rows with mask != 0 (vqb_rvq_backward); the residuals are replayed from x and the indices."""
     import ctypes as C
     L.require_cuda(x, "x")
+    x = L.aligned(x)
     N, d = x.shape
     Q = len(codebooks)
-    keep = [c.contiguous() for c in codebooks] + [i.contiguous() for i in idxs]
+    keep = [L.aligned(c) for c in codebooks] + [i.contiguous() for i in idxs]
     cbp = (C.c_void_p * Q)(*[L.ptr(c) for c in keep[:Q]])
     ixp = (C.c_void_p * Q)(*[L.ptr(i) for i in keep[Q:]])
     trp = (C.c_int * Q)(*[int(bool(t)) for t in training])
     coef = coef.to(device=x.device, dtype=torch.float32).contiguous()
-    g = g_out.contiguous().float() if g_out is not None else None
+    # a contiguous fp32 gradient can still start at any element (a view into a larger buffer): the kernel reads it
+    # with 128-bit loads
+    g = L.aligned(g_out.float()) if g_out is not None else None
     gx = torch.empty((N, d), dtype=torch.float32, device=x.device)
     L.check(L.lib().vqb_rvq_backward(L.ptr(x), C.cast(cbp, C.c_void_p), C.cast(ixp, C.c_void_p),
                                      C.cast(trp, C.c_void_p), Q, L.ptr(coef), L.ptr(g), L.ptr(mask_u8), L.ptr(gx), N, d,
@@ -469,6 +477,9 @@ def rvq_level_ema(residual: torch.Tensor, residual_next: torch.Tensor, embedding
     L.require_cuda(residual, "residual")
     L.require_cuda(residual_next, "residual_next")
     assert residual.dtype == torch.float32 and residual.ndim == 2 and residual_next.shape == residual.shape
+    residual, embeddings = L.aligned(residual), L.aligned(embeddings)
+    for t, n in ((residual_next, "residual_next"), (quantized_out, "quantized_out"), (q_out, "q_out")):
+        L.require_aligned(t, n)
     N, d = residual.shape
     K = embeddings.shape[-2]
     dev = residual.device

@@ -114,8 +114,10 @@ class ResidualVQ(nn.Module):
         return out, all_idx, all_loss
 
     @torch.no_grad()
-    def _fused_levels(self, x, mask, freeze_codebook):
-        """Everything of the fused level loop that needs no host round trip (capturable in a CUDA graph)."""
+    def _fused_levels(self, x, mask, freeze_codebook, for_backward=False):
+        """Everything of the fused level loop that needs no host round trip (capturable in a CUDA graph).
+        `for_backward`: the codebooks each level gathered from are kept as copies for `_FusedRVQ.backward`, which may
+        run after they moved (a later training forward of the same module refreshes them in place)."""
         B, n, d = x.shape
         N = B * n
         dev = x.device
@@ -155,7 +157,7 @@ class ResidualVQ(nn.Module):
             training = self.training and layer.training
             do_ema = training and cb.ema_update and not freeze_codebook
             if defer or replay:   # the codebook the gather uses (the EMA refresh below overwrites it in place)
-                pre_emb.append((emb.clone() if do_ema else emb, training))
+                pre_emb.append((emb.clone() if do_ema or for_backward else emb, training))
             # the next level's operands are prepared in the same pass when its codebook cache is already final:
             # a different codebook object (not shared) that is initialised
             next_cache = None
@@ -350,7 +352,7 @@ class _FusedRVQ(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, rvq, mask, freeze_codebook):
         with torch.no_grad():
-            out, all_idx, all_loss, late = rvq._fused_levels(x.detach(), mask, freeze_codebook)
+            out, all_idx, all_loss, late = rvq._fused_levels(x.detach(), mask, freeze_codebook, for_backward=True)
             rvq._fused_expiry(late, mask)
         _, _, x0, pre_emb, _, loss_bufs = late
         ctx.x0, ctx.pre_emb, ctx.loss_bufs = x0, pre_emb, loss_bufs
