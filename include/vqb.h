@@ -122,6 +122,16 @@ int    vqb_st_commit_backward(const float* grad_q, const float* grad_loss, const
                               const float* codebook, const int64_t* idx, const uint8_t* mask,
                               float coef, float* grad_x,
                               int64_t H, int64_t N, int K, int d, void* stream);
+/* Same, with the rotation-trick gradient (Fifty et al., arXiv:2410.06424; upstream VectorQuantize(rotation_trick=True))
+ * in place of the straight-through one.  Per row with mask != 0, c = C[idx], sx = max(|x|, 1e-6), sc = max(|c|, 1e-6),
+ * u = x / sx, q = c / sc, w = (u + q) / max(|u + q|, 1e-12) and lambda = |c| / sx:
+ *   grad_x = lambda (g - 2 (g.w) w + 2 (g.q) u) + coef * grad_loss[0] * (x - c),   g = grad_q;
+ * rows with mask == 0 get grad_q.  |u + q| is summed elementwise, |x|^2 and |c|^2 in fp64; one warp per row, no atomics
+ * (bitwise repeatable).  Any d, any H, x fp32 / bf16 / fp16, as vqb_st_commit_backward. */
+int    vqb_rot_commit_backward(const float* grad_q, const float* grad_loss, const void* x, int x_dtype,
+                               const float* codebook, const int64_t* idx, const uint8_t* mask,
+                               float coef, float* grad_x,
+                               int64_t H, int64_t N, int K, int d, void* stream);
 
 /* ---- EMA statistics: deterministic sort-and-segment reduction -------------------------
  * Replaces codebooks.py:405-408 (masked one-hot column sums) and :413 (x^T . onehot SGEMM).
@@ -240,6 +250,13 @@ int    vqb_column_moments(const void* x, int x_dtype, const uint8_t* mask, int64
 int    vqb_rvq_backward(const float* x, const float* const* codebooks, const int64_t* const* idx, const int* training,
                         int num_levels, const float* coef, const float* g_out, const uint8_t* mask, float* grad_x,
                         int64_t N, int d, void* stream);
+/* vqb_rvq_backward for levels that use the rotation-trick gradient (see vqb_rot_commit_backward): each level's
+ * output gradient is transported by T_l, the rotation Jacobian on (r_l, c_l), instead of passed through:
+ *   grad_x = sum_l T_l(g_out) + sum_l [mask != 0] coef[l] * (r_l - c_l),   T_l = identity on rows with mask == 0.
+ * Same arguments and limits as vqb_rvq_backward (d % 4 == 0, d <= 512, num_levels <= 32). */
+int    vqb_rvq_backward_rot(const float* x, const float* const* codebooks, const int64_t* const* idx,
+                            const int* training, int num_levels, const float* coef, const float* g_out,
+                            const uint8_t* mask, float* grad_x, int64_t N, int d, void* stream);
 
 /* ---- sharded-codebook merge (K >= 64K split across GPUs) ------------------------------
  * No reference counterpart (SURVEY 3.4).  key = (orderable(score) << 32) | index, so an

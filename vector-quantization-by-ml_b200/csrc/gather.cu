@@ -194,8 +194,56 @@ __global__ void loss_finalize_kernel(const double* __restrict__ part, const long
   }
 }
 
+// Rotation-trick transport of one row (Fifty et al., arXiv:2410.06424; upstream vector-quantize-pytorch `rotate_to`):
+// with sx = max(|x|, 1e-6), sc = max(|c|, 1e-6), u = x / sx, q = c / sc, w = (u + q) / max(|u + q|, 1e-12) and
+// lambda = |c| / sx, the gradient g of the rotated output becomes
+//   T(g) = lambda (g - 2 (g.w) w + 2 (g.q) u) = lambda g - 2 lambda (g.w) / nw (u + q) + 2 lambda (g.q) u.
+// The squared norms are accumulated in fp64: at |x_i| ~ 1e-20 the fp32 squares are below the normal range and lambda
+// would lose digits.  |u + q| is summed from the elementwise sums (not expanded: that cancels on antiparallel rows).
+struct RotCoef {
+  float sx, sc;     // max(|x|, 1e-6), max(|c|, 1e-6)
+  float rx, rc;     // RN(1 / sx), RN(1 / sc)
+  float lam;        // lambda
+  float a;          // coefficient of (u + q): -2 lambda (g.w) / nw
+  float b;          // coefficient of u: 2 lambda (g.q)
+};
+// nx2 = |x|^2, nc2 = |c|^2 (fp64)
+__device__ __forceinline__ RotCoef rot_scales(double nx2, double nc2) {
+  const double nc = sqrt(nc2), sx = fmax(sqrt(nx2), 1e-6);
+  RotCoef r;
+  r.sx = (float)sx;
+  r.sc = (float)fmax(nc, 1e-6);
+  r.rx = __frcp_rn(r.sx);
+  r.rc = __frcp_rn(r.sc);
+  r.lam = (float)(nc / sx);
+  r.a = r.b = 0.f;
+  return r;
+}
+// v / s from r = RN(1/s) and one fma correction: the correctly rounded quotient (Markstein) for the normal-range
+// operands met here, without the slow-path call of a general division
+__device__ __forceinline__ float rot_div(float v, float s, float r) {
+  const float q0 = __fmul_rn(v, r);
+  return fmaf(fmaf(-q0, s, v), r, q0);
+}
+// u and q are correctly rounded quotients and u + q is formed without contraction, so a pair that is exactly
+// antiparallel after normalisation (c = -2x, or opposite signs at d = 1) sums to 0 as it does in exact arithmetic, and
+// w = 0 there, as F.normalize returns; the (u + q) term then vanishes whatever g.w rounds to.
+// gx = g.x, gc = g.c, nw2 = |u + q|^2
+__device__ __forceinline__ void rot_finish(RotCoef& r, float gx, float gc, float nw2) {
+  const float nw = fmaxf(sqrtf(nw2), 1e-12f), rnw = __frcp_rn(nw);
+  const float gq = rot_div(gc, r.sc, r.rc);
+  const float gw = rot_div(__fadd_rn(rot_div(gx, r.sx, r.rx), gq), nw, rnw);
+  r.a = nw2 > 0.f ? -2.f * r.lam * rot_div(gw, nw, rnw) : 0.f;
+  r.b = 2.f * r.lam * gq;
+}
+__device__ __forceinline__ float rot_u(float xv, const RotCoef& r) { return rot_div(xv, r.sx, r.rx); }
+__device__ __forceinline__ float rot_sum(float xv, float cv, const RotCoef& r) {
+  return __fadd_rn(rot_div(xv, r.sx, r.rx), rot_div(cv, r.sc, r.rc));
+}
+
 // grad_x = grad_q + coef * grad_loss[0] * (x - c)   (rows with mask==0: grad_q only)
-template <typename T>
+// kRot: grad_x = T(grad_q) + coef * grad_loss[0] * (x - c) on the rows with mask != 0 (T above), grad_q on the others.
+template <typename T, bool kRot>
 __global__ void __launch_bounds__(kGatherThreads)
 st_commit_backward_kernel(const float* __restrict__ gq, const float* __restrict__ gl, const T* __restrict__ x,
                           const float* __restrict__ cb, const int64_t* __restrict__ idx,
@@ -213,7 +261,32 @@ st_commit_backward_kernel(const float* __restrict__ gq, const float* __restrict_
     const float* cr = cb + (h * K + idx[row]) * (int64_t)d;
     const float* gr = gq + row * (int64_t)d;
     float* o = gx + row * (int64_t)d;
-    for (int j = lane; j < d; j += 32) o[j] = fmaf(sc, to_f32<T>(xr[j]) - cr[j], gr[j]);
+    if (!kRot || !in_loss) {
+      for (int j = lane; j < d; j += 32) o[j] = fmaf(sc, to_f32<T>(xr[j]) - cr[j], gr[j]);
+      continue;
+    }
+    // pass 1: |x|^2, |c|^2 (fp64), g.x, g.c -- lane-strided partials, then a fixed butterfly over the warp
+    double nx2 = 0.0, nc2 = 0.0;
+    float gdx = 0.f, gdc = 0.f;
+    for (int j = lane; j < d; j += 32) {
+      const float xv = to_f32<T>(xr[j]), cv = cr[j], g = gr[j];
+      nx2 = fma((double)xv, (double)xv, nx2);
+      nc2 = fma((double)cv, (double)cv, nc2);
+      gdx = fmaf(g, xv, gdx);
+      gdc = fmaf(g, cv, gdc);
+    }
+    RotCoef rc = rot_scales(warp_sum(nx2), warp_sum(nc2));
+    // pass 2: |u + q|^2 from the elementwise sums (the row is in L1 now)
+    float nw2 = 0.f;
+    for (int j = lane; j < d; j += 32) {
+      const float e = rot_sum(to_f32<T>(xr[j]), cr[j], rc);
+      nw2 = fmaf(e, e, nw2);
+    }
+    rot_finish(rc, warp_sum(gdx), warp_sum(gdc), warp_sum(nw2));
+    for (int j = lane; j < d; j += 32) {
+      const float xv = to_f32<T>(xr[j]), cv = cr[j];
+      o[j] = fmaf(sc, xv - cv, fmaf(rc.b, rot_u(xv, rc), fmaf(rc.a, rot_sum(xv, cv, rc), rc.lam * gr[j])));
+    }
   }
 }
 
@@ -455,11 +528,23 @@ rvq_replay_out_kernel(const float* __restrict__ x, const uint8_t* __restrict__ m
 // next residual subtracts a DETACHED quantity (identity again), so d out / d x = Q I, and the commitment loss of level
 // l, mean((c_l - r_l)^2) over the live rows, contributes coef_l (r_l - c_l) with coef_l = g_loss_l w_l 2 / (rows_l d):
 //   grad_x = Q g_out + sum_l live coef_l (r_l - c_l)        (c_l from the codebook as it was BEFORE level l's EMA step)
+// kRot (rotation trick): each level's output is the rotation of r_l onto c_l instead, whose Jacobian is the transport
+// T_l of st_commit_backward_kernel evaluated on (r_l, c_l) -- the identity on masked rows:
+//   grad_x = sum_l T_l(g_out) + sum_l live coef_l (r_l - c_l)
 struct BackwardArgs {
   ReplayArgs R;
   const float* coef;       // (Q) device
 };
-template <int VEC>
+// r_{l+1} = fl(r_l - q_l) with q_l of vqb_rvq_level
+__device__ __forceinline__ float4 rvq_next_residual(float4 v, float4 c, bool live, bool tr) {
+  float4 qv;
+  if (!live) qv = v;
+  else if (tr) qv = make_float4(__fadd_rn(v.x, __fsub_rn(c.x, v.x)), __fadd_rn(v.y, __fsub_rn(c.y, v.y)),
+                                __fadd_rn(v.z, __fsub_rn(c.z, v.z)), __fadd_rn(v.w, __fsub_rn(c.w, v.w)));
+  else qv = c;
+  return make_float4(__fsub_rn(v.x, qv.x), __fsub_rn(v.y, qv.y), __fsub_rn(v.z, qv.z), __fsub_rn(v.w, qv.w));
+}
+template <int VEC, bool kRot>
 __global__ void __launch_bounds__(kGatherThreads)
 rvq_backward_kernel(const float* __restrict__ x, const float* __restrict__ g_out, const uint8_t* __restrict__ mask,
                     float* __restrict__ grad_x, int64_t N, int d, const __grid_constant__ BackwardArgs B) {
@@ -469,17 +554,22 @@ rvq_backward_kernel(const float* __restrict__ x, const float* __restrict__ g_out
   const float my_coef = lane < A.Q ? B.coef[lane] : 0.f;
   for (int64_t row = (int64_t)blockIdx.x * wpb + warp; row < N; row += (int64_t)gridDim.x * wpb) {
     const bool live = mask == nullptr || mask[row] != 0;
-    float4 r[VEC], acc[VEC];
+    float4 r[VEC], acc[VEC], g[kRot ? VEC : 1];
 #pragma unroll
     for (int t = 0; t < VEC; ++t) {
       const int j = lane * 4 + 128 * t;
       r[t] = acc[t] = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (kRot) g[t] = r[t];
       if (j < d) {
         r[t] = __ldcs(reinterpret_cast<const float4*>(x + row * (int64_t)d + j));
-        const float4 g = g_out ? __ldcs(reinterpret_cast<const float4*>(g_out + row * (int64_t)d + j))
-                               : make_float4(0.f, 0.f, 0.f, 0.f);
-        const float q = (float)A.Q;
-        acc[t] = make_float4(q * g.x, q * g.y, q * g.z, q * g.w);
+        const float4 gv = g_out ? __ldcs(reinterpret_cast<const float4*>(g_out + row * (int64_t)d + j))
+                                : make_float4(0.f, 0.f, 0.f, 0.f);
+        if (kRot) {
+          g[t] = gv;
+        } else {
+          const float q = (float)A.Q;
+          acc[t] = make_float4(q * gv.x, q * gv.y, q * gv.z, q * gv.w);
+        }
       }
     }
     const long long my_k = lane < A.Q ? (long long)A.idx[lane][row] : 0ll;
@@ -487,20 +577,71 @@ rvq_backward_kernel(const float* __restrict__ x, const float* __restrict__ g_out
       const float* cr = A.cb[l] + __shfl_sync(0xffffffffu, my_k, l) * (int64_t)d;
       const float cf = live ? __shfl_sync(0xffffffffu, my_coef, l) : 0.f;
       const bool tr = A.training[l] != 0;
+      if constexpr (kRot) {
+        // level l's output is rotated r_l -> c_l: acc += T_l(g_out) (identity on masked rows, whose level returns r_l);
+        // five warp reductions on the row held in registers (|r|^2, |c|^2 in fp64, g.r, g.c, then |u + q|^2)
+        float4 c[VEC];
 #pragma unroll
-      for (int t = 0; t < VEC; ++t) {
-        const int j = lane * 4 + 128 * t;
-        if (j >= d) continue;
-        const float4 c = __ldg(reinterpret_cast<const float4*>(cr + j));
-        const float4 v = r[t];
-        acc[t].x = fmaf(cf, v.x - c.x, acc[t].x); acc[t].y = fmaf(cf, v.y - c.y, acc[t].y);
-        acc[t].z = fmaf(cf, v.z - c.z, acc[t].z); acc[t].w = fmaf(cf, v.w - c.w, acc[t].w);
-        float4 qv;
-        if (!live) qv = v;
-        else if (tr) qv = make_float4(__fadd_rn(v.x, __fsub_rn(c.x, v.x)), __fadd_rn(v.y, __fsub_rn(c.y, v.y)),
-                                      __fadd_rn(v.z, __fsub_rn(c.z, v.z)), __fadd_rn(v.w, __fsub_rn(c.w, v.w)));
-        else qv = c;
-        r[t] = make_float4(__fsub_rn(v.x, qv.x), __fsub_rn(v.y, qv.y), __fsub_rn(v.z, qv.z), __fsub_rn(v.w, qv.w));
+        for (int t = 0; t < VEC; ++t) {
+          const int j = lane * 4 + 128 * t;
+          c[t] = j < d ? __ldg(reinterpret_cast<const float4*>(cr + j)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+        if (live) {
+          double nx2 = 0.0, nc2 = 0.0;
+          float gdx = 0.f, gdc = 0.f;
+#pragma unroll
+          for (int t = 0; t < VEC; ++t) {
+            const float4 v = r[t], cv = c[t], gv = g[t];
+            nx2 = fma((double)v.x, (double)v.x, nx2); nx2 = fma((double)v.y, (double)v.y, nx2);
+            nx2 = fma((double)v.z, (double)v.z, nx2); nx2 = fma((double)v.w, (double)v.w, nx2);
+            nc2 = fma((double)cv.x, (double)cv.x, nc2); nc2 = fma((double)cv.y, (double)cv.y, nc2);
+            nc2 = fma((double)cv.z, (double)cv.z, nc2); nc2 = fma((double)cv.w, (double)cv.w, nc2);
+            gdx = fmaf(gv.x, v.x, gdx); gdx = fmaf(gv.y, v.y, gdx); gdx = fmaf(gv.z, v.z, gdx); gdx = fmaf(gv.w, v.w, gdx);
+            gdc = fmaf(gv.x, cv.x, gdc); gdc = fmaf(gv.y, cv.y, gdc); gdc = fmaf(gv.z, cv.z, gdc); gdc = fmaf(gv.w, cv.w, gdc);
+          }
+          RotCoef rc = rot_scales(warp_sum(nx2), warp_sum(nc2));
+          float nw2 = 0.f;
+#pragma unroll
+          for (int t = 0; t < VEC; ++t) {
+            const float4 v = r[t], cv = c[t];    // zero beyond d: contributes 0
+            const float e0 = rot_sum(v.x, cv.x, rc), e1 = rot_sum(v.y, cv.y, rc);
+            const float e2 = rot_sum(v.z, cv.z, rc), e3 = rot_sum(v.w, cv.w, rc);
+            nw2 = fmaf(e0, e0, nw2); nw2 = fmaf(e1, e1, nw2); nw2 = fmaf(e2, e2, nw2); nw2 = fmaf(e3, e3, nw2);
+          }
+          rot_finish(rc, warp_sum(gdx), warp_sum(gdc), warp_sum(nw2));
+#pragma unroll
+          for (int t = 0; t < VEC; ++t) {
+            const float4 v = r[t], cv = c[t], gv = g[t];
+            auto tr1 = [&](float xv, float cc, float gg) {
+              return fmaf(rc.b, rot_u(xv, rc), fmaf(rc.a, rot_sum(xv, cc, rc), rc.lam * gg));
+            };
+            acc[t].x += tr1(v.x, cv.x, gv.x); acc[t].y += tr1(v.y, cv.y, gv.y);
+            acc[t].z += tr1(v.z, cv.z, gv.z); acc[t].w += tr1(v.w, cv.w, gv.w);
+          }
+        } else {
+#pragma unroll
+          for (int t = 0; t < VEC; ++t) {
+            acc[t].x += g[t].x; acc[t].y += g[t].y; acc[t].z += g[t].z; acc[t].w += g[t].w;
+          }
+        }
+#pragma unroll
+        for (int t = 0; t < VEC; ++t) {
+          const float4 v = r[t];
+          acc[t].x = fmaf(cf, v.x - c[t].x, acc[t].x); acc[t].y = fmaf(cf, v.y - c[t].y, acc[t].y);
+          acc[t].z = fmaf(cf, v.z - c[t].z, acc[t].z); acc[t].w = fmaf(cf, v.w - c[t].w, acc[t].w);
+          r[t] = rvq_next_residual(v, c[t], live, tr);
+        }
+      } else {
+#pragma unroll
+        for (int t = 0; t < VEC; ++t) {
+          const int j = lane * 4 + 128 * t;
+          if (j >= d) continue;
+          const float4 c = __ldg(reinterpret_cast<const float4*>(cr + j));
+          const float4 v = r[t];
+          acc[t].x = fmaf(cf, v.x - c.x, acc[t].x); acc[t].y = fmaf(cf, v.y - c.y, acc[t].y);
+          acc[t].z = fmaf(cf, v.z - c.z, acc[t].z); acc[t].w = fmaf(cf, v.w - c.w, acc[t].w);
+          r[t] = rvq_next_residual(v, c, live, tr);
+        }
       }
     }
 #pragma unroll
@@ -574,7 +715,21 @@ extern "C" int vqb_st_commit_backward(const float* grad_q, const float* grad_los
   if (H * N == 0) return VQB_OK;
   const int grid = gather_grid(H * N);
   VQB_DISPATCH_DTYPE(x_dtype, T,
-    st_commit_backward_kernel<T><<<grid, kGatherThreads, 0, (cudaStream_t)stream>>>(
+    st_commit_backward_kernel<T, false><<<grid, kGatherThreads, 0, (cudaStream_t)stream>>>(
+        grad_q, grad_loss, (const T*)x, codebook, idx, mask, coef, grad_x, H, N, K, d));
+  VQB_LAUNCH_CHECK();
+  return VQB_OK;
+}
+
+extern "C" int vqb_rot_commit_backward(const float* grad_q, const float* grad_loss, const void* x, int x_dtype,
+                                       const float* codebook, const int64_t* idx, const uint8_t* mask, float coef,
+                                       float* grad_x, int64_t H, int64_t N, int K, int d, void* stream) {
+  VQB_REQUIRE(grad_q && grad_loss && x && codebook && idx && grad_x, VQB_ERR_INVALID,
+              "vqb_rot_commit_backward: null pointer");
+  if (H * N == 0) return VQB_OK;
+  const int grid = gather_grid(H * N);
+  VQB_DISPATCH_DTYPE(x_dtype, T,
+    st_commit_backward_kernel<T, true><<<grid, kGatherThreads, 0, (cudaStream_t)stream>>>(
         grad_q, grad_loss, (const T*)x, codebook, idx, mask, coef, grad_x, H, N, K, d));
   VQB_LAUNCH_CHECK();
   return VQB_OK;
@@ -651,25 +806,45 @@ extern "C" int vqb_rvq_replay_out(const float* x, const float* const* codebooks,
   return VQB_OK;
 }
 
-extern "C" int vqb_rvq_backward(const float* x, const float* const* codebooks, const int64_t* const* idx,
-                                const int* training, int num_levels, const float* coef, const float* g_out,
-                                const uint8_t* mask, float* grad_x, int64_t N, int d, void* stream) {
-  VQB_REQUIRE(x && codebooks && idx && training && coef && grad_x, VQB_ERR_INVALID, "vqb_rvq_backward: null pointer");
+static int rvq_backward_launch(const char* what, bool rot, const float* x, const float* const* codebooks,
+                               const int64_t* const* idx, const int* training, int num_levels, const float* coef,
+                               const float* g_out, const uint8_t* mask, float* grad_x, int64_t N, int d, void* stream) {
+  VQB_REQUIRE(x && codebooks && idx && training && coef && grad_x, VQB_ERR_INVALID, "%s: null pointer", what);
   VQB_REQUIRE(vqb_rvq_replay_out_supported(d, num_levels), VQB_ERR_UNSUPPORTED,
-              "vqb_rvq_backward: d=%d (multiple of 4, <= 512), levels=%d (<= %d)", d, num_levels, kMaxReplayLevels);
+              "%s: d=%d (multiple of 4, <= 512), levels=%d (<= %d)", what, d, num_levels, kMaxReplayLevels);
   if (N <= 0) return VQB_OK;
   BackwardArgs B = {};
   B.R.Q = num_levels;
   B.coef = coef;
   for (int l = 0; l < num_levels; ++l) {
-    VQB_REQUIRE(codebooks[l] && idx[l], VQB_ERR_INVALID, "vqb_rvq_backward: null level pointer");
+    VQB_REQUIRE(codebooks[l] && idx[l], VQB_ERR_INVALID, "%s: null level pointer", what);
     B.R.cb[l] = codebooks[l]; B.R.idx[l] = idx[l]; B.R.training[l] = training[l];
   }
   cudaStream_t st = (cudaStream_t)stream;
   const int grid = gather_grid(N);
-  if (d <= 128) rvq_backward_kernel<1><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
-  else if (d <= 256) rvq_backward_kernel<2><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
-  else rvq_backward_kernel<4><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
+  if (rot) {
+    if (d <= 128) rvq_backward_kernel<1, true><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
+    else if (d <= 256) rvq_backward_kernel<2, true><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
+    else rvq_backward_kernel<4, true><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
+  } else {
+    if (d <= 128) rvq_backward_kernel<1, false><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
+    else if (d <= 256) rvq_backward_kernel<2, false><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
+    else rvq_backward_kernel<4, false><<<grid, kGatherThreads, 0, st>>>(x, g_out, mask, grad_x, N, d, B);
+  }
   VQB_LAUNCH_CHECK();
   return VQB_OK;
+}
+
+extern "C" int vqb_rvq_backward(const float* x, const float* const* codebooks, const int64_t* const* idx,
+                                const int* training, int num_levels, const float* coef, const float* g_out,
+                                const uint8_t* mask, float* grad_x, int64_t N, int d, void* stream) {
+  return rvq_backward_launch("vqb_rvq_backward", false, x, codebooks, idx, training, num_levels, coef, g_out, mask,
+                             grad_x, N, d, stream);
+}
+
+extern "C" int vqb_rvq_backward_rot(const float* x, const float* const* codebooks, const int64_t* const* idx,
+                                    const int* training, int num_levels, const float* coef, const float* g_out,
+                                    const uint8_t* mask, float* grad_x, int64_t N, int d, void* stream) {
+  return rvq_backward_launch("vqb_rvq_backward_rot", true, x, codebooks, idx, training, num_levels, coef, g_out, mask,
+                             grad_x, N, d, stream);
 }

@@ -41,6 +41,7 @@ SIGNATURES = {
     "vqb_gather_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "vqb_gather_st_loss": (_i32, [_p, _i32, _p, _p, _p, _i32, _i32, _p, _p, _i64, _i64, _i32, _i32, _p, _sz, _p]),
     "vqb_st_commit_backward": (_i32, [_p, _p, _p, _i32, _p, _p, _p, _f32, _p, _i64, _i64, _i32, _i32, _p]),
+    "vqb_rot_commit_backward": (_i32, [_p, _p, _p, _i32, _p, _p, _p, _f32, _p, _i64, _i64, _i32, _i32, _p]),
     "vqb_ema_workspace_bytes": (_sz, [_i64, _i64, _i32, _i32]),
     "vqb_ema_reduce": (_i32, [_p, _i32, _p, _p, _p, _i64, _i64, _i32, _i32, _p, _p, _sz, _p]),
     "vqb_ema_apply": (_i32, [_p, _p, _p, _p, _f32, _f64, _i32, _i64, _i32, _i32, _p, _sz, _p]),
@@ -56,6 +57,7 @@ SIGNATURES = {
                                        _i64, _i64, _i32, _i32, _p]),
     "vqb_dense_scores": (_i32, [_p, _i32, _p, _p, _p, _i32, _p, _i64, _i64, _i32, _i32, _p]),
     "vqb_rvq_backward": (_i32, [_p, _p, _p, _p, _i32, _p, _p, _p, _p, _i64, _i32, _p]),
+    "vqb_rvq_backward_rot": (_i32, [_p, _p, _p, _p, _i32, _p, _p, _p, _p, _i64, _i32, _p]),
     "vqb_rvq_replay_out_supported": (_i32, [_i32, _i32]),
     "vqb_rvq_replay_out": (_i32, [_p, _p, _p, _p, _i32, _p, _p, _i64, _i32, _p]),
     "vqb_rvq_level_ema_supported": (_i32, [_i32]),

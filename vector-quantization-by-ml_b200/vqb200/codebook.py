@@ -387,7 +387,7 @@ class Codebook(nn.Module):
                                    self.embed_avg.data[h], self.embeddings.data[h])
         self._dirty = self._replica_dirty = True
 
-    def _run_sharded(self, x, mask, freeze_codebook, fuse_st, want_commit, normalize_input):
+    def _run_sharded(self, x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, rotation=False):
         """`_run` for a row-sharded codebook.  Every rank ends up with the quantised vectors / indices of ITS latents
         (all of them when the input is replicated) and updates ITS rows of the EMA buffers from the rows they won --
         no statistics all_reduce; the only exchanges are the min-key all_reduce, one scalar all_reduce for the Laplace
@@ -430,12 +430,13 @@ class Codebook(nn.Module):
             # replicated input: gather/ST/loss over all rows and the EMA sums of ALL codes in one pass; this rank
             # keeps the statistics of its own rows of the codebook
             quant, commit, stats_full = ops.quantize_training(flat, replica, gidx, None, want_commit, ema=True,
-                                                              bound_ws=self.last_search_ws)
+                                                              bound_ws=self.last_search_ws, rotation=rotation)
         elif whole:
             with torch.no_grad():
                 quant, _, stats_full = ops.quantize_ema(flat, replica, gidx, False, False, bound_ws=self.last_search_ws)
         elif fuse_st and training:
-            quant, commit, _ = ops.quantize_training(flat, replica, gidx.contiguous(), mask_u8, want_commit)
+            quant, commit, _ = ops.quantize_training(flat, replica, gidx.contiguous(), mask_u8, want_commit,
+                                                     rotation=rotation)
         else:
             with torch.no_grad():
                 quant, _ = ops.gather_st_loss(flat, replica, gidx.contiguous(), None, False, False)
@@ -542,7 +543,8 @@ class Codebook(nn.Module):
         outs = [piece(flat[:, lo:lo + rows], emb_g, idx[:, lo:lo + rows]) for lo in range(0, N, rows)]
         return torch.cat(outs, dim=1)
 
-    def _run_variants(self, x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, keep_dense):
+    def _run_variants(self, x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, keep_dense,
+                      rotation=False):
         """`_run` with the affine re-parametrisation and / or gumbel sampling (see the module docstring): the same
         kernels, un-fused; returns what `_run` returns."""
         g = self.gumbel
@@ -610,12 +612,19 @@ class Codebook(nn.Module):
                 if want_commit:
                     per = (q_graph - xf) ** 2
                     commit = per[:, mask_u8.bool()].mean() if mask_u8 is not None else per.mean()
-                quant = xf + (q_graph - xf).detach()
+                if rotation:
+                    # the rotation-trick gradient towards c = q_graph (a detached (H,N,d) "codebook" gathered row by
+                    # row): same forward value fl(x + fl(c - x)), same op as the gather path below
+                    c = q_graph.detach().contiguous()
+                    rows = torch.arange(N, device=c.device).expand(H, N).contiguous()
+                    quant, _, _ = ops.quantize_training(xf, c, rows, mask_u8, False, rotation=True)
+                else:
+                    quant = xf + (q_graph - xf).detach()
             else:
                 quant = q_graph
         elif fuse_st and training:
             quant, commit, _ = ops.quantize_training(flat, emb_val if emb_param is None else emb_eff.contiguous(), idx,
-                                                     mask_u8, want_commit)
+                                                     mask_u8, want_commit, rotation=rotation)
         elif emb_param is not None:
             quant = ops.gather_codes(emb_eff.contiguous(), idx)
         else:
@@ -639,17 +648,20 @@ class Codebook(nn.Module):
 
     # ------------------------------------------------------------------ core
     def _run(self, x: torch.Tensor, mask: Optional[torch.Tensor], freeze_codebook: bool, fuse_st: bool,
-             want_commit: bool, normalize_input: bool = False, keep_dense: bool = False):
+             want_commit: bool, normalize_input: bool = False, keep_dense: bool = False, rotation: bool = False):
         """Shared by forward() and VectorQuantize.  x: (H, ..., d).  Returns (quantize (H,...,d), idx (H,...),
         commit scalar | None).  `keep_dense`: leave in `self.dense_ctx` what the consumers of the dense similarities
         (cross-entropy to indices, CE commitment, diversity loss) need: the (H,N,d) latents the search saw and the
-        codebook as it was BEFORE this forward's EMA step (reference codebooks.py:386 runs before :425)."""
+        codebook as it was BEFORE this forward's EMA step (reference codebooks.py:386 runs before :425).
+        `rotation`: where `fuse_st` applies the straight-through estimator, use the rotation-trick gradient instead
+        (`VectorQuantize.rotation_trick`; the returned values do not change)."""
         if self.sharded:
             if keep_dense:
                 raise NotImplementedError("vqb200: the dense-similarity losses are not available on a sharded codebook")
-            return self._run_sharded(x, mask, freeze_codebook, fuse_st, want_commit, normalize_input)
+            return self._run_sharded(x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, rotation)
         if self._variants_active():
-            return self._run_variants(x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, keep_dense)
+            return self._run_variants(x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, keep_dense,
+                                      rotation)
         _lib.require_device(x)        # raises for a CPU tensor: there is no CPU implementation
         flat, lead = self._flatten(x)
         H, N, d = flat.shape
@@ -704,13 +716,14 @@ class Codebook(nn.Module):
             and emb_param is None
         stats = None
         if fused and fuse_st:
-            quant, commit, stats = ops.quantize_training(flat, emb, idx, None, want_commit, ema=True, bound_ws=ws)
+            quant, commit, stats = ops.quantize_training(flat, emb, idx, None, want_commit, ema=True, bound_ws=ws,
+                                                         rotation=rotation)
         elif fused:
             with torch.no_grad():
                 quant, _, stats = ops.quantize_ema(flat, emb, idx, False, False, bound_ws=ws)
         elif fuse_st and training:
             quant, commit, _ = ops.quantize_training(flat, emb if emb_param is None else emb_param, idx, mask_u8,
-                                                     want_commit)
+                                                     want_commit, rotation=rotation)
         elif emb_param is not None:
             quant = ops.gather_codes(emb_param, idx)
         else:

@@ -237,16 +237,34 @@ def st_commit_backward(grad_q: torch.Tensor, g: torch.Tensor, x: torch.Tensor, e
     return gx
 
 
+@_on_device
+def rot_commit_backward(grad_q: torch.Tensor, g: torch.Tensor, x: torch.Tensor, embeddings: torch.Tensor,
+                        idx: torch.Tensor, mask_u8: Optional[torch.Tensor]) -> torch.Tensor:
+    """grad_x (H,N,d) fp32 = T(grad_q) + g[0] * (x - C[idx]) on the rows with mask != 0, grad_q on the others, where T
+    is the rotation-trick transport of each row (vqb_rot_commit_backward)."""
+    H, N, d = x.shape
+    K = embeddings.shape[1]
+    grad_q, x, embeddings = L.aligned(grad_q.float()), L.aligned(x), L.aligned(embeddings)
+    gx = torch.empty((H, N, d), dtype=torch.float32, device=x.device)
+    L.check(L.lib().vqb_rot_commit_backward(L.ptr(grad_q), L.ptr(g), L.ptr(x), L.dtype_code(x), L.ptr(embeddings),
+                                            L.ptr(idx), L.ptr(mask_u8), 1.0, L.ptr(gx), H, N, K, d,
+                                            L.stream_ptr(x.device)), "vqb_rot_commit_backward")
+    return gx
+
+
 class _QuantizeST(torch.autograd.Function):
     """Training-mode quantize: returns (x + (c - x).detach(), mse(c.detach(), x), stats | None).
 
     With `ema` set (no mask) the forward is the fused pass that also produces the EMA statistics.
     Backward (SURVEY K16; reference autograd through vector_quantize_pytorch.py:273,362):
       grad_x = grad_q + grad_commit * 2 (x - c) / (rows_used * d);  the codebook gets no gradient.
+    With `rotation` the gradient of `q` is the rotation trick's (upstream `rotate_to`, arXiv:2410.06424) instead:
+      grad_x = T(grad_q) + grad_commit * 2 (x - c) / (rows_used * d)   on the rows with mask != 0 (vqb_rot_commit_backward);
+    the forward value stays the straight-through one, fl(x + fl(c - x)), bit for bit.
     """
 
     @staticmethod
-    def forward(ctx, x, embeddings, idx, mask_u8, want_loss, ema, bound_ws):
+    def forward(ctx, x, embeddings, idx, mask_u8, want_loss, ema, bound_ws, rotation=False):
         stats = None
         if ema:
             q, loss, stats = quantize_ema(x, embeddings, idx, True, want_loss, bound_ws)
@@ -256,6 +274,7 @@ class _QuantizeST(torch.autograd.Function):
                               if loss is not None else torch.empty(0))
         ctx.has_mask = mask_u8 is not None
         ctx.want_loss = want_loss
+        ctx.rotation = bool(rotation)
         commit = loss[0] if want_loss else torch.zeros((), device=x.device)
         if stats is None:
             stats = torch.empty(0, device=x.device)
@@ -270,19 +289,21 @@ class _QuantizeST(torch.autograd.Function):
         if grad_q is None:
             grad_q = torch.zeros((H, N, d), dtype=torch.float32, device=x.device)
         grad_q = grad_q.contiguous().float()
-        none = (None,) * 6
         g_emb = None
         if ctx.needs_input_grad[1] and ctx.want_loss and grad_commit is not None:
             # learnable codebook: d mse(C[idx], x) / d C[k] = 2 (n_k C[k] - sum of the rows assigned to k) / (rows * d),
             # from the same deterministic segmented sums as the EMA statistics
             st = ema_reduce(x, idx, mask_u8 if ctx.has_mask else None, K)
             g_emb = (grad_commit.float() * (2.0 / d) / loss[1]) * (st[..., d:] * embeddings.detach() - st[..., :d])
-        none = (g_emb,) + (None,) * 5
-        if not ctx.want_loss or grad_commit is None:
+        none = (g_emb,) + (None,) * 6
+        has_commit = ctx.want_loss and grad_commit is not None
+        if not has_commit and not ctx.rotation:
             return (grad_q.to(x.dtype),) + none
         # device scalar: grad_commit * 2 / (rows_used * d)   (no host sync)
-        g = (grad_commit.float() * (2.0 / d) / loss[1]).reshape(1).contiguous()
-        gx = st_commit_backward(grad_q, g, x, embeddings, idx, mask_u8 if ctx.has_mask else None)
+        g = (grad_commit.float() * (2.0 / d) / loss[1]).reshape(1).contiguous() if has_commit \
+            else torch.zeros(1, dtype=torch.float32, device=x.device)
+        mask = mask_u8 if ctx.has_mask else None
+        gx = (rot_commit_backward if ctx.rotation else st_commit_backward)(grad_q, g, x, embeddings, idx, mask)
         return (gx.to(x.dtype),) + none
 
 
@@ -309,10 +330,11 @@ def gather_codes(embeddings: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
     return _GatherCodes.apply(embeddings, idx)
 
 
-def quantize_training(x, embeddings, idx, mask_u8, want_loss, ema: bool = False, bound_ws=None):
-    """(q, commit, stats | None); `ema=True` (mask must be None) uses the fused gather+EMA pass."""
+def quantize_training(x, embeddings, idx, mask_u8, want_loss, ema: bool = False, bound_ws=None, rotation: bool = False):
+    """(q, commit, stats | None); `ema=True` (mask must be None) uses the fused gather+EMA pass; `rotation`: the
+    rotation-trick gradient instead of the straight-through one (same forward values)."""
     assert not (ema and mask_u8 is not None)
-    q, commit, stats = _QuantizeST.apply(x, embeddings, idx, mask_u8, want_loss, ema, bound_ws)
+    q, commit, stats = _QuantizeST.apply(x, embeddings, idx, mask_u8, want_loss, ema, bound_ws, rotation)
     return q, commit, (stats if ema else None)
 
 
@@ -440,11 +462,7 @@ def rvq_replay_out(x: torch.Tensor, codebooks, idxs, training, mask_u8: Optional
     return out
 
 
-@_on_device
-def rvq_backward(x: torch.Tensor, codebooks, idxs, training, coef: torch.Tensor, g_out: Optional[torch.Tensor],
-                 mask_u8: Optional[torch.Tensor]) -> torch.Tensor:
-    """Input gradient (N,d) of a ResidualVQ training forward: Q * g_out + sum_l coef[l] * (r_l - C_l[idx_l]) on the
-    rows with mask != 0 (vqb_rvq_backward); the residuals are replayed from x and the indices."""
+def _rvq_backward(entry: str, x, codebooks, idxs, training, coef, g_out, mask_u8) -> torch.Tensor:
     import ctypes as C
     L.require_cuda(x, "x")
     x = L.aligned(x)
@@ -459,10 +477,26 @@ def rvq_backward(x: torch.Tensor, codebooks, idxs, training, coef: torch.Tensor,
     # with 128-bit loads
     g = L.aligned(g_out.float()) if g_out is not None else None
     gx = torch.empty((N, d), dtype=torch.float32, device=x.device)
-    L.check(L.lib().vqb_rvq_backward(L.ptr(x), C.cast(cbp, C.c_void_p), C.cast(ixp, C.c_void_p),
-                                     C.cast(trp, C.c_void_p), Q, L.ptr(coef), L.ptr(g), L.ptr(mask_u8), L.ptr(gx), N, d,
-                                     L.stream_ptr(x.device)), "vqb_rvq_backward")
+    L.check(getattr(L.lib(), entry)(L.ptr(x), C.cast(cbp, C.c_void_p), C.cast(ixp, C.c_void_p),
+                                    C.cast(trp, C.c_void_p), Q, L.ptr(coef), L.ptr(g), L.ptr(mask_u8), L.ptr(gx), N, d,
+                                    L.stream_ptr(x.device)), entry)
     return gx
+
+
+@_on_device
+def rvq_backward(x: torch.Tensor, codebooks, idxs, training, coef: torch.Tensor, g_out: Optional[torch.Tensor],
+                 mask_u8: Optional[torch.Tensor]) -> torch.Tensor:
+    """Input gradient (N,d) of a ResidualVQ training forward: Q * g_out + sum_l coef[l] * (r_l - C_l[idx_l]) on the
+    rows with mask != 0 (vqb_rvq_backward); the residuals are replayed from x and the indices."""
+    return _rvq_backward("vqb_rvq_backward", x, codebooks, idxs, training, coef, g_out, mask_u8)
+
+
+@_on_device
+def rvq_backward_rot(x: torch.Tensor, codebooks, idxs, training, coef: torch.Tensor, g_out: Optional[torch.Tensor],
+                     mask_u8: Optional[torch.Tensor]) -> torch.Tensor:
+    """`rvq_backward` for levels with the rotation-trick gradient: sum_l T_l(g_out) + sum_l coef[l] * (r_l - c_l) on
+    the rows with mask != 0, T_l the rotation transport of level l (identity on masked rows; vqb_rvq_backward_rot)."""
+    return _rvq_backward("vqb_rvq_backward_rot", x, codebooks, idxs, training, coef, g_out, mask_u8)
 
 
 def rvq_level_ema_supported(d: int) -> bool:

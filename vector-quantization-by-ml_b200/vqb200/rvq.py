@@ -27,7 +27,8 @@ def _round_up_multiple(num, mult):
 
 class ResidualVQ(nn.Module):
     def __init__(self, *, dim, num_quantizers, codebook_dim=None, shared_codebook=False, heads=1,
-                 quantize_dropout=False, quantize_dropout_cutoff_index=0, quantize_dropout_multiple_of=1, **kwargs):
+                 quantize_dropout=False, quantize_dropout_cutoff_index=0, quantize_dropout_multiple_of=1,
+                 rotation_trick=False, **kwargs):
         super().__init__()
         assert heads == 1, "residual vq is not compatible with multi-headed codes"
         codebook_dim = codebook_dim if codebook_dim is not None else dim
@@ -39,6 +40,8 @@ class ResidualVQ(nn.Module):
         self.layers = nn.ModuleList([VectorQuantize(dim=codebook_dim, codebook_dim=codebook_dim, **kwargs)
                                      for _ in range(num_quantizers)])
         assert all(not vq.has_projections for vq in self.layers)
+        for vq in self.layers:                  # the rotation-trick gradient (VectorQuantize.rotation_trick) on every level
+            vq.rotation_trick = bool(rotation_trick)
         self.quantize_dropout = quantize_dropout and num_quantizers > 1
         assert quantize_dropout_cutoff_index >= 0
         self.quantize_dropout_cutoff_index = quantize_dropout_cutoff_index
@@ -97,10 +100,11 @@ class ResidualVQ(nn.Module):
 
     def _can_fuse_autograd(self, x) -> bool:
         """The fused loop under autograd (`_FusedRVQ`): training mode, EMA codebooks (the gradient to the input is all
-        there is), at least two levels and a width the replay kernels take."""
+        there is), at least two levels, a width the replay kernels take and one gradient estimator for all levels."""
         d = x.shape[-1]
         return bool(self.training and all(l.training for l in self.layers)
                     and not any(l._codebook.learnable_codebook for l in self.layers)
+                    and len({l.rotation_trick for l in self.layers}) == 1
                     and len(self.layers) >= 2 and ops.rvq_replay_out_supported(d, len(self.layers)))
 
     def _forward_fused(self, x, mask, freeze_codebook):
@@ -347,7 +351,9 @@ class _FusedRVQ(torch.autograd.Function):
     level returns r_l + (q_l - r_l).detach() and the next residual subtracts a detached quantity, so d out / d x = Q I;
     the commitment loss of level l, mse(c_l.detach(), r_l), adds w_l 2 (r_l - c_l) / (rows d).  Backward is ONE pass
     that replays the residuals from x and the indices (vqb_rvq_backward) against the codebooks as they were before each
-    level's EMA step -- the generic per-level loop instead keeps Q (N,d) residuals alive for autograd."""
+    level's EMA step -- the generic per-level loop instead keeps Q (N,d) residuals alive for autograd.  With
+    `rotation_trick` on every level, each level's output gradient is transported by that level's rotation instead of
+    passed through (vqb_rvq_backward_rot); the forward is the same."""
 
     @staticmethod
     def forward(ctx, x, rvq, mask, freeze_codebook):
@@ -359,6 +365,7 @@ class _FusedRVQ(torch.autograd.Function):
         ctx.idx = [i.reshape(-1) for i in all_idx]
         ctx.mask_u8 = rvq.layers[0]._codebook._expand_mask(mask, x0.shape[0])
         ctx.shape, ctx.dtype = x.shape, x.dtype
+        ctx.rotation = rvq.layers[0].rotation_trick
         idx = torch.stack(all_idx, 0)
         ctx.mark_non_differentiable(idx)
         return out, idx, torch.cat(all_loss, 0)
@@ -372,8 +379,9 @@ class _FusedRVQ(torch.autograd.Function):
             # grad of level l's loss * commitment weight * 2 / (rows used * d), all on the device
             coef = torch.stack([g_losses[l].float() * (w * 2.0 / d) / lb[1] for l, (lb, w) in enumerate(ctx.loss_bufs)])
         g = g_out.reshape(N, d) if g_out is not None else None
-        gx = ops.rvq_backward(ctx.x0, [e[0] for e, _ in ctx.pre_emb], ctx.idx, [tr for _, tr in ctx.pre_emb], coef, g,
-                              ctx.mask_u8)
+        backward = ops.rvq_backward_rot if ctx.rotation else ops.rvq_backward
+        gx = backward(ctx.x0, [e[0] for e, _ in ctx.pre_emb], ctx.idx, [tr for _, tr in ctx.pre_emb], coef, g,
+                      ctx.mask_u8)
         return gx.reshape(ctx.shape).to(ctx.dtype), None, None, None
 
 

@@ -85,6 +85,11 @@ class VectorQuantize(nn.Module):
         assert 0 <= sync_update_v <= 1.0
         assert not (sync_update_v > 0.0 and not codebook_params.learnable_codebook), "learnable codebook must be turned on"
         self.sync_update_v = sync_update_v
+        # upstream vector-quantize-pytorch's `rotation_trick` option (arXiv:2410.06424): when set, the gradient reaches the
+        # input through the rotation of x onto its code instead of the straight-through identity; the forward values do
+        # not change.  An attribute, not a constructor argument, so that the constructor keeps the reference's
+        # parameters exactly; `ResidualVQ(rotation_trick=...)` sets it on every level.
+        self.rotation_trick = False
         kw = asdict(self.codebook_params)
         self._codebook = Codebook(**kw)
         # commit_quantize is detached unless VectorQuantize's OWN learnable_codebook is set (reference :262-268)
@@ -205,10 +210,12 @@ class VectorQuantize(nn.Module):
         if self.in_place_codebook_optimizer is not None and training and not freeze_codebook:
             inplace_loss = self._inplace_optimize(cb_in, mask, multi)
         # transform_input (reference :221) happens inside _run, fused with the search's operand preparation
+        # `rotation` is passed only when set, so a `_run` override without that keyword keeps working by default
+        rot = {"rotation": True} if self.rotation_trick else {}
         quantize, embed_ind, commit = self._codebook._run(cb_in, mask, freeze_codebook, fuse_st=True,
                                                           want_commit=want_commit,
                                                           normalize_input=self._codebook.input_l2norm,
-                                                          keep_dense=keep_dense)
+                                                          keep_dense=keep_dense, **rot)
         dense = self._codebook.dense_ctx
         self._codebook.dense_ctx = None
         # learnable codebook: the similarities stay attached to `embeddings` (reference codebooks.py:375-377, whatever
