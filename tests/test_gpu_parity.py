@@ -478,13 +478,15 @@ def test_in_place_codebook_optimizer_matches_reference_fixture(name):
 @pytest.mark.parametrize("cos", [False, True])
 @pytest.mark.parametrize("case", ["mixed_row_scales", "zero_codebook", "huge_codes_tiny_rows", "huge_rows_tiny_codes",
                                   "padded_codes", "constant_rows"])
-def test_search_scale_extremes_match_exact_scan(case, cos):
+@pytest.mark.parametrize("N", [3000, 100])
+def test_search_scale_extremes_match_exact_scan(N, case, cos):
     """The bias k-step folds s_row 2^-q and s_c 2^q |c|^2/2 into fp16 operands: rows / codebooks at the edges of those
     ranges (zero rows, 10 orders of magnitude between rows, all-zero codebook, bias far larger or smaller than the dot
-    products, padded code columns) must still give the exact scan's answer, index and score, bit for bit."""
+    products, padded code columns) must still give the exact scan's answer, index and score, bit for bit.  N = 100 is
+    one row tile: that search adds the bias in the epilogue of the single-CTA kernel instead."""
     from vqb200 import ops
     g = torch.Generator().manual_seed(sum(map(ord, case)))
-    N, K, d = 3000, 1024, 128
+    K, d = 1024, 128
     x = torch.randn(1, N, d, generator=g)
     c = torch.randn(1, K, d, generator=g) * 0.5
     if case == "mixed_row_scales":
@@ -587,34 +589,20 @@ def test_state_dict_roundtrip_and_cache_invalidation():
     assert torch.equal(i1.cpu(), ref), "search must see embeddings written through load_state_dict"
 
 
-@pytest.mark.parametrize("mode", ["1", "2"])
-def test_alternate_search_kernel_modes_match_exact_scan(mode):
-    """VQB_CLUSTER=1 (independent CTAs) and =2 (2-CTA TMA multicast of the codebook stream) are opt-in variants of
-    the search kernel (default: 3 = cta_group::2 pair MMA); they must give the same indices as the exact scan (env is read once per process -> subprocess)."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = r'''
-import sys, torch
-sys.path.insert(0, r"%s")
-from vqb200 import ops
-dev = torch.device("cuda:0")
-for (H, N, K, d, cos) in [(1, 700, 300, 72, False), (2, 1500, 520, 256, True), (1, 40000, 2048, 128, False), (1, 257, 4096, 512, False)]:
+@pytest.mark.parametrize("H,N,K,d,cos", [(1, 700, 300, 72, False), (2, 1500, 520, 256, True),
+                                         (1, 40000, 2048, 128, False), (1, 257, 4096, 512, False)])
+def test_default_search_kernels_match_exact_scan(H, N, K, d, cos):
+    """The tensor-core search must give the exact scan's indices: several heads, both metrics, many row tiles, d = 512."""
+    from vqb200 import ops
     g = torch.Generator().manual_seed(N)
-    x = torch.randn(H, N, d, generator=g).to(dev)
-    c = (torch.randn(H, K, d, generator=g) * 0.5).to(dev)
+    x = torch.randn(H, N, d, generator=g).to(_dev())
+    c = (torch.randn(H, K, d, generator=g) * 0.5).to(_dev())
     cache = ops.prepare_codebook(c, cos)
     a, _, ws = ops.search(x, c, cache, cos)
     st = ops.search_stats(ws)
     b, _, _ = ops.search(x, c, cache, cos, force_exact=True)
     assert st["tensor_core_pass"] == 1
     assert torch.equal(a, b), (H, N, K, d, int((a != b).sum()))
-print("MODE OK")
-''' % os.path.join(root, "vector-quantization-by-ml_b200")
-    env = dict(os.environ, VQB_CLUSTER=mode)
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300, env=env)
-    assert out.returncode == 0 and "MODE OK" in out.stdout, out.stdout[-1500:] + out.stderr[-3000:]
 
 
 @pytest.mark.parametrize("name", gu.rvq_learnable_fixture_names())

@@ -1,4 +1,5 @@
-"""Times only the tensor-core search kernel (CUDA events from the library) under the env knobs set by the caller."""
+"""Times only the tensor-core search kernel (CUDA events from the library) under the env set by the caller:
+VQB_FUSED_PREP, and VQB_LIB_OVERRIDE for another build of the library (e.g. with a patch from profiles/ applied)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "vector-quantization-by-ml_b200"))
@@ -23,19 +24,6 @@ for _ in range(5):
 torch.cuda.synchronize()
 t = ops.search_kernel_times_ms()
 ms = sum(t) / len(t)
-import ctypes as C
-from vqb200 import _lib
-buf = (C.c_ulonglong * 18)()
-_lib.lib().vqb_debug_counters(buf)
-cy = [buf[2 + i] for i in range(16)]
-if cy[3]:
-    nb = 148 * 8   # CTAs x timed launches (3 warm-up + 5 timed)
-    f = lambda v: f"{v / nb / 1e3:9.1f}k"
-    print(f"   per CTA-launch cycles: producer total {f(cy[0])} wait a_empty {f(cy[1])} wait stage-empty {f(cy[2])}")
-    print(f"                          mma      total {f(cy[3])} wait tmem_empty {f(cy[4])} wait a_full {f(cy[5])} wait stage-full {f(cy[6])}")
-    print(f"                          epi warp total {f(cy[7])} wait tmem_full {f(cy[8])} wait bias {f(cy[9])} tmem ld wait {f(cy[10])} try tmem_full {f(cy[11])}")
-if buf[0] + buf[1]:
-    print(f"   ranked chunks {buf[0]}  skipped {buf[1]}  -> ranked fraction {buf[0] / (buf[0] + buf[1]):.3f}")
 print(os.environ.get('VQB_LIB_OVERRIDE','shipped'), end=' ')
-print(f"VQB_DRAIN={os.environ.get('VQB_DRAIN','-')} VQB_CLUSTER={os.environ.get('VQB_CLUSTER','-')} VQB_TC_DEBUG={os.environ.get('VQB_TC_DEBUG','0')} N={N} K={K} d={d}: "
+print(f"N={N} K={K} d={d}: "
       f"tc kernel {ms:.3f} ms  {2*N*K*d/ms/1e9:.0f} TFLOP/s", flush=True)

@@ -253,9 +253,10 @@ struct ConvArgs {
   int x_dtype = 0;
   int d = 0;
 };
-// xaug / caug: the bias k-step operands (both NULL: bias added in the epilogue from `bias`)
-// aug_mode (search_tc_aug_mode): 0 = bias added in the epilogue from `bias`; 1 = bias as an extra MMA k-step;
-// 2 = same kernel without the k-step (dot metric, no padded codes)
+// xaug / caug: the bias k-step operands (not read when aug_mode is 0)
+// aug_mode (search_tc_aug_mode): 0 = one row tile per codebook: search_tc_kernel adds the bias in the epilogue from
+// `bias`; 1 = search_aug_kernel, bias as an extra MMA k-step; 2 = search_aug_kernel without the k-step (dot metric,
+// no padded codes)
 // xn2 / tie: per-row bound of |x|^2 and the tie-window coefficient (kTieSlack for the Euclidean metric, 0 for dot)
 int launch_search_tc(const __half* xb, const float* xinv, const float* xn2, float tie, const __half* xaug,
                      const __half* cb, const __half* caug, const float* chdr, const float* bias, int aug_mode,

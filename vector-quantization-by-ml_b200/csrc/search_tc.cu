@@ -11,8 +11,8 @@
 // the whole codebook streams through a ring of 32 KB stages (B operand, 256 codes x 64 dims).
 // Accumulators are double buffered in TMEM (2 x 256 columns) so the epilogue of N-tile i
 // overlaps the MMAs of N-tile i+1.  The N x K score matrix never leaves the SM.
-// With CLUSTER=2 the two CTAs of a cluster work on neighbouring row tiles and share every B
-// stage: each loads half of it and multicasts to both (halves L2->SM traffic).
+// search_tc_kernel (bias added in the epilogue) serves problems with one row tile per codebook; every other search
+// runs search_aug_kernel (CTA pairs, bias as an extra MMA k-step), below.
 //
 // Operands are fp16 with exact power-of-two scales (per latent row, per codebook) that the epilogue
 // undoes with the same FFMA that adds the bias.
@@ -65,13 +65,6 @@ __device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
       : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
   return ok != 0;
 }
-// mbar_wait that adds the cycles spent to `acc` when profiling is on (bring-up only)
-__device__ __forceinline__ void mbar_wait_t(uint32_t bar, uint32_t parity, bool prof, unsigned long long& acc) {
-  if (!prof) { mbar_wait(bar, parity); return; }
-  const long long t0 = clock64();
-  mbar_wait(bar, parity);
-  acc += (unsigned long long)(clock64() - t0);
-}
 __device__ __forceinline__ void fence_barrier_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
@@ -107,13 +100,6 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map
       "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
       " [%0], [%1, {%3, %4, %5}], [%2], %6;"
       ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "l"(hint) : "memory");
-}
-__device__ __forceinline__ void tma_load_3d_mc(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1,
-                                               int c2, uint16_t mask, uint64_t hint) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster.L2::cache_hint"
-      " [%0], [%1, {%4, %5, %6}], [%2], %3, %7;"
-      ::"r"(dst), "l"(map), "r"(bar), "h"(mask), "r"(c0), "r"(c1), "r"(c2), "l"(hint) : "memory");
 }
 
 // ---- 2-CTA ("pair") forms: one tcgen05.mma.cta_group::2 covers 256 rows (128 per CTA) x 256 codes (each CTA holds
@@ -154,11 +140,6 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
 // arrive on an mbarrier once all previously issued MMAs have completed (implies fence::before_thread_sync)
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(bar), "h"(mask) : "memory");
 }
 
 // K-major, 128B-swizzled smem operand descriptor (cute::UMMA::SmemDescriptor bit layout):
@@ -204,8 +185,6 @@ __device__ __forceinline__ void top2_pair(float& m1, float& m2, float a, float b
   m1 = fminf(m1, lo);
 }
 
-__device__ unsigned long long g_dbg_cycles[16];    // bring-up only (VQB_TC_DEBUG & 32): where each role waits
-__device__ unsigned long long g_dbg_counters[2];   // bring-up only (VQB_TC_DEBUG & 16): ranked / skipped chunks
 #ifdef VQB_TRACE
 // bring-up only (-DVQB_TRACE): cluster 0 stamps clock64 per tile.  g_trace_mma[role][tile]: 0 tmem_empty seen,
 // 1 MMAs + commits issued, 2 (with -DVQB_TRACE_MMA_LAT) tmem_full seen by the issuing warp itself.
@@ -232,7 +211,7 @@ __device__ __forceinline__ float pack_id(float v, uint32_t mask) {
 }
 
 // The epilogue is a software pipeline over 16-column chunks of one thread's row: a thread owns one row (TMEM lane)
-// and a 64-column quarter of the tile = 4 chunks.  Measured with the cycle counters below: a tcgen05.ld -> wait round
+// and a 64-column quarter of the tile = 4 chunks.  Measured with in-kernel cycle counters: a tcgen05.ld -> wait round
 // trip costs ~400 cycles of latency plus ~8 cycles per column of transfer while the tensor pipe is accumulating into
 // TMEM; with four epilogue warps per sub-partition those waits overlap.
 //   scores : wait for the chunk's accumulators (tcgen05.wait::ld), score = acc*ninv + bias (FFMA, undoes the operand
@@ -244,16 +223,9 @@ __device__ __forceinline__ float pack_id(float v, uint32_t mask) {
 //            no candidate and nothing else is done.  SLOW PATH -- 6-bit id PARITY*32 + CH*8 + i packed into the low
 //            mantissa bits (column j = 2*i + c is class c), running top-2 per class, exactly as if no chunk had been
 //            skipped.
-template <int MODE>
 __device__ __forceinline__ float chunk_scores(const uint32_t (&r)[16], const float4* bias4, float ninv,
-                                              float (&key)[16], bool prof, unsigned long long& w_ld) {
-  if (MODE == 1 && prof) {
-    const long long t0 = clock64();
-    tmem_ld_wait();
-    w_ld += (unsigned long long)(clock64() - t0);
-  } else {
-    tmem_ld_wait();
-  }
+                                              float (&key)[16]) {
+  tmem_ld_wait();
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const float4 b = bias4[i];          // shared memory, same address in every lane: broadcast
@@ -274,17 +246,11 @@ __device__ __forceinline__ void pack_pair(float (&key)[16], int i, uint32_t mask
   key[2 * i + 1] = pack_id<ID>(key[2 * i + 1], mask);
 }
 
-template <int PARITY, int CH, int MODE>
+template <int PARITY, int CH>
 __device__ __forceinline__ void chunk_rank(float (&key)[16], float cmin, uint32_t idmask, float tconst, float& m_run,
                                            float& t_run, int* row_slot, float (&a1)[2], float (&a2)[2],
-                                           bool& any_slow, int dbg) {
-  bool trig = __any_sync(0xffffffffu, cmin <= t_run);
-  if (MODE == 1 && dbg) {   // bring-up knobs: 4 = never rank, 8 = always rank, 16 = count ranked / skipped chunks
-    if (dbg & 4) trig = false;
-    if (dbg & 8) trig = true;
-    if ((dbg & 16) && (threadIdx.x & 31) == 0) atomicAdd(g_dbg_counters + (trig ? 0 : 1), 1ull);
-  }
-  if (trig) {
+                                           bool& any_slow) {
+  if (__any_sync(0xffffffffu, cmin <= t_run)) {
     any_slow = true;
     constexpr uint32_t kBase = (uint32_t)(PARITY * 32 + CH * 8);
     pack_pair<kBase + 0>(key, 0, idmask); pack_pair<kBase + 1>(key, 1, idmask);
@@ -345,8 +311,7 @@ struct SearchParams {
   int KB;              // k-blocks = d_pad / 64
   int NT;              // N tiles = Kp / 256
   int S;               // B stages
-  int GPH;             // row-tile groups per head = ceil(ceil(N/128) / CLUSTER)
-  int dbg;             // bring-up knobs (env VQB_TC_DEBUG): 4 = never rank, 8 = always rank, 16 = count ranked chunks
+  int MT;              // row tiles per head = ceil(N/128)
 };
 
 struct Barriers {
@@ -357,7 +322,6 @@ struct Barriers {
   uint64_t tmem_full[2];
   uint64_t tmem_empty[2];
   uint64_t bias_full[2];
-  uint64_t bias_empty[2];   // pair mode only: the local epilogue released the bias slot
   uint32_t tmem_base;
   uint32_t pad;
   alignas(16) float bias[2][kBlockN];   // per-accumulator-buffer copy of the N tile's biases (staged by warp 3)
@@ -369,11 +333,8 @@ struct Barriers {
   int rowmin[3][kBlockM];
 };
 
-// CLUSTER = 1: independent CTAs.  CLUSTER = 2, !PAIR: two CTAs share every B stage by TMA multicast (each runs its own
-// 128-row MMAs).  CLUSTER = 2, PAIR: cta_group::2 -- one 256-row MMA per pair, each CTA stores only half of B (half the
-// shared-memory operand traffic per SM, twice the stages in flight).
-// MODE 0 = production (no knobs compiled in), 1 = bring-up knobs (VQB_TC_DEBUG)
-template <int CLUSTER, bool PAIR, int MODE>
+// Persistent, one CTA per SM and no clusters: each CTA walks the (codebook, 128-row tile) items with a stride of the
+// grid.  Launched for problems with a single row tile per codebook (search_tc_aug_mode() == 0).
 __global__ void __launch_bounds__(kThreads, 1)
 search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_c,
                  const SearchParams P) {
@@ -383,13 +344,11 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
   const uint32_t smem_base = smem_u32(smem);
   const uint32_t a_base = smem_base;
   const uint32_t b_base = smem_base + (uint32_t)P.KB * kSlabBytes;
-  constexpr uint32_t kStageStride = PAIR ? kStageBytes / 2 : kStageBytes;   // bytes of one B stage in THIS CTA
-  Barriers* bars = reinterpret_cast<Barriers*>(smem + (size_t)P.KB * kSlabBytes + (size_t)P.S * kStageStride);
+  Barriers* bars = reinterpret_cast<Barriers*>(smem + (size_t)P.KB * kSlabBytes + (size_t)P.S * kStageBytes);
 
-  const uint32_t rank = CLUSTER > 1 ? cluster_ctarank() : 0u;
-  const int cid = blockIdx.x / CLUSTER;
-  const int num_clusters = gridDim.x / CLUSTER;
-  const int G = P.H * P.GPH;
+  const int cta = blockIdx.x;
+  const int num_ctas = gridDim.x;
+  const int G = P.H * P.MT;                    // (codebook, row tile) work items
 
   if (threadIdx.x == 0 && (smem_base & 1023u)) {   // the swizzle pattern assumes 1024B-aligned tiles
     atomicExch(P.scal + 5, 1u);
@@ -402,7 +361,7 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
   if (warp == kWarpMma && lane == 0) {
     for (int i = 0; i < P.S; ++i) {
       mbar_init(smem_u32(&bars->full[i]), 1);
-      mbar_init(smem_u32(&bars->empty[i]), PAIR ? 1 : CLUSTER);
+      mbar_init(smem_u32(&bars->empty[i]), 1);
     }
     for (int i = 0; i < P.KB; ++i) {
       mbar_init(smem_u32(&bars->a_full[i]), 1);
@@ -410,142 +369,84 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(smem_u32(&bars->tmem_full[i]), 1);
-      mbar_init(smem_u32(&bars->tmem_empty[i]), PAIR ? 2 * kNumEpiWarps : kNumEpiWarps);
+      mbar_init(smem_u32(&bars->tmem_empty[i]), kNumEpiWarps);
       mbar_init(smem_u32(&bars->bias_full[i]), 1);
-      mbar_init(smem_u32(&bars->bias_empty[i]), kNumEpiWarps);
     }
     fence_barrier_init();
   }
   if (threadIdx.x < 3 * kBlockM) (&bars->rowmin[0][0])[threadIdx.x] = 0x7fffffff;
   if (warp == kWarpAlloc) {
-    if (PAIR) {   // both CTAs of the pair issue it, same warp id, same destination offset
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
-                   ::"r"(smem_u32(&bars->tmem_base)), "n"(kTmemCols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                   ::"r"(smem_u32(&bars->tmem_base)), "n"(kTmemCols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                 ::"r"(smem_u32(&bars->tmem_base)), "n"(kTmemCols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
-  if (CLUSTER > 1) cluster_sync_all(); else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = bars->tmem_base;
 
   if (warp == kWarpTma) {
     // =============================== TMA producer ===============================
     // The whole warp runs the loop (barrier waits are warp-uniform); one elected lane issues expect_tx + TMA.
-    {
-      uint32_t stage = 0, ph = 0, a_ph = 0;
-      const bool prof = MODE == 1 && (P.dbg & 32) != 0;
-      unsigned long long w_a = 0, w_e = 0;
-      const long long t_begin = clock64();
-      for (int g = cid; g < G; g += num_clusters) {
-        const int h = g / P.GPH;
-        const int mt = (g - h * P.GPH) * CLUSTER + (int)rank;
-        const int row0 = mt * kBlockM;
-        for (int nt = 0; nt < P.NT; ++nt) {
-          for (int kb = 0; kb < P.KB; ++kb) {
-            if (nt == 0) {   // (re)load slab kb of this row tile as soon as the previous tile's MMAs released it
-              mbar_wait_t(smem_u32(&bars->a_empty[kb]), a_ph ^ 1u, prof, w_a);
-              if (elect_one()) {
-                if (PAIR) {   // both CTAs' slabs complete on the LEADER's barrier
-                  if (rank == 0) mbar_expect_tx(smem_u32(&bars->a_full[kb]), 2 * kSlabBytes);
-                  tma_load_3d_pair(a_base + kb * kSlabBytes, &map_x, smem_u32(&bars->a_full[kb]) & kPeerBitMask,
-                                   kb * kBlockK, row0, h, kEvictFirst);
-                } else {
-                  mbar_expect_tx(smem_u32(&bars->a_full[kb]), kSlabBytes);
-                  tma_load_3d(a_base + kb * kSlabBytes, &map_x, smem_u32(&bars->a_full[kb]), kb * kBlockK, row0, h,
-                              kEvictFirst);
-                }
-              }
-              __syncwarp();
-            }
-            mbar_wait_t(smem_u32(&bars->empty[stage]), ph ^ 1u, prof, w_e);
+    uint32_t stage = 0, ph = 0, a_ph = 0;
+    for (int g = cta; g < G; g += num_ctas) {
+      const int h = g / P.MT;
+      const int row0 = (g - h * P.MT) * kBlockM;
+      for (int nt = 0; nt < P.NT; ++nt) {
+        for (int kb = 0; kb < P.KB; ++kb) {
+          if (nt == 0) {   // (re)load slab kb of this row tile as soon as the previous tile's MMAs released it
+            mbar_wait(smem_u32(&bars->a_empty[kb]), a_ph ^ 1u);
             if (elect_one()) {
-              if (PAIR) {   // this CTA's 128 codes of the N tile into ITS stage; bytes counted on the leader's barrier
-                if (rank == 0) mbar_expect_tx(smem_u32(&bars->full[stage]), kStageBytes);
-                tma_load_3d_pair(b_base + stage * kStageStride, &map_c, smem_u32(&bars->full[stage]) & kPeerBitMask,
-                                 kb * kBlockK, nt * kBlockN + (int)rank * (kBlockN / 2), h, kEvictLast);
-              } else {
-                mbar_expect_tx(smem_u32(&bars->full[stage]), kStageBytes);
-                if (CLUSTER > 1) {
-                  constexpr int rows = kBlockN / CLUSTER;
-                  tma_load_3d_mc(b_base + stage * kStageBytes + rank * (rows * kBlockK * 2), &map_c,
-                                 smem_u32(&bars->full[stage]), kb * kBlockK, nt * kBlockN + (int)rank * rows, h,
-                                 (uint16_t)((1u << CLUSTER) - 1u), kEvictLast);
-                } else {
-                  tma_load_3d(b_base + stage * kStageBytes, &map_c, smem_u32(&bars->full[stage]), kb * kBlockK,
-                              nt * kBlockN, h, kEvictLast);
-                }
-              }
+              mbar_expect_tx(smem_u32(&bars->a_full[kb]), kSlabBytes);
+              tma_load_3d(a_base + kb * kSlabBytes, &map_x, smem_u32(&bars->a_full[kb]), kb * kBlockK, row0, h,
+                          kEvictFirst);
             }
             __syncwarp();
-            if (++stage == (uint32_t)P.S) { stage = 0; ph ^= 1u; }
           }
+          mbar_wait(smem_u32(&bars->empty[stage]), ph ^ 1u);
+          if (elect_one()) {
+            mbar_expect_tx(smem_u32(&bars->full[stage]), kStageBytes);
+            tma_load_3d(b_base + stage * kStageBytes, &map_c, smem_u32(&bars->full[stage]), kb * kBlockK,
+                        nt * kBlockN, h, kEvictLast);
+          }
+          __syncwarp();
+          if (++stage == (uint32_t)P.S) { stage = 0; ph ^= 1u; }
         }
-        a_ph ^= 1u;
       }
-      if (prof && lane == 0) {
-        atomicAdd(g_dbg_cycles + 0, (unsigned long long)(clock64() - t_begin));
-        atomicAdd(g_dbg_cycles + 1, w_a);
-        atomicAdd(g_dbg_cycles + 2, w_e);
-      }
+      a_ph ^= 1u;
     }
   } else if (warp == kWarpMma) {
-    // =============================== MMA issuer (pair mode: leader CTA only) ===============================
+    // =============================== MMA issuer ===============================
     // The whole warp runs the loop; one elected lane issues the tcgen05.mma / tcgen05.commit instructions.
-    if (!PAIR || rank == 0) {
-      uint32_t stage = 0, ph = 0, a_ph = 0, acc = 0, acc_ph = 0;
-      const bool prof = MODE == 1 && (P.dbg & 32) != 0;
-      unsigned long long w_te = 0, w_a = 0, w_f = 0;
-      const long long t_begin = clock64();
-      for (int g = cid; g < G; g += num_clusters) {
-        for (int nt = 0; nt < P.NT; ++nt) {
-          mbar_wait_t(smem_u32(&bars->tmem_empty[acc]), acc_ph ^ 1u, prof, w_te);   // epilogue drained this accumulator
+    uint32_t stage = 0, ph = 0, a_ph = 0, acc = 0, acc_ph = 0;
+    for (int g = cta; g < G; g += num_ctas) {
+      for (int nt = 0; nt < P.NT; ++nt) {
+        mbar_wait(smem_u32(&bars->tmem_empty[acc]), acc_ph ^ 1u);   // epilogue drained this accumulator
+        tc_fence_after();
+        const uint32_t d_tmem = tmem_base + acc * (uint32_t)kBlockN;
+        for (int kb = 0; kb < P.KB; ++kb) {
+          if (nt == 0) mbar_wait(smem_u32(&bars->a_full[kb]), a_ph);
+          mbar_wait(smem_u32(&bars->full[stage]), ph);
           tc_fence_after();
-          const uint32_t d_tmem = tmem_base + acc * (uint32_t)kBlockN;
-          for (int kb = 0; kb < P.KB; ++kb) {
-            if (nt == 0) mbar_wait_t(smem_u32(&bars->a_full[kb]), a_ph, prof, w_a);
-            mbar_wait_t(smem_u32(&bars->full[stage]), ph, prof, w_f);
-            tc_fence_after();
-            if (elect_one()) {
-              const uint64_t adesc = make_sw128_desc(a_base + kb * kSlabBytes);
-              const uint64_t bdesc = make_sw128_desc(b_base + stage * kStageStride);
+          if (elect_one()) {
+            const uint64_t adesc = make_sw128_desc(a_base + kb * kSlabBytes);
+            const uint64_t bdesc = make_sw128_desc(b_base + stage * kStageBytes);
 #pragma unroll
-              for (int kk = 0; kk < kBlockK / 16; ++kk) {
-                // +32 B per 16-element k step inside the 128B swizzle atom = +2 in the (addr>>4) field
-                if (PAIR) umma_f16_pair(d_tmem, adesc + (uint64_t)(kk * 2), bdesc + (uint64_t)(kk * 2), kIdescPair,
-                                        (kb | kk) != 0 ? 1u : 0u);
-                else umma_f16(d_tmem, adesc + (uint64_t)(kk * 2), bdesc + (uint64_t)(kk * 2), kIdesc,
-                              (kb | kk) != 0 ? 1u : 0u);
-              }
-              if (PAIR) umma_commit_pair(smem_u32(&bars->empty[stage]));
-              else if (CLUSTER > 1) umma_commit_mc(smem_u32(&bars->empty[stage]), (uint16_t)((1u << CLUSTER) - 1u));
-              else umma_commit(smem_u32(&bars->empty[stage]));
-              if (nt == P.NT - 1) {                                            // slab kb may be overwritten
-                if (PAIR) umma_commit_pair(smem_u32(&bars->a_empty[kb]));
-                else umma_commit(smem_u32(&bars->a_empty[kb]));
-              }
-              if (kb == P.KB - 1) {                                            // accumulator complete
-                if (PAIR) umma_commit_pair(smem_u32(&bars->tmem_full[acc]));
-                else umma_commit(smem_u32(&bars->tmem_full[acc]));
-              }
+            for (int kk = 0; kk < kBlockK / 16; ++kk) {
+              // +32 B per 16-element k step inside the 128B swizzle atom = +2 in the (addr>>4) field
+              umma_f16(d_tmem, adesc + (uint64_t)(kk * 2), bdesc + (uint64_t)(kk * 2), kIdesc,
+                       (kb | kk) != 0 ? 1u : 0u);
             }
-            __syncwarp();
-            if (++stage == (uint32_t)P.S) { stage = 0; ph ^= 1u; }
+            umma_commit(smem_u32(&bars->empty[stage]));
+            if (nt == P.NT - 1) umma_commit(smem_u32(&bars->a_empty[kb]));     // slab kb may be overwritten
+            if (kb == P.KB - 1) umma_commit(smem_u32(&bars->tmem_full[acc]));  // accumulator complete
           }
-          if (++acc == 2) { acc = 0; acc_ph ^= 1u; }
+          __syncwarp();
+          if (++stage == (uint32_t)P.S) { stage = 0; ph ^= 1u; }
         }
-        a_ph ^= 1u;
+        if (++acc == 2) { acc = 0; acc_ph ^= 1u; }
       }
-      if (prof && lane == 0) {
-        atomicAdd(g_dbg_cycles + 3, (unsigned long long)(clock64() - t_begin));
-        atomicAdd(g_dbg_cycles + 4, w_te);
-        atomicAdd(g_dbg_cycles + 5, w_a);
-        atomicAdd(g_dbg_cycles + 6, w_f);
-      }
+      a_ph ^= 1u;
     }
   } else if (warp == kWarpStager) {
     // =============================== bias stager ===============================
@@ -555,24 +456,23 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
     // released that buffer (same cadence as the MMA warp).
     // The loads of tile i+1 are issued before the wait for tile i's slot, so their L2 latency is off the critical path.
     uint32_t acc = 0, acc_ph = 0;
-    int g = cid, nt = 0;
+    int g = cta, nt = 0;
     float4 v0 = make_float4(0.f, 0.f, 0.f, 0.f), v1 = v0;
     if (g < G) {
-      const float* b = P.bias + (size_t)(g / P.GPH) * P.Kp;
+      const float* b = P.bias + (size_t)(g / P.MT) * P.Kp;
       v0 = __ldg(reinterpret_cast<const float4*>(b) + lane);
       v1 = __ldg(reinterpret_cast<const float4*>(b) + 32 + lane);
     }
     while (g < G) {
       int g2 = g, nt2 = nt + 1;
-      if (nt2 == P.NT) { nt2 = 0; g2 += num_clusters; }
+      if (nt2 == P.NT) { nt2 = 0; g2 += num_ctas; }
       float4 n0 = v0, n1 = v1;
       if (g2 < G) {
-        const float* b = P.bias + (size_t)(g2 / P.GPH) * P.Kp + nt2 * kBlockN;
+        const float* b = P.bias + (size_t)(g2 / P.MT) * P.Kp + nt2 * kBlockN;
         n0 = __ldg(reinterpret_cast<const float4*>(b) + lane);
         n1 = __ldg(reinterpret_cast<const float4*>(b) + 32 + lane);
       }
-      if (PAIR) mbar_wait(smem_u32(&bars->bias_empty[acc]), acc_ph ^ 1u);   // local epilogue released the slot
-      else mbar_wait(smem_u32(&bars->tmem_empty[acc]), acc_ph ^ 1u);
+      mbar_wait(smem_u32(&bars->tmem_empty[acc]), acc_ph ^ 1u);
       reinterpret_cast<float4*>(bars->bias[acc])[lane] = v0;
       reinterpret_cast<float4*>(bars->bias[acc])[32 + lane] = v1;
       __syncwarp();
@@ -589,20 +489,16 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16) + quarter * 64;
     // Emax * (2 + slack): the part of the candidate threshold that does not depend on the row minimum
     const float tconst = __uint_as_float(P.scal[6]) * (2.f + kPackSlackTC);
-    const bool prof = MODE == 1 && (P.dbg & 32) != 0 && warp == 0;
-    unsigned long long w_tf = 0, w_bias = 0, w_ld = 0, w_try = 0;
-    const long long t_begin = clock64();
     uint32_t r[16];
     uint32_t tile_it = 0;                           // row tiles processed by this CTA so far
-    if (cid < G) {   // pipeline prologue: first chunk of the very first tile (later ones are prefetched in the loop)
+    if (cta < G) {   // pipeline prologue: first chunk of the very first tile (later ones are prefetched in the loop)
       mbar_wait(smem_u32(&bars->tmem_full[0]), 0);
       tc_fence_after();
       TMEM_LD16(lane_addr, r);
     }
-    for (int g = cid; g < G; g += num_clusters) {
-      const int h = g / P.GPH;
-      const int mt = (g - h * P.GPH) * CLUSTER + (int)rank;
-      const int64_t row = (int64_t)mt * kBlockM + q * 32 + lane;
+    for (int g = cta; g < G; g += num_ctas) {
+      const int h = g / P.MT;
+      const int64_t row = (int64_t)(g - h * P.MT) * kBlockM + q * 32 + lane;
       float M1[2], M2[2], M3[2];
       int C1[2], C2[2], C3[2];
 #pragma unroll
@@ -617,7 +513,7 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
       float m_run = INF, t_run = INF;              // running row minimum (this thread's columns) and its threshold
       // shared running minimum of the row (all four quarters); disabled for tiny codebooks (see Barriers::rowmin)
       int* row_slot = nullptr;
-      if (P.NT >= 4 && !(MODE == 1 && (P.dbg & 64))) {
+      if (P.NT >= 4) {
         bars->rowmin[(tile_it + 1) % 3][q * 32 + lane] = 0x7fffffff;        // reset the NEXT row tile's slot
         row_slot = &bars->rowmin[tile_it % 3][q * 32 + lane];
       }
@@ -636,45 +532,36 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
           if (nt + par < P.NT) {
             // r[] already holds (or is receiving) chunk 0 of this tile
             const uint32_t taddr = lane_addr + acc * (uint32_t)kBlockN;
-            mbar_wait_t(smem_u32(&bars->bias_full[acc]), acc_ph, prof, w_bias);
+            mbar_wait(smem_u32(&bars->bias_full[acc]), acc_ph);
             const float4* bias4 = reinterpret_cast<const float4*>(bars->bias[acc] + quarter * 64);
             float key[16];
             float cmin;
 #define VQB_CHUNK(CH)                                                                                      \
-            cmin = chunk_scores<MODE>(r, bias4 + (CH) * 4, ninv, key, prof, w_ld);                                   \
+            cmin = chunk_scores(r, bias4 + (CH) * 4, ninv, key);                                           \
             TMEM_LD16(taddr + ((CH) + 1) * 16, r);                                                         \
-            if (par == 0) chunk_rank<0, (CH), MODE>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow, P.dbg); \
-            else chunk_rank<1, (CH), MODE>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow, P.dbg);
+            if (par == 0) chunk_rank<0, (CH)>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow); \
+            else chunk_rank<1, (CH)>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow);
             VQB_CHUNK(0) VQB_CHUNK(1) VQB_CHUNK(2)
 #undef VQB_CHUNK
             // last chunk: once its scores are formed every TMEM read of this tile is complete -> hand the buffer
             // back to the MMA warp, then start loading the next tile's first chunk (before this chunk's ranking
             // work if that accumulator is already complete)
-            cmin = chunk_scores<MODE>(r, bias4 + 12, ninv, key, prof, w_ld);
+            cmin = chunk_scores(r, bias4 + 12, ninv, key);
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) {
-              if (PAIR) {   // the leader's MMA thread waits for BOTH CTAs' epilogues; the bias slot is local
-                mbar_arrive_leader(smem_u32(&bars->tmem_empty[acc]));
-                mbar_arrive(smem_u32(&bars->bias_empty[acc]));
-              } else {
-                mbar_arrive(smem_u32(&bars->tmem_empty[acc]));
-              }
-            }
+            if (lane == 0) mbar_arrive(smem_u32(&bars->tmem_empty[acc]));
             if (++acc == 2) { acc = 0; acc_ph ^= 1u; }
-            const bool more = (nt + par + 1 < P.NT) || (g + num_clusters < G);
+            const bool more = (nt + par + 1 < P.NT) || (g + num_ctas < G);
             bool issued = false;
-            const long long t_try = (MODE == 1 && prof) ? clock64() : 0;
             if (more && mbar_try(smem_u32(&bars->tmem_full[acc]), acc_ph)) {
               tc_fence_after();
               TMEM_LD16(lane_addr + acc * (uint32_t)kBlockN, r);
               issued = true;
             }
-            if (MODE == 1 && prof) w_try += (unsigned long long)(clock64() - t_try);
-            if (par == 0) chunk_rank<0, 3, MODE>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow, P.dbg);
-            else chunk_rank<1, 3, MODE>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow, P.dbg);
+            if (par == 0) chunk_rank<0, 3>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow);
+            else chunk_rank<1, 3>(key, cmin, idmask, trow, m_run, t_run, row_slot, a1, a2, any_slow);
             if (more && !issued) {
-              mbar_wait_t(smem_u32(&bars->tmem_full[acc]), acc_ph, prof, w_tf);
+              mbar_wait(smem_u32(&bars->tmem_full[acc]), acc_ph);
               tc_fence_after();
               TMEM_LD16(lane_addr + acc * (uint32_t)kBlockN, r);
             }
@@ -702,22 +589,13 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
         out4[2] = make_uint4(__float_as_uint(M2[1]), (uint32_t)C2[1], __float_as_uint(M3[1]), (uint32_t)C3[1]);
       }
     }
-    if (prof && lane == 0) {
-      atomicAdd(g_dbg_cycles + 7, (unsigned long long)(clock64() - t_begin));
-      atomicAdd(g_dbg_cycles + 8, w_tf);
-      atomicAdd(g_dbg_cycles + 9, w_bias);
-      atomicAdd(g_dbg_cycles + 10, w_ld);
-      atomicAdd(g_dbg_cycles + 11, w_try);
-    }
   }
 
   // teardown: everything issued has been consumed (epilogue waited on the last tmem_full)
   tc_fence_before();
-  if (CLUSTER > 1) cluster_sync_all(); else __syncthreads();
-  if (warp == kWarpAlloc) {
-    if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
-  }
+  __syncthreads();
+  if (warp == kWarpAlloc)
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols) : "memory");
 }
 
 // ------------------------------------------------------------------------------------------
@@ -843,9 +721,7 @@ __device__ __forceinline__ void convert_rows16(const T* __restrict__ x, int64_t 
   }
 }
 
-template <bool WAIT = true>
 __device__ __forceinline__ float chunk_min16(const uint32_t (&r)[16]) {
-  if (WAIT) tmem_ld_wait();
   float cm[4];
 #pragma unroll
   for (int c = 0; c < 4; ++c)
@@ -854,25 +730,24 @@ __device__ __forceinline__ float chunk_min16(const uint32_t (&r)[16]) {
   return fminf(min3f(cm[0], cm[1], cm[2]), cm[3]);
 }
 
-// DRAIN: an epilogue warp first copies its whole 64-column quarter of the accumulator into registers and hands the
-// TMEM buffer back, THEN ranks from the registers.  The buffer is then held for ~150 cycles instead of the whole
-// epilogue of the tile, so the next-but-one tile's MMAs (and the barrier round trips around them) overlap the ranking:
-// with the chunk-by-chunk form the epilogue warps of a d = 64 search waited for `tmem_full` a third of the time and
-// the MMA warp for `tmem_empty` 63 % of it (ncu source page / cycle counters), each side waiting for the other's
+// The epilogue DRAINS: an epilogue warp first copies its whole 64-column quarter of the accumulator into registers and
+// hands the TMEM buffer back, THEN ranks from the registers.  The buffer is then held for ~150 cycles instead of the
+// whole epilogue of the tile, so the next-but-one tile's MMAs (and the barrier round trips around them) overlap the
+// ranking: with a chunk-by-chunk form the epilogue warps of a d = 64 search waited for `tmem_full` a third of the time
+// and the MMA warp for `tmem_empty` 63 % of it (ncu source page / cycle counters), each side waiting for the other's
 // latency.  Costs 64 live accumulator registers: 18 warps (the TMA warp also allocates TMEM and writes the zero
 // chunk) x 32 x 112 registers.
-constexpr int kThreadsDrain = 576;
+constexpr int kThreadsAug = 576;
 constexpr int kThreadsConv = 640;      // + two converter warps (18, 19)
-template <bool DRAIN, bool CONV = false>
-__global__ void __launch_bounds__(CONV ? kThreadsConv : (DRAIN ? kThreadsDrain : kThreads), 1)
+template <bool CONV>
+__global__ void __launch_bounds__(CONV ? kThreadsConv : kThreadsAug, 1)
 search_aug_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_c,
                   const __grid_constant__ CUtensorMap map_xa, const __grid_constant__ CUtensorMap map_ca,
                   const AugParams P) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  constexpr int kWarpTma = DRAIN ? 16 : vqb::kWarpTma, kWarpMma = DRAIN ? 17 : vqb::kWarpMma;
-  constexpr int kWarpAlloc = DRAIN ? 16 : vqb::kWarpAlloc, kWarpStager = DRAIN ? 16 : vqb::kWarpStager;
+  constexpr int kWarpTma = 16, kWarpMma = 17, kWarpAlloc = 16, kWarpStager = 16;
   const uint32_t smem_base = smem_u32(smem);
   const uint32_t a_base = smem_base;
   const uint32_t b_base = smem_base + (uint32_t)P.KB * kSlabBytes;
@@ -1109,14 +984,8 @@ search_aug_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_consta
     const float INF = __int_as_float(0x7f800000);
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16) + quarter * 64;
     const float tconst = __uint_as_float(P.scal[6]) * (2.f + kPackSlackTC);
-    uint32_t rA[16], rB[16];                 // chunk-by-chunk form: two alternating register sets
-    uint32_t rD[DRAIN ? 4 : 1][16];          // DRAIN form: the whole 64-column quarter
+    uint32_t rD[4][16];                      // the whole 64-column quarter
     uint32_t tile_it = 0;
-    if (!DRAIN && cid < G) {
-      mbar_wait(smem_u32(&bars->tmem_full[0]), 0);
-      tc_fence_after();
-      TMEM_LD16(lane_addr, rA);
-    }
     for (int g = cid; g < G; g += num_clusters) {
       const int h = g / P.GPH;
       const int mt = (g - h * P.GPH) * 2 + (int)rank;
@@ -1155,83 +1024,47 @@ search_aug_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_consta
         bool any_slow = false;
 #pragma unroll
         for (int par = 0; par < 2; ++par) {
-          if (DRAIN) {
-            if (nt + par < P.NT) {
-              const uint32_t taddr = lane_addr + acc * (uint32_t)kBlockN;
-              mbar_wait(smem_u32(&bars->tmem_full[acc]), acc_ph);
-              if (CONV && nt == 0 && par == 0) {
-                const volatile float* vx = P.xinv;
-                const volatile float* vn = P.xn2;
-                inv = row < P.N ? fabsf(vx[(size_t)h * P.N + row]) * P.chdr[h * kHdrFloats + 1] : 0.f;
-                trow = inv > 0.f ? (tconst + P.tie * vn[(size_t)h * P.N + row]) / inv : 0.f;
-              }
-#ifdef VQB_TRACE
-              const int tr_t = (int)(tile_it - 1) * P.NT + nt + par;
-              const bool tr_on = cid == 0 && lane == 0;
-              const int tr_w = (int)rank * 16 + warp;
-              if (tr_on) VQB_STAMP_EPI(0, tr_w, tr_t);
-#endif
-              tc_fence_after();
-              TMEM_LD16(taddr, rD[0]);
-              TMEM_LD16(taddr + 16, rD[DRAIN ? 1 : 0]);
-              TMEM_LD16(taddr + 32, rD[DRAIN ? 2 : 0]);
-              TMEM_LD16(taddr + 48, rD[DRAIN ? 3 : 0]);
-              tmem_ld_wait();
-              tc_fence_before();
-              __syncwarp();
-              if (lane == 0) mbar_arrive_leader(smem_u32(&bars->tmem_empty[acc]));   // buffer handed back: rank from registers
-#ifdef VQB_TRACE
-              if (tr_on) VQB_STAMP_EPI(1, tr_w, tr_t);
-#endif
-              if (++acc == 2) { acc = 0; acc_ph ^= 1u; }
-              float cmin;
-#define VQB_DRAIN_CHUNK(CH)                                                                                 \
-              cmin = chunk_min16<false>(rD[DRAIN ? (CH) : 0]);                                              \
-              if (par == 0) chunk_rank<0, (CH), 0>(reinterpret_cast<float(&)[16]>(rD[DRAIN ? (CH) : 0]), cmin, idmask, \
-                                                   trow, m_run, t_run, row_slot, a1, a2, any_slow, 0);      \
-              else chunk_rank<1, (CH), 0>(reinterpret_cast<float(&)[16]>(rD[DRAIN ? (CH) : 0]), cmin, idmask, trow,   \
-                                          m_run, t_run, row_slot, a1, a2, any_slow, 0);
-              VQB_DRAIN_CHUNK(0) VQB_DRAIN_CHUNK(1) VQB_DRAIN_CHUNK(2) VQB_DRAIN_CHUNK(3)
-#undef VQB_DRAIN_CHUNK
-#ifdef VQB_TRACE
-              if (tr_on) VQB_STAMP_EPI(2, tr_w, tr_t);
-#endif
-            }
-          } else if (nt + par < P.NT) {
+          if (nt + par < P.NT) {
             const uint32_t taddr = lane_addr + acc * (uint32_t)kBlockN;
-            float cmin;
-            // the accumulator registers ARE the keys: two register sets alternate so that the next chunk's
-            // tcgen05.ld is in flight while this chunk is ranked
-#define VQB_AUG_CHUNK(CH, RCUR, RNEXT)                                                                      \
-            cmin = chunk_min16<true>(RCUR);                                                                 \
-            TMEM_LD16(taddr + ((CH) + 1) * 16, RNEXT);                                                      \
-            if (par == 0) chunk_rank<0, (CH), 0>(reinterpret_cast<float(&)[16]>(RCUR), cmin, idmask, trow, m_run, \
-                                                 t_run, row_slot, a1, a2, any_slow, 0);                     \
-            else chunk_rank<1, (CH), 0>(reinterpret_cast<float(&)[16]>(RCUR), cmin, idmask, trow, m_run, t_run,  \
-                                        row_slot, a1, a2, any_slow, 0);
-            VQB_AUG_CHUNK(0, rA, rB) VQB_AUG_CHUNK(1, rB, rA) VQB_AUG_CHUNK(2, rA, rB)
-#undef VQB_AUG_CHUNK
-            cmin = chunk_min16<true>(rB);
+            mbar_wait(smem_u32(&bars->tmem_full[acc]), acc_ph);
+            if (CONV && nt == 0 && par == 0) {
+              const volatile float* vx = P.xinv;
+              const volatile float* vn = P.xn2;
+              inv = row < P.N ? fabsf(vx[(size_t)h * P.N + row]) * P.chdr[h * kHdrFloats + 1] : 0.f;
+              trow = inv > 0.f ? (tconst + P.tie * vn[(size_t)h * P.N + row]) / inv : 0.f;
+            }
+#ifdef VQB_TRACE
+            const int tr_t = (int)(tile_it - 1) * P.NT + nt + par;
+            const bool tr_on = cid == 0 && lane == 0;
+            const int tr_w = (int)rank * 16 + warp;
+            if (tr_on) VQB_STAMP_EPI(0, tr_w, tr_t);
+#endif
+            tc_fence_after();
+            TMEM_LD16(taddr, rD[0]);
+            TMEM_LD16(taddr + 16, rD[1]);
+            TMEM_LD16(taddr + 32, rD[2]);
+            TMEM_LD16(taddr + 48, rD[3]);
+            tmem_ld_wait();
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive_leader(smem_u32(&bars->tmem_empty[acc]));
+            if (lane == 0) mbar_arrive_leader(smem_u32(&bars->tmem_empty[acc]));   // buffer handed back: rank from registers
+#ifdef VQB_TRACE
+            if (tr_on) VQB_STAMP_EPI(1, tr_w, tr_t);
+#endif
             if (++acc == 2) { acc = 0; acc_ph ^= 1u; }
-            const bool more = (nt + par + 1 < P.NT) || (g + num_clusters < G);
-            bool issued = false;
-            if (more && mbar_try(smem_u32(&bars->tmem_full[acc]), acc_ph)) {
-              tc_fence_after();
-              TMEM_LD16(lane_addr + acc * (uint32_t)kBlockN, rA);
-              issued = true;
-            }
-            if (par == 0) chunk_rank<0, 3, 0>(reinterpret_cast<float(&)[16]>(rB), cmin, idmask, trow, m_run, t_run,
-                                              row_slot, a1, a2, any_slow, 0);
-            else chunk_rank<1, 3, 0>(reinterpret_cast<float(&)[16]>(rB), cmin, idmask, trow, m_run, t_run, row_slot,
-                                     a1, a2, any_slow, 0);
-            if (more && !issued) {
-              mbar_wait(smem_u32(&bars->tmem_full[acc]), acc_ph);
-              tc_fence_after();
-              TMEM_LD16(lane_addr + acc * (uint32_t)kBlockN, rA);
-            }
+            float cmin;
+            // the accumulator registers ARE the keys
+#define VQB_RANK_CHUNK(CH)                                                                                  \
+            cmin = chunk_min16(rD[CH]);                                                                     \
+            if (par == 0) chunk_rank<0, (CH)>(reinterpret_cast<float(&)[16]>(rD[CH]), cmin, idmask, trow, m_run, \
+                                              t_run, row_slot, a1, a2, any_slow);                           \
+            else chunk_rank<1, (CH)>(reinterpret_cast<float(&)[16]>(rD[CH]), cmin, idmask, trow, m_run, t_run,   \
+                                     row_slot, a1, a2, any_slow);
+            VQB_RANK_CHUNK(0) VQB_RANK_CHUNK(1) VQB_RANK_CHUNK(2) VQB_RANK_CHUNK(3)
+#undef VQB_RANK_CHUNK
+#ifdef VQB_TRACE
+            if (tr_on) VQB_STAMP_EPI(2, tr_w, tr_t);
+#endif
           }
         }
         if (!any_slow) continue;
@@ -1302,35 +1135,37 @@ static int make_map(CUtensorMap* m, const void* base, int inner, int64_t rows, i
   return VQB_OK;
 }
 
-static int g_cluster_override = -1;   // env VQB_CLUSTER: 1, 2 (multicast) or 3 (pair MMA)
-constexpr int kDefaultMode = 3;   // cta_group::2 pair MMA: measured fastest on B200 for d >= 256, equal at d = 64
-
 // timing ring for VQB_SEARCH_TIMING: event pairs recorded on the search stream around the kernel launch
 constexpr int kTimingSlots = 64;
 static cudaEvent_t g_ev0[kTimingSlots], g_ev1[kTimingSlots];
 static bool g_ev_made = false;
 static int g_ev_dev = -1;              // the events belong to the device of the first timed search
 static int g_ev_count = 0;
+static int g_num_sms = 0;              // SMs of the device of the first search: one CTA per SM
 
-template <int CLUSTER, bool PAIR, int MODE>
-static int launch_impl(const CUtensorMap& mx, const CUtensorMap& mc, const SearchParams& P, size_t smem_bytes,
-                       int grid, bool timing, cudaStream_t st) {
+// Launches a persistent search kernel: clusters of `cluster` CTAs, one CTA per SM but no more clusters than the G
+// work items, 227 KB of dynamic shared memory allowed; `timing` brackets the launch with an event pair of the ring.
+template <auto Kernel, typename... Args>
+static int launch_search_kernel(int cluster, int G, int threads, size_t smem_bytes, bool timing, cudaStream_t st,
+                                const Args&... args) {
   static bool configured[64] = {};      // function attributes are per device
   int dev = 0;
   VQB_CUDA_TRY(cudaGetDevice(&dev));
   if (dev < 0 || dev >= 64 || !configured[dev]) {
-    VQB_CUDA_TRY(cudaFuncSetAttribute(search_tc_kernel<CLUSTER, PAIR, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      227 * 1024));
+    VQB_CUDA_TRY(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     if (dev >= 0 && dev < 64) configured[dev] = true;
   }
+  if (!g_num_sms) VQB_CUDA_TRY(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
+  int nclusters = g_num_sms / cluster;
+  if (nclusters > G) nclusters = G;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(kThreads);
+  cfg.gridDim = dim3((unsigned)(nclusters * cluster));
+  cfg.blockDim = dim3(threads);
   cfg.dynamicSmemBytes = smem_bytes;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CLUSTER;
+  attr[0].val.clusterDim.x = cluster;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
@@ -1348,42 +1183,17 @@ static int launch_impl(const CUtensorMap& mx, const CUtensorMap& mc, const Searc
     if (g_ev_count < kTimingSlots) slot = g_ev_count++;
   }
   if (slot >= 0) VQB_CUDA_TRY(cudaEventRecord(g_ev0[slot], st));
-  VQB_CUDA_TRY(cudaLaunchKernelEx(&cfg, search_tc_kernel<CLUSTER, PAIR, MODE>, mx, mc, P));
+  VQB_CUDA_TRY(cudaLaunchKernelEx(&cfg, Kernel, args...));
   ++g_launch_count;
   if (slot >= 0) VQB_CUDA_TRY(cudaEventRecord(g_ev1[slot], st));
   return VQB_OK;
 }
 
-static int aug_env() {   // env VQB_AUG=0: bias added in the epilogue (the first version of the kernel), for A/B runs
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("VQB_AUG"); v = e ? atoi(e) : 1; }
-  return v;
-}
-static int mode_env() {
-  if (g_cluster_override < 0) {
-    const char* e = getenv("VQB_CLUSTER");
-    g_cluster_override = e ? atoi(e) : 0;
-  }
-  return g_cluster_override;
-}
-static int dbg_env() {
-  static int dbg = -1;
-  if (dbg < 0) { const char* e = getenv("VQB_TC_DEBUG"); dbg = e ? atoi(e) : 0; }
-  return dbg;
-}
-
-// the bias k-step needs the pair kernel (>= 2 row tiles) and no bring-up knob / alternate mode requested
-// returns 0: bias in the epilogue (first kernel); 1: bias k-step; 2: no bias at all (dot metric, no padded codes)
+// 0: one row tile per codebook, bias added in the epilogue (search_tc_kernel); 1: search_aug_kernel with the bias
+// k-step; 2: search_aug_kernel without any bias (dot metric, no padded codes).  The pair kernel needs >= 2 row tiles.
 int search_tc_aug_mode(int64_t N, int K, int metric) {
-  const int mode = mode_env();
-  if (aug_env() == 0 || dbg_env() != 0 || (mode >= 1 && mode <= 2) || (N + kBlockM - 1) / kBlockM < 2) return 0;
+  if ((N + kBlockM - 1) / kBlockM < 2) return 0;
   return (metric == VQB_DOT && K % kBlockN == 0) ? 2 : 1;
-}
-
-static int drain_env() {     // env VQB_DRAIN=0: chunk-by-chunk epilogue (the TMEM buffer is held while it is ranked)
-  static int drain = -1;
-  if (drain < 0) { const char* e = getenv("VQB_DRAIN"); drain = e ? atoi(e) : 1; }
-  return drain;
 }
 
 // In-kernel conversion of 16-bit latents (CONV, opt-in: VQB_SEARCH_FUSED_PREP): the two converter warps keep up when
@@ -1395,7 +1205,7 @@ int search_tc_conv_ok(int64_t N, int K, int d, int x_dtype, int aug_mode, int re
   if (env == -2) { const char* e = getenv("VQB_FUSED_PREP"); env = e ? atoi(e) : -1; }
   const int on = env >= 0 ? env : (requested ? 1 : 0);
   if (on == 2) return 2;
-  if (!on || !aug_mode || !drain_env() || x_dtype == VQB_F32 || (d & 7) || d > 256) return 0;
+  if (!on || !aug_mode || x_dtype == VQB_F32 || (d & 7) || d > 256) return 0;
   const int dp = d_pad(d);
   const int64_t work = (int64_t)(k_pad(K) / kBlockN) * (dp / kBlockK);       // MMA k-blocks per row tile
   return (work >= 96 && N >= 64 * kBlockM) ? 1 : 0;
@@ -1406,21 +1216,6 @@ static int launch_aug(const __half* xb, const float* xinv, const float* xn2, flo
                       const float* chdr, int64_t H, int64_t N, int K, int dp, int aug_on, void* cand, uint32_t* scal,
                       bool timing, cudaStream_t st, const ConvArgs& conv) {
   const int Kp = k_pad(K);
-  static int num_sms = 0;
-  int dev = 0;
-  VQB_CUDA_TRY(cudaGetDevice(&dev));
-  if (!num_sms) VQB_CUDA_TRY(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
-  static bool configured[64] = {};
-  if (dev < 0 || dev >= 64 || !configured[dev]) {
-    VQB_CUDA_TRY(cudaFuncSetAttribute(search_aug_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    VQB_CUDA_TRY(cudaFuncSetAttribute(search_aug_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    VQB_CUDA_TRY(cudaFuncSetAttribute(search_aug_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      227 * 1024));
-    if (dev >= 0 && dev < 64) configured[dev] = true;
-  }
-  const int drain = drain_env();
-  const bool do_conv = conv.x != nullptr;
-  VQB_REQUIRE(!do_conv || drain, VQB_ERR_INVALID, "in-kernel latent conversion needs the draining epilogue");
   AugParams P;
   P.xraw = conv.x; P.xdtype = conv.x_dtype; P.d = conv.d; P.dp = dp; P.xb_w = xb; P.xaug_w = xaug;
   P.xinv = xinv; P.xn2 = xn2; P.tie = tie; P.chdr = chdr; P.cand = cand; P.scal = scal; P.N = N; P.Kp = Kp;
@@ -1437,8 +1232,6 @@ static int launch_aug(const __half* xb, const float* xinv, const float* xn2, flo
   P.GPH = (MT + 1) / 2;
   const size_t smem_bytes = fixed + (size_t)S * kStageStrideAug;
   const int G = (int)H * P.GPH;
-  int nclusters = num_sms / 2;
-  if (nclusters > G) nclusters = G;
   CUtensorMap mx, mc, mxa, mca;
   int rc = make_map(&mx, xb, dp, N, H, kBlockM);
   if (rc) return rc;
@@ -1448,37 +1241,9 @@ static int launch_aug(const __half* xb, const float* xinv, const float* xn2, flo
   if (rc) return rc;
   rc = make_map(&mca, caug, 8, Kp, H, kBlockN / 2, 8);
   if (rc) return rc;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(nclusters * 2));
-  cfg.blockDim = dim3(do_conv ? kThreadsConv : (drain ? kThreadsDrain : kThreads));
-  cfg.dynamicSmemBytes = smem_bytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  int slot = -1;
-  if (timing && (g_ev_dev < 0 || g_ev_dev == dev)) {
-    if (!g_ev_made) {
-      g_ev_dev = dev;
-      for (int i = 0; i < kTimingSlots; ++i) {
-        VQB_CUDA_TRY(cudaEventCreate(&g_ev0[i]));
-        VQB_CUDA_TRY(cudaEventCreate(&g_ev1[i]));
-      }
-      g_ev_made = true;
-    }
-    if (g_ev_count < kTimingSlots) slot = g_ev_count++;
-  }
-  if (slot >= 0) VQB_CUDA_TRY(cudaEventRecord(g_ev0[slot], st));
-  if (do_conv) VQB_CUDA_TRY(cudaLaunchKernelEx(&cfg, search_aug_kernel<true, true>, mx, mc, mxa, mca, P));
-  else if (drain) VQB_CUDA_TRY(cudaLaunchKernelEx(&cfg, search_aug_kernel<true>, mx, mc, mxa, mca, P));
-  else VQB_CUDA_TRY(cudaLaunchKernelEx(&cfg, search_aug_kernel<false>, mx, mc, mxa, mca, P));
-  ++g_launch_count;
-  if (slot >= 0) VQB_CUDA_TRY(cudaEventRecord(g_ev1[slot], st));
-  return VQB_OK;
+  if (conv.x != nullptr)
+    return launch_search_kernel<search_aug_kernel<true>>(2, G, kThreadsConv, smem_bytes, timing, st, mx, mc, mxa, mca, P);
+  return launch_search_kernel<search_aug_kernel<false>>(2, G, kThreadsAug, smem_bytes, timing, st, mx, mc, mxa, mca, P);
 }
 
 int launch_search_tc(const __half* xb, const float* xinv, const float* xn2, float tie, const __half* xaug,
@@ -1496,61 +1261,25 @@ int launch_search_tc(const __half* xb, const float* xinv, const float* xn2, floa
   }
   VQB_REQUIRE(dp % kBlockK == 0 && dp / kBlockK <= kMaxKB, VQB_ERR_UNSUPPORTED, "d_pad %d unsupported by the TC path", dp);
   VQB_REQUIRE(N < (1ll << 31) - kBlockM, VQB_ERR_UNSUPPORTED, "N too large for TMA coordinates");
-  static int num_sms = 0;
-  if (!num_sms) {
-    int dev = 0;
-    VQB_CUDA_TRY(cudaGetDevice(&dev));
-    VQB_CUDA_TRY(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
-  }
-  mode_env();
-  const int MT = (int)((N + kBlockM - 1) / kBlockM);
-  // VQB_CLUSTER: 1 = independent CTAs, 2 = 2-CTA TMA multicast of B (measured: not faster, L2 is not the limiter),
-  // 3 = cta_group::2 pair MMA (each CTA holds half of B).  Default: see below.
-  int mode = g_cluster_override >= 1 && g_cluster_override <= 3 ? g_cluster_override : kDefaultMode;
-  if (MT < 2) mode = 1;
-  const bool pair = mode == 3;
-  const int cluster = mode == 1 ? 1 : 2;
-
   SearchParams P;
   P.bias = bias; P.xinv = xinv; P.xn2 = xn2; P.tie = tie; P.chdr = chdr; P.cand = cand; P.scal = scal; P.N = N;
   P.Kp = Kp; P.H = (int)H;
-  P.dbg = dbg_env();
   P.KB = dp / kBlockK;
   P.NT = Kp / kBlockN;
-  const size_t stage_bytes = pair ? kStageBytes / 2 : kStageBytes;     // per CTA
   const size_t fixed = (size_t)P.KB * kSlabBytes + sizeof(Barriers);
-  int S = (int)((227 * 1024 - fixed) / stage_bytes);
+  int S = (int)((227 * 1024 - fixed) / kStageBytes);
   if (S > kMaxStages) S = kMaxStages;
   VQB_REQUIRE(S >= 2, VQB_ERR_UNSUPPORTED, "not enough shared memory for d_pad=%d", dp);
   P.S = S;
-  P.GPH = (MT + cluster - 1) / cluster;
-  const size_t smem_bytes = fixed + (size_t)S * stage_bytes;
-  const int G = (int)H * P.GPH;
-  int nclusters = num_sms / cluster;
-  if (nclusters > G) nclusters = G;
-  const int grid = nclusters * cluster;
+  P.MT = (int)((N + kBlockM - 1) / kBlockM);
+  const size_t smem_bytes = fixed + (size_t)S * kStageBytes;
 
   CUtensorMap mx, mc;
   int rc = make_map(&mx, xb, dp, N, H, kBlockM);
   if (rc) return rc;
-  rc = make_map(&mc, cb, dp, Kp, H, kBlockN / cluster);
+  rc = make_map(&mc, cb, dp, Kp, H, kBlockN);
   if (rc) return rc;
-#define VQB_LAUNCH_MODE(C, PR)                                                                         \
-  (P.dbg == 0 ? launch_impl<C, PR, 0>(mx, mc, P, smem_bytes, grid, timing, st)                         \
-              : launch_impl<C, PR, 1>(mx, mc, P, smem_bytes, grid, timing, st))
-  if (pair) return VQB_LAUNCH_MODE(2, true);
-  if (cluster == 2) return VQB_LAUNCH_MODE(2, false);
-  return VQB_LAUNCH_MODE(1, false);
-#undef VQB_LAUNCH_MODE
-}
-
-int debug_counters(unsigned long long* out18) {   // [0..1] ranked/skipped chunks, [2..17] cycle counters
-  VQB_CUDA_TRY(cudaMemcpyFromSymbol(out18, g_dbg_counters, 16));
-  VQB_CUDA_TRY(cudaMemcpyFromSymbol(out18 + 2, g_dbg_cycles, 128));
-  unsigned long long z[16] = {0};
-  VQB_CUDA_TRY(cudaMemcpyToSymbol(g_dbg_counters, z, 16));
-  VQB_CUDA_TRY(cudaMemcpyToSymbol(g_dbg_cycles, z, 128));
-  return VQB_OK;
+  return launch_search_kernel<search_tc_kernel>(1, (int)H * P.MT, kThreads, smem_bytes, timing, st, mx, mc, P);
 }
 
 int search_timing(float* host_ms, int cap) {
@@ -1574,5 +1303,3 @@ extern "C" int vqb_debug_trace(long long* mma, long long* epi) {   // [3][kTrace
 }
 #endif
 extern "C" int vqb_search_timing(float* host_ms, int cap) { return vqb::search_timing(host_ms, cap); }
-// bring-up aid, not part of include/vqb.h
-extern "C" int vqb_debug_counters(unsigned long long* out2) { return vqb::debug_counters(out2); }
