@@ -1,7 +1,7 @@
 """f4 variants (gumbel sampling, affine re-parametrisation, orthogonal regularisation, materialised similarities): the
-product's host logic -- `Codebook._run_variants`, the VectorQuantize / ResidualVQ glue -- on CPU with the plain-torch
-statements of the C entry points (tests/cpu_kernels.py), against the fixtures recorded from the live reference
-(tests/golden/make_golden_f4.py).  The kernels behind the entry points are tested on the GPU (test_gpu_f4.py)."""
+product's host logic -- `Codebook._run` with the variants on, the VectorQuantize / ResidualVQ glue -- on CPU with the
+plain-torch statements of the C entry points (tests/cpu_kernels.py), against the fixtures recorded from the live
+reference (tests/golden/make_golden_f4.py).  The kernels behind the entry points are tested on the GPU (test_gpu_f4.py)."""
 import pytest
 import torch
 

@@ -2,9 +2,10 @@
 
 The tensor-level wrappers of `vqb200.ops` are replaced by plain-torch statements of their C entry points
 (tests/cpu_kernels.py), and the two rotation-trick backward ops by the statements below, which also count their calls.
-The checks: the flag reaches `_QuantizeST.backward` from `Codebook._run`, `_run_variants` (gumbel straight-through,
-affine) and `_run_sharded` (two Gloo ranks), and `_FusedRVQ.backward` / the generic level loop of ResidualVQ; with the
-flag off neither op is called.  The kernels themselves are tested on the GPU (tests/test_gpu_rotation_trick.py)."""
+The checks: the flag reaches `_QuantizeST.backward` from `Codebook._run` on the plain path, with the variants (gumbel
+straight-through, affine) and on a sharded codebook (two Gloo ranks), and `_FusedRVQ.backward` / the generic level
+loop of ResidualVQ; with the flag off neither op is called.  The kernels themselves are tested on the GPU
+(tests/test_gpu_rotation_trick.py)."""
 import datetime
 import os
 import socket

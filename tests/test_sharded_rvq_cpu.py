@@ -1,7 +1,7 @@
 """world_size-2 Gloo tests (CPU) of a ResidualVQ over SHARDED codebooks and of the codebook accessors on shards, through
 the product's orchestration with the tensor-level wrappers replaced by plain-torch statements (tests/cpu_kernels.py).
 
-A sharded level must take the generic per-level loop (`VectorQuantize` -> `Codebook._run_sharded`): the fused level
+A sharded level must take the generic per-level loop (`VectorQuantize` -> `Codebook._run` on shards): the fused level
 kernels search and update one whole codebook.  The accessors (`VectorQuantize.codebook`, `get_codes_from_indices`,
 `ResidualVQ.codebooks`) speak in global code ids, so they read the full codebook, and the `codebook` setter takes the
 full codebook and keeps this rank's rows."""

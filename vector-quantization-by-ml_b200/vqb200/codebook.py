@@ -6,7 +6,7 @@ the numeric work (search, gather, EMA statistics, refresh, expiry scatter) runs 
 libvqb200.so.  ``learnable_codebook=True`` makes ``embeddings`` a Parameter that receives the gradient
 of the commitment loss / of the gathered codes (a segmented sum over the rows of each code).
 
-Variants off the named hot path take `_run_variants` (same kernels, no fused passes):
+Variants off the named hot path run through the same `_run` with the fused passes off:
   * gumbel sampling (reference utils/general.py:107-151, codebooks.py:388): `stochastic` = argmax of
     similarities / temperature + gumbel noise as an epilogue of the tiled fp32 score pass (vqb_dense_gumbel_sample;
     the noise is generated in the kernel from torch's Philox stream, no N x K tensor exists);
@@ -200,25 +200,34 @@ class Codebook(nn.Module):
     # ------------------------------------------------------------------ kmeans init (reference utils/kmeans.py)
     @torch.no_grad()
     def _kmeans_init(self, flat: torch.Tensor, mask_u8: Optional[torch.Tensor]) -> None:
+        """reference utils/kmeans.py:38-120.  On a sharded codebook rank 0's draw picks the K start rows (all ranks hold
+        the same latents) and every iteration is a sharded search + segment means on the owned rows."""
+        from . import distributed as D
         H, N, d = flat.shape
         K = self.codebook_size
         data = flat.float()
         if mask_u8 is not None:
-            keep = mask_u8.bool()
-            data = data[:, keep].contiguous()
+            data = data[:, mask_u8.bool()].contiguous()
             N = data.shape[1]
         iters = int((self.kmeans_params or {"iter": 10})["iter"])
-        sync = self.use_ddp and self._kmeans_sync
-        from . import distributed as D
-        if sync and D.is_distributed():      # reference codebooks.py:164-168: identical centroids on every rank
-            cents = torch.stack([D.sample_vectors_distributed(data[h], K, self._draw_rows) for h in range(H)], 0)
+        sync = self.use_ddp and self._kmeans_sync and not self.sharded
+        if self.sharded:
+            lo, Ks = self.shard_offset, self.shard_size
+            cents = [data[h][D.broadcast_from_rank0(self._draw_rows(N, K, data.device).to(torch.long))[lo:lo + Ks]]
+                     for h in range(H)]
+        elif sync and D.is_distributed():    # reference codebooks.py:164-168: identical centroids on every rank
+            cents = [D.sample_vectors_distributed(data[h], K, self._draw_rows) for h in range(H)]
         else:
-            cents = torch.stack([data[h][self._draw_rows(N, K, data.device)] for h in range(H)], 0).contiguous()
-        counts = torch.zeros(H, K, device=data.device)
+            cents = [data[h][self._draw_rows(N, K, data.device)] for h in range(H)]
+        cents = torch.stack(cents, 0).contiguous()
+        counts = torch.zeros(H, self.shard_size, device=data.device)
         for _ in range(iters):
             cache = ops.prepare_codebook(cents, self.use_cosine_sim)
-            idx, _, ws = ops.search(data, cents, cache, self.use_cosine_sim)
-            stats = ops.ema_reduce(data, idx, None, K, bound_ws=ws)
+            if self.sharded:
+                stats = self._shard_stats(data, self._shard_search(data, cents, cache), None)
+            else:
+                idx, _, ws = ops.search(data, cents, cache, self.use_cosine_sim)
+                stats = ops.ema_reduce(data, idx, None, K, bound_ws=ws)
             counts = stats[..., d].clone()
             if sync:
                 self._all_reduce(counts)
@@ -233,6 +242,22 @@ class Codebook(nn.Module):
         self.embeddings.data.copy_(cents)
         self.embed_avg.data.copy_(cents * counts[..., None])
         self.cluster_size.data.copy_(counts)
+        self._dirty = self._replica_dirty = True
+
+    # ------------------------------------------------------------------ EMA refresh
+    def _apply_ema(self, stats: torch.Tensor) -> None:
+        """Refresh the buffers from one step's statistics (H, K, d+1), already all-reduced under data parallel; on a
+        shard, the statistics of this rank's codes.  No host sync: ResidualVQ's fused level loop calls this inside a
+        CUDA graph."""
+        if self.sharded:
+            from . import distributed as D
+            ops.ema_apply_sharded(stats, self.cluster_size.data, self.embed_avg.data, self.embeddings.data,
+                                  1 - self.decay, self.eps_for_smoothing, self.weights_l2norm, self.codebook_size,
+                                  D.all_reduce_sum)
+            self._replica_dirty = True
+        else:
+            ops.ema_apply(stats, self.cluster_size.data, self.embed_avg.data, self.embeddings.data, 1 - self.decay,
+                          self.eps_for_smoothing, self.weights_l2norm)
         self._dirty = True
 
     # ------------------------------------------------------------------ expiry (reference codebooks.py:230-255)
@@ -325,40 +350,15 @@ class Codebook(nn.Module):
         gidx, _ = ops.minkey_unpack(keys)
         return gidx.reshape(H, N)
 
-    @torch.no_grad()
-    def _kmeans_init_sharded(self, flat: torch.Tensor, mask_u8: Optional[torch.Tensor]) -> None:
-        """reference utils/kmeans.py:38-120 on a row-sharded set of K centroids: rank 0's draw picks the K start rows
-        (all ranks hold the same latents), every iteration is a sharded search + segment means on the owned rows."""
-        from . import distributed as D
-        H, N, d = flat.shape
-        data = flat.float()
-        if mask_u8 is not None:
-            data = data[:, mask_u8.bool()].contiguous()
-            N = data.shape[1]
-        iters = int((self.kmeans_params or {"iter": 10})["iter"])
+    def _shard_stats(self, rows: torch.Tensor, gidx: torch.Tensor, mask_u8: Optional[torch.Tensor]) -> torch.Tensor:
+        """EMA statistics (H, K/W, d+1) of this rank's codes: the sums over the rows whose global code id is one of
+        them."""
         lo, Ks = self.shard_offset, self.shard_size
-        cents = []
-        for h in range(H):
-            rows = D.broadcast_from_rank0(self._draw_rows(N, self.codebook_size, data.device).to(torch.long))
-            cents.append(data[h][rows[lo:lo + Ks]])
-        cents = torch.stack(cents, 0).contiguous()
-        counts = torch.zeros(H, Ks, device=data.device)
-        for _ in range(iters):
-            cache = ops.prepare_codebook(cents, self.use_cosine_sim)
-            gidx = self._shard_search(data, cents, cache)
-            mine = (gidx >= lo) & (gidx < lo + Ks)
-            stats = torch.stack([ops.ema_reduce(data[h:h + 1], (gidx[h:h + 1] - lo).clamp_(0, Ks - 1),
-                                                mine[h].to(torch.uint8), Ks)[0] for h in range(H)], 0)
-            counts = stats[..., d].clone()
-            empty = counts == 0
-            means = stats[..., :d] / counts.masked_fill(empty, 1.0)[..., None]
-            if self.use_cosine_sim:
-                means = ops.l2norm_rows(means.contiguous())
-            cents = torch.where(empty[..., None], cents, means).contiguous()
-        self.embeddings.data.copy_(cents)
-        self.embed_avg.data.copy_(cents * counts[..., None])
-        self.cluster_size.data.copy_(counts)
-        self._dirty = self._replica_dirty = True
+        mine = (gidx >= lo) & (gidx < lo + Ks)
+        if mask_u8 is not None:
+            mine = mine & mask_u8.bool()[None]
+        return torch.stack([ops.ema_reduce(rows[h:h + 1], (gidx[h:h + 1] - lo).clamp_(0, Ks - 1),
+                                           mine[h].to(torch.uint8), Ks)[0] for h in range(rows.shape[0])], 0)
 
     @torch.no_grad()
     def _expire_codes_sharded(self, flat: torch.Tensor) -> None:
@@ -386,77 +386,6 @@ class Codebook(nn.Module):
                                    float(self.reset_cluster_size), self.weights_l2norm, self.cluster_size.data[h],
                                    self.embed_avg.data[h], self.embeddings.data[h])
         self._dirty = self._replica_dirty = True
-
-    def _run_sharded(self, x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, rotation=False):
-        """`_run` for a row-sharded codebook.  Every rank ends up with the quantised vectors / indices of ITS latents
-        (all of them when the input is replicated) and updates ITS rows of the EMA buffers from the rows they won --
-        no statistics all_reduce; the only exchanges are the min-key all_reduce, one scalar all_reduce for the Laplace
-        normaliser and the all_gather that refreshes the codebook replica the gather reads."""
-        from . import distributed as D
-        _lib.require_device(x)
-        flat, lead = self._flatten(x)
-        H, n_local, d = flat.shape
-        if H != self.num_codebooks or d != self.embeddings.shape[-1]:
-            raise ValueError(f"vqb200.Codebook: input {tuple(x.shape)} does not match codebook "
-                             f"(H={self.num_codebooks}, d={self.embeddings.shape[-1]})")
-        if torch.is_grad_enabled() and flat.requires_grad and normalize_input:
-            flat = ops.l2norm_rows_autograd(flat)
-        elif normalize_input:
-            flat = ops.l2norm_rows(flat)
-        mask_u8 = self._expand_mask(mask, n_local)
-        gathered = self.sharded_input == "all_gather"
-        rows_all, mask_all = flat.detach(), mask_u8
-        if gathered:
-            rows_all = D.all_gather_rows(flat.detach(), dim=1)
-            if mask_u8 is not None:
-                mask_all = D.all_gather_rows(mask_u8, dim=0)
-        N = rows_all.shape[1]
-        if not self.is_initialized:
-            self._kmeans_init_sharded(rows_all, mask_all)
-            self.is_initialized = True
-
-        gidx_all = self._shard_search(rows_all, self.embeddings.detach(), self._codebook_cache())
-        replica = self.full_codebook()
-        training = self.training
-        update = training and self.ema_update and not freeze_codebook
-        if torch.is_grad_enabled() and flat.requires_grad:
-            replica = replica.clone()          # backward reads the codes of this forward (see _run)
-        lo_r = self.shard_rank * n_local if gathered else 0
-        gidx = gidx_all[:, lo_r:lo_r + n_local] if gathered else gidx_all
-        commit = None
-        stats_full = None
-        whole = update and not gathered and mask_u8 is None and self.fused_quantize_ema and ops.quantize_ema_supported(d)
-        if whole and fuse_st:
-            # replicated input: gather/ST/loss over all rows and the EMA sums of ALL codes in one pass; this rank
-            # keeps the statistics of its own rows of the codebook
-            quant, commit, stats_full = ops.quantize_training(flat, replica, gidx, None, want_commit, ema=True,
-                                                              bound_ws=self.last_search_ws, rotation=rotation)
-        elif whole:
-            with torch.no_grad():
-                quant, _, stats_full = ops.quantize_ema(flat, replica, gidx, False, False, bound_ws=self.last_search_ws)
-        elif fuse_st and training:
-            quant, commit, _ = ops.quantize_training(flat, replica, gidx.contiguous(), mask_u8, want_commit,
-                                                     rotation=rotation)
-        else:
-            with torch.no_grad():
-                quant, _ = ops.gather_st_loss(flat, replica, gidx.contiguous(), None, False, False)
-        if update:
-            with torch.no_grad():
-                lo, Ks = self.shard_offset, self.shard_size
-                if stats_full is not None:
-                    stats = stats_full[:, lo:lo + Ks].contiguous()
-                else:
-                    mine = (gidx_all >= lo) & (gidx_all < lo + Ks)
-                    if mask_all is not None:
-                        mine = mine & mask_all.bool()[None]
-                    stats = torch.stack([ops.ema_reduce(rows_all[h:h + 1], (gidx_all[h:h + 1] - lo).clamp_(0, Ks - 1),
-                                                        mine[h].to(torch.uint8), Ks)[0] for h in range(H)], 0)
-                ops.ema_apply_sharded(stats, self.cluster_size.data, self.embed_avg.data, self.embeddings.data,
-                                      1 - self.decay, self.eps_for_smoothing, self.weights_l2norm, self.codebook_size,
-                                      D.all_reduce_sum)
-                self._dirty = self._replica_dirty = True
-                self._expire_codes_sharded(rows_all)
-        return quant.reshape(H, *lead, d), gidx.reshape(H, *lead), commit
 
     # ------------------------------------------------------------------ variants: gumbel sampling, affine
     def _variant_sampling(self):
@@ -504,7 +433,8 @@ class Codebook(nn.Module):
         self._update_with_decay("batch_mean", mean.float()[:, None, :], ap["batch_decay"])
         self._update_with_decay("batch_variance", var.float()[:, None, :], ap["batch_decay"])
 
-    def _gumbel_st_quantize(self, flat: torch.Tensor, emb_g: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
+    def _gumbel_st_quantize(self, flat: torch.Tensor, emb_g: torch.Tensor, idx: torch.Tensor,
+                            mask_u8: Optional[torch.Tensor], fuse_st: bool, want_commit: bool, rotation: bool):
         """quantize = one_hot' @ embeddings with the straight-through / reinmax one-hot of reference
         utils/general.py:139-149, as torch ops under autograd (library code): only the gradient through the one-hot
         differs from a gather.  Row-chunked (bounds the size of each temporary, not the total the graph keeps);
@@ -513,7 +443,7 @@ class Codebook(nn.Module):
         which this forward's EMA step overwrites in place before backward runs -- the reference's graph has exactly that
         aliasing (its saved `embeddings.detach()` shares the buffer's storage, codebooks.py:375-377,425), so the same
         torch ops on the same alias reproduce its gradient: pre-update distances and probabilities, post-update code
-        vectors."""
+        vectors.  Returns (quantize, commit | None); with `fuse_st`, VectorQuantize's straight-through output."""
         import torch.nn.functional as F
         g = self.gumbel
         tau, K, cos = float(g["temperature"]), emb_g.shape[1], self.use_cosine_sim
@@ -536,115 +466,29 @@ class Codebook(nn.Module):
                 one_hot = one_hot + prob1 - prob1.detach()
             return torch.einsum("hnc,hcd->hnd", one_hot, e)
 
-        N = flat.shape[1]
+        H, N = idx.shape
         rows = N if g["reinmax"] else max(1, (1 << 24) // max(K, 1))
         if rows >= N:
-            return piece(flat, emb_g, idx)
-        outs = [piece(flat[:, lo:lo + rows], emb_g, idx[:, lo:lo + rows]) for lo in range(0, N, rows)]
-        return torch.cat(outs, dim=1)
-
-    def _run_variants(self, x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, keep_dense,
-                      rotation=False):
-        """`_run` with the affine re-parametrisation and / or gumbel sampling (see the module docstring): the same
-        kernels, un-fused; returns what `_run` returns."""
-        g = self.gumbel
-        assert not (g["reinmax"] and not g["straight_through"]), \
-            "reinmax can only be turned on if using straight through gumbel softmax"
-        _lib.require_device(x)
-        flat, lead = self._flatten(x)
-        H, N, d = flat.shape
-        K = self.codebook_size
-        if H != self.num_codebooks or d != self.embeddings.shape[-1]:
-            raise ValueError(f"vqb200.Codebook: input {tuple(x.shape)} does not match codebook "
-                             f"{tuple(self.embeddings.shape)}")
-        mask_u8 = self._expand_mask(mask, N)
-        if normalize_input:
-            flat = ops.l2norm_rows_autograd(flat) if (torch.is_grad_enabled() and flat.requires_grad) \
-                else ops.l2norm_rows(flat)
-        if not self.is_initialized:
-            self._kmeans_init(flat, mask_u8)
-            self.is_initialized = True
-
-        training = self.training
-        update = training and self.ema_update and not freeze_codebook
-        grad_on = torch.is_grad_enabled()
-        emb_param = self.embeddings if (self.learnable_codebook and self.commit_grad_to_codebook and training
-                                        and not freeze_codebook and grad_on and self.embeddings.requires_grad) else None
-        base = emb_param if emb_param is not None else self.embeddings.detach()
-        inv_scale = cm = bm = None
-        if self.use_affine:
-            self._update_affine(flat, mask_u8)
-            codebook_std = self.codebook_variance.clamp(min=1e-5).sqrt()
-            batch_std = self.batch_variance.clamp(min=1e-5).sqrt()
-            cm, bm, inv_scale = self.codebook_mean, self.batch_mean, codebook_std / batch_std
-            emb_eff = (base - cm) * (batch_std / codebook_std) + bm          # reference :381-384
+            q_graph = piece(flat, emb_g, idx)
         else:
-            emb_eff = base
-        emb_val = emb_eff.detach().contiguous()
-        if emb_val.data_ptr() == self.embeddings.data_ptr() and (keep_dense or (grad_on and flat.requires_grad)):
-            emb_val = emb_val.clone()          # backward reads the codes of this forward (see _run)
-        if keep_dense:
-            self.dense_ctx = ops._DenseCtx(flat, emb_val, emb_val if self.use_affine else self.embeddings,
-                                           self.use_cosine_sim)
-
-        stochastic, st = self._variant_sampling()
-        x_det = flat.detach()
-        if stochastic:
-            u = self._uniform_queue.pop(0) if self._uniform_queue else None
-            idx = ops.dense_gumbel_sample(x_det, emb_val, self.use_cosine_sim, float(g["temperature"]), uniforms=u)
-            self.last_search_ws = None
-        else:
-            cache = ops.prepare_codebook(emb_val, self.use_cosine_sim) if self.use_affine else self._codebook_cache()
-            idx, _, ws = ops.search(x_det, emb_val, cache, self.use_cosine_sim)
-            self.last_search_ws = ws
-        if self.return_similarities and not fuse_st:
-            self._sim = ops.dense_scores(x_det, emb_val, self.use_cosine_sim)
-
+            q_graph = torch.cat([piece(flat[:, lo:lo + rows], emb_g, idx[:, lo:lo + rows]) for lo in range(0, N, rows)],
+                                dim=1)
+        if not fuse_st:
+            return q_graph, None
+        # reference vector_quantize_pytorch.py:262-273,335-362 with commit_quantize attached
+        xf = flat.float()
         commit = None
-        wants_x = grad_on and flat.requires_grad
-        need_graph = st and training and grad_on and (emb_param is not None if fuse_st
-                                                      else (wants_x or emb_param is not None))
-        if need_graph:
-            emb_graph = emb_eff if (emb_param is not None or self.use_affine) else self.embeddings.detach()
-            q_graph = self._gumbel_st_quantize(flat, emb_graph, idx)
-            if fuse_st:     # reference vector_quantize_pytorch.py:262-273,335-362 with commit_quantize attached
-                xf = flat.float()
-                if want_commit:
-                    per = (q_graph - xf) ** 2
-                    commit = per[:, mask_u8.bool()].mean() if mask_u8 is not None else per.mean()
-                if rotation:
-                    # the rotation-trick gradient towards c = q_graph (a detached (H,N,d) "codebook" gathered row by
-                    # row): same forward value fl(x + fl(c - x)), same op as the gather path below
-                    c = q_graph.detach().contiguous()
-                    rows = torch.arange(N, device=c.device).expand(H, N).contiguous()
-                    quant, _, _ = ops.quantize_training(xf, c, rows, mask_u8, False, rotation=True)
-                else:
-                    quant = xf + (q_graph - xf).detach()
-            else:
-                quant = q_graph
-        elif fuse_st and training:
-            quant, commit, _ = ops.quantize_training(flat, emb_val if emb_param is None else emb_eff.contiguous(), idx,
-                                                     mask_u8, want_commit, rotation=rotation)
-        elif emb_param is not None:
-            quant = ops.gather_codes(emb_eff.contiguous(), idx)
-        else:
-            with torch.no_grad():
-                quant, _ = ops.gather_st_loss(x_det, emb_val, idx, None, False, False)
-
-        if update:
-            with torch.no_grad():
-                stats = ops.ema_reduce(x_det, idx, mask_u8, K)
-                if self.use_affine:
-                    # reference :400-403 transforms every latent, (x - batch_mean) * (codebook_std / batch_std) +
-                    # codebook_mean, before the sums; the map is affine, so the per-code sums transform the same way
-                    cnt = stats[..., d:]
-                    stats[..., :d] = (stats[..., :d] - cnt * bm) * inv_scale + cnt * cm
-                self._all_reduce(stats)
-                ops.ema_apply(stats, self.cluster_size.data, self.embed_avg.data, self.embeddings.data,
-                              1 - self.decay, self.eps_for_smoothing, self.weights_l2norm)
-                self._dirty = True
-                self.expire_codes_(x_det)
-        return quant.reshape(H, *lead, d), idx.reshape(H, *lead), commit
+        if want_commit:
+            per = (q_graph - xf) ** 2
+            commit = per[:, mask_u8.bool()].mean() if mask_u8 is not None else per.mean()
+        if not rotation:
+            return xf + (q_graph - xf).detach(), commit
+        # the rotation-trick gradient towards c = q_graph (a detached (H,N,d) "codebook" gathered row by row): same
+        # forward value fl(x + fl(c - x)), same op as the gather path of `_run`
+        c = q_graph.detach().contiguous()
+        rows = torch.arange(N, device=c.device).expand(H, N).contiguous()
+        quant, _, _ = ops.quantize_training(xf, c, rows, mask_u8, False, rotation=True)
+        return quant, commit
 
     # ------------------------------------------------------------------ core
     def _run(self, x: torch.Tensor, mask: Optional[torch.Tensor], freeze_codebook: bool, fuse_st: bool,
@@ -654,92 +498,151 @@ class Codebook(nn.Module):
         (cross-entropy to indices, CE commitment, diversity loss) need: the (H,N,d) latents the search saw and the
         codebook as it was BEFORE this forward's EMA step (reference codebooks.py:386 runs before :425).
         `rotation`: where `fuse_st` applies the straight-through estimator, use the rotation-trick gradient instead
-        (`VectorQuantize.rotation_trick`; the returned values do not change)."""
-        if self.sharded:
-            if keep_dense:
-                raise NotImplementedError("vqb200: the dense-similarity losses are not available on a sharded codebook")
-            return self._run_sharded(x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, rotation)
-        if self._variants_active():
-            return self._run_variants(x, mask, freeze_codebook, fuse_st, want_commit, normalize_input, keep_dense,
-                                      rotation)
+        (`VectorQuantize.rotation_trick`; the returned values do not change).
+
+        One sequence for every configuration; the variants (gumbel sampling, affine; see the module docstring) and the
+        sharded codebook differ from the plain EMA path only where noted.  A shard ends up with the quantised vectors /
+        indices of ITS latents (all of them when the input is replicated) and updates ITS rows of the EMA buffers from
+        the rows they won -- no statistics all_reduce; its exchanges are the min-key all_reduce of the search, one
+        scalar all_reduce in the refresh and the all_gather of the codebook replica the gather reads."""
+        if self.sharded and keep_dense:
+            raise NotImplementedError("vqb200: the dense-similarity losses are not available on a sharded codebook")
+        g = self.gumbel
+        variants = not self.sharded and self._variants_active()
+        stochastic, st = self._variant_sampling() if variants else (False, False)
+        assert not (variants and g["reinmax"] and not g["straight_through"]), \
+            "reinmax can only be turned on if using straight through gumbel softmax"
         _lib.require_device(x)        # raises for a CPU tensor: there is no CPU implementation
         flat, lead = self._flatten(x)
-        H, N, d = flat.shape
+        H, n, d = flat.shape
         if H != self.num_codebooks or d != self.embeddings.shape[-1]:
             raise ValueError(f"vqb200.Codebook: input {tuple(x.shape)} does not match codebook "
-                             f"{tuple(self.embeddings.shape)}")
-        mask_u8 = self._expand_mask(mask, N)
+                             f"(H={self.num_codebooks}, d={self.embeddings.shape[-1]})")
+        mask_u8 = self._expand_mask(mask, n)
+        grad_on = torch.is_grad_enabled()
 
         prepared = False
         if normalize_input:
-            # transform_input="l2norm" (reference vector_quantize_pytorch.py:221): normalisation and the search's operand
-            # preparation share one pass over x when the codebook cache is already final
-            if torch.is_grad_enabled() and flat.requires_grad:
+            # transform_input="l2norm" (reference vector_quantize_pytorch.py:221)
+            if grad_on and flat.requires_grad:
                 # the encoder's gradient passes through the normalisation: same kernel forward (so the values do not
                 # depend on whether a gradient is wanted), F.normalize's Jacobian on the way back
                 flat = ops.l2norm_rows_autograd(flat)
-            elif self.is_initialized and ops.l2norm_prepare_supported(d):
+            elif not (self.sharded or variants) and self.is_initialized and ops.l2norm_prepare_supported(d):
+                # normalisation and the search's operand preparation share one pass over x when the codebook cache is
+                # already final
                 flat = ops.l2norm_prepare(flat, self.codebook_size, self._codebook_cache())
                 prepared = True
             else:
                 flat = ops.l2norm_rows(flat)
+        wants_x = grad_on and flat.requires_grad
 
+        # the latents the search, the EMA statistics and the expiry read: on a shard with "all_gather" input, the
+        # batches of all ranks
+        rows, rows_mask = flat, mask_u8
+        gathered = self.sharded and self.sharded_input == "all_gather"
+        if self.sharded:
+            from . import distributed as D
+            rows = flat.detach()
+            if gathered:
+                rows = D.all_gather_rows(rows, dim=1)
+                if mask_u8 is not None:
+                    rows_mask = D.all_gather_rows(mask_u8, dim=0)
         if not self.is_initialized:
-            self._kmeans_init(flat, mask_u8)
+            self._kmeans_init(rows, rows_mask)
             self.is_initialized = True
 
-        emb = self.embeddings.detach()
-        update = self.training and self.ema_update and not freeze_codebook
-        if keep_dense or (torch.is_grad_enabled() and flat.requires_grad):
-            # the EMA step of this forward, or of a later training forward before backward runs (gradient
-            # accumulation; this one may be frozen), overwrites `embeddings` in place; the reference's commitment
-            # loss holds the gathered codes of THIS forward (vector_quantize_pytorch.py:262-268, a tensor
-            # materialised at codebooks.py:395 before :425), so everything saved for backward reads a snapshot
-            emb = emb.clone()
-        if keep_dense:
-            self.dense_ctx = ops._DenseCtx(flat, emb, self.embeddings, self.use_cosine_sim)
-        idx, _, ws = ops.search(flat, emb, self._codebook_cache(), self.use_cosine_sim, latents_prepared=prepared)
-        self.last_search_ws = ws
-        if self.return_similarities and not fuse_st:
-            self._sim = ops.dense_scores(flat.detach(), emb, self.use_cosine_sim)   # before the EMA step, as :386
-
+        # the codebook of this forward
         training = self.training
-        commit = None
         update = training and self.ema_update and not freeze_codebook
         # learnable codebook (reference codebooks.py:375-377, vector_quantize_pytorch.py:262-268): the commitment loss
         # and the gathered codes are differentiable with respect to `embeddings`
         emb_param = self.embeddings if (self.learnable_codebook and self.commit_grad_to_codebook and training
-                                        and not freeze_codebook and torch.is_grad_enabled()
-                                        and self.embeddings.requires_grad) else None
-        # un-masked training step: gather/ST/loss and the EMA sums share ONE pass over the latents
-        fused = update and mask_u8 is None and self.fused_quantize_ema and ops.quantize_ema_supported(d) \
-            and emb_param is None
-        stats = None
-        if fused and fuse_st:
-            quant, commit, stats = ops.quantize_training(flat, emb, idx, None, want_commit, ema=True, bound_ws=ws,
+                                        and not freeze_codebook and grad_on and self.embeddings.requires_grad) else None
+        live = self.full_codebook() if self.sharded else self.embeddings.detach()
+        emb_eff = live if emb_param is None else emb_param          # the codes as autograd sees them
+        if self.use_affine:
+            self._update_affine(flat, mask_u8)
+            codebook_std = self.codebook_variance.clamp(min=1e-5).sqrt()
+            batch_std = self.batch_variance.clamp(min=1e-5).sqrt()
+            cm, bm, inv_scale = self.codebook_mean, self.batch_mean, codebook_std / batch_std
+            emb_eff = ((emb_eff - cm) * (batch_std / codebook_std) + bm).contiguous()          # reference :381-384
+            codes = emb_eff.detach()
+        elif keep_dense or wants_x:
+            # the EMA step of this forward, or of a later training forward before backward runs (gradient
+            # accumulation; this one may be frozen), overwrites `embeddings` (on a shard: the replica) in place; the
+            # reference's commitment loss holds the gathered codes of THIS forward (vector_quantize_pytorch.py:262-268,
+            # a tensor materialised at codebooks.py:395 before :425), so everything saved for backward reads a snapshot
+            codes = live.clone()
+        else:
+            codes = live
+        if keep_dense:
+            self.dense_ctx = ops._DenseCtx(flat, codes, codes if self.use_affine else self.embeddings,
+                                           self.use_cosine_sim)
+
+        # index assignment
+        if self.sharded:
+            idx_rows = self._shard_search(rows, self.embeddings.detach(), self._codebook_cache())
+            ws = self.last_search_ws
+            lo_r = self.shard_rank * n                              # this rank's batch among the gathered rows
+            idx = idx_rows[:, lo_r:lo_r + n].contiguous() if gathered else idx_rows
+        else:
+            if stochastic:
+                u = self._uniform_queue.pop(0) if self._uniform_queue else None
+                idx = ops.dense_gumbel_sample(rows, codes, self.use_cosine_sim, float(g["temperature"]), uniforms=u)
+                ws = None
+            else:
+                cache = ops.prepare_codebook(codes, self.use_cosine_sim) if self.use_affine else self._codebook_cache()
+                idx, _, ws = ops.search(rows, codes, cache, self.use_cosine_sim, latents_prepared=prepared)
+            self.last_search_ws = ws
+            idx_rows = idx
+            if self.return_similarities and not fuse_st:
+                self._sim = ops.dense_scores(flat.detach(), codes, self.use_cosine_sim)   # before the EMA step, as :386
+
+        # quantize.  Un-masked EMA training step: gather/ST/loss and the EMA sums share ONE pass over the latents (on a
+        # shard with replicated input: the sums of all codes, of which this rank keeps its own)
+        fused = update and mask_u8 is None and not (variants or gathered) and self.fused_quantize_ema \
+            and ops.quantize_ema_supported(d) and emb_param is None
+        commit = stats = None
+        if st and training and grad_on and (emb_param is not None or (wants_x and not fuse_st)):
+            quant, commit = self._gumbel_st_quantize(flat, emb_eff, idx, mask_u8, fuse_st, want_commit, rotation)
+        elif fused and fuse_st:
+            quant, commit, stats = ops.quantize_training(flat, codes, idx, None, want_commit, ema=True, bound_ws=ws,
                                                          rotation=rotation)
         elif fused:
             with torch.no_grad():
-                quant, _, stats = ops.quantize_ema(flat, emb, idx, False, False, bound_ws=ws)
+                quant, _, stats = ops.quantize_ema(flat, codes, idx, False, False, bound_ws=ws)
         elif fuse_st and training:
-            quant, commit, _ = ops.quantize_training(flat, emb if emb_param is None else emb_param, idx, mask_u8,
+            quant, commit, _ = ops.quantize_training(flat, codes if emb_param is None else emb_eff, idx, mask_u8,
                                                      want_commit, rotation=rotation)
         elif emb_param is not None:
-            quant = ops.gather_codes(emb_param, idx)
+            quant = ops.gather_codes(emb_eff, idx)
         else:
             with torch.no_grad():
-                quant, _ = ops.gather_st_loss(flat, emb, idx, None, False, False)
+                quant, _ = ops.gather_st_loss(flat, codes, idx, None, False, False)
 
         if update:
             with torch.no_grad():
-                if stats is None:
-                    stats = ops.ema_reduce(flat, idx, mask_u8, self.codebook_size, bound_ws=ws)
-                self._all_reduce(stats)                       # one packed (H,K,d+1) allreduce (reference: two)
-                ops.ema_apply(stats, self.cluster_size.data, self.embed_avg.data, self.embeddings.data,
-                              1 - self.decay, self.eps_for_smoothing, self.weights_l2norm)
-                self._dirty = True
-                self.expire_codes_(flat)
-
+                if self.sharded:
+                    lo, Ks = self.shard_offset, self.shard_size
+                    stats = stats[:, lo:lo + Ks].contiguous() if stats is not None \
+                        else self._shard_stats(rows, idx_rows, rows_mask)
+                else:
+                    if stats is None:
+                        # the variants take no search bound (it picks the fixed-point scale of the sums)
+                        stats = ops.ema_reduce(rows, idx, mask_u8, self.codebook_size,
+                                               bound_ws=None if variants else ws)
+                    if self.use_affine:
+                        # reference :400-403 transforms every latent, (x - batch_mean) * (codebook_std / batch_std) +
+                        # codebook_mean, before the sums; the map is affine, so the per-code sums transform the same way
+                        cnt = stats[..., d:]
+                        stats[..., :d] = (stats[..., :d] - cnt * bm) * inv_scale + cnt * cm
+                    self._all_reduce(stats)                   # one packed (H,K,d+1) allreduce (reference: two)
+                self._apply_ema(stats)
+                if self.sharded:
+                    self._expire_codes_sharded(rows)
+                else:
+                    self.expire_codes_(rows)
         return quant.reshape(H, *lead, d), idx.reshape(H, *lead), commit
 
     @torch.amp.autocast(device_type="cuda", enabled=False)

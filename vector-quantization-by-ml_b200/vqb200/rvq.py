@@ -81,7 +81,7 @@ class ResidualVQ(nn.Module):
         if not self.use_fused_levels or dropout_active or not x.is_cuda or x.ndim != 3:
             return False
         if any(l._codebook.sharded for l in self.layers):
-            return False        # the level kernels search and update one whole codebook; shards need `_run_sharded`
+            return False        # the level kernels search and update one whole codebook; shards need `Codebook._run`
         if torch.is_grad_enabled() and x.requires_grad and not self._can_fuse_autograd(x):
             return False
         l0 = self.layers[0]
@@ -185,9 +185,7 @@ class ResidualVQ(nn.Module):
                 late_apply.append((dist.all_reduce(stats, async_op=True), stats, cb, li))
             elif do_ema:
                 cb._all_reduce(stats)
-                ops.ema_apply(stats, cb.cluster_size.data, cb.embed_avg.data, cb.embeddings.data, 1 - cb.decay,
-                              cb.eps_for_smoothing, cb.weights_l2norm)
-                cb._dirty = True
+                cb._apply_ema(stats)
                 if not defer:
                     cb.expire_codes_(flat)
                 elif cb.threshold_ema_dead_code != 0:
@@ -203,9 +201,7 @@ class ResidualVQ(nn.Module):
                                      [tr for _, tr in pre_emb], books[0]._expand_mask(mask, N))
         for work, stats, cb, li in late_apply:
             work.wait()
-            ops.ema_apply(stats, cb.cluster_size.data, cb.embed_avg.data, cb.embeddings.data, 1 - cb.decay,
-                          cb.eps_for_smoothing, cb.weights_l2norm)
-            cb._dirty = True
+            cb._apply_ema(stats)
             if cb.threshold_ema_dead_code != 0:
                 pending.append((li, cb, (cb.cluster_size < cb.threshold_ema_dead_code).sum()))
         dead_counts = torch.stack([p[2] for p in pending]) if pending else None
