@@ -139,8 +139,18 @@ int    vqb_rot_commit_backward(const float* grad_q, const float* grad_loss, cons
  * Stable counting sort of rows by code, fixed-order segmented sums: bitwise reproducible. */
 size_t vqb_ema_workspace_bytes(int64_t H, int64_t N, int K, int d);
 /* absmax_bound2: nullable device pointer to two floats (a, b) with a + b >= max|x_j| over the batch
- * (the first 8 bytes of a search workspace after vqb_search on the same x hold exactly that);
- * when NULL the bound is computed with one extra pass over x.  It only sizes the fixed-point scale. */
+ * (all codebooks, masked rows included); when NULL the bound is computed with one extra pass over x.
+ * It only sizes the fixed-point scale: a bound below max|x_j| makes the integer sums wrap around.
+ * The first 8 bytes of a search workspace hold such a pair after vqb_search on the same x, with no
+ * other search through that workspace in between.  Per route of vqb_search:
+ *   tensor-core search, operands prepared by the search: a = bound of the row norms |x~|, b = bound of
+ *     the rounding residuals |x - x~| (prepare.cu), so a + b >= |x| >= max|x_j|;
+ *   VQB_SEARCH_LATENTS_PREPARED: the same pair, as vqb_rvq_level / vqb_rvq_level_ema / the l2norm
+ *     pass left it with the operands;
+ *   VQB_SEARCH_FUSED_PREP (in-kernel conversion): a = the sampled row-norm bound, b = the largest norm
+ *     bound of the rows above it (the rows the exact rescan takes);
+ *   exact scan (VQB_SEARCH_FORCE_EXACT, no cache, or d_pad > 512): a = max|x_j| itself, b = 0.
+ * A non-finite bound (rows whose |x|^2 overflows fp32) falls back to 1. */
 int    vqb_ema_reduce(const void* x, int x_dtype, const int64_t* idx, const uint8_t* mask,
                       const float* absmax_bound2,
                       int64_t H, int64_t N, int K, int d, float* stats,

@@ -247,7 +247,11 @@ int launch_make_bias(const void* cache, const CacheLayout& CL, int64_t H, int K,
 // In-kernel conversion of 16-bit latents (search_tc.cu, CONV): scal[0] = bound of the row norms from a strided sample
 // (times kSampleGuard); the search kernel converts every row itself and sends rows that exceed the bound to the exact
 // rescan (negative xinv), so the bound only has to be right for the rows that keep their tensor-core candidates.
+// conv_outlier_bound_kernel (search_resolve.cu) then raises scal[1] to the norm bound of those rows, so that
+// scal[0] + scal[1] bounds max|x_j| over the whole batch, as a search workspace promises the EMA kernels (vqb.h).
 int launch_sample_bound(const void* x, int x_dtype, int64_t rows, int d, uint32_t* scal, cudaStream_t st);
+// *out = max|x_i| over n elements, exactly (atomicMax of the float bits; *out must be 0 or a smaller bound before)
+int launch_absmax(const void* x, int x_dtype, int64_t n, uint32_t* out, cudaStream_t st);
 struct ConvArgs {
   const void* x = nullptr;   // raw latents [H][N][d], bf16 or fp16; nullptr: operands were prepared by a separate pass
   int x_dtype = 0;

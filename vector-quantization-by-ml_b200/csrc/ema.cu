@@ -62,6 +62,12 @@ __global__ void absmax_kernel(const T* __restrict__ x, int64_t n, uint32_t* __re
   if ((threadIdx.x & 31) == 0) atomicMax(out, __float_as_uint(m));
 }
 
+int launch_absmax(const void* x, int x_dtype, int64_t n, uint32_t* out, cudaStream_t st) {
+  VQB_DISPATCH_DTYPE(x_dtype, T, absmax_kernel<T><<<1184, 256, 0, st>>>((const T*)x, n, out));
+  VQB_LAUNCH_CHECK();
+  return VQB_OK;
+}
+
 // s = 61 - ceil(log2(bound * rows)), clamped; scale[0] = s
 __global__ void ema_scale_kernel(const float* __restrict__ bound2, const uint32_t* __restrict__ own_bound,
                                  int64_t rows, int* __restrict__ scale) {
@@ -896,11 +902,8 @@ extern "C" int vqb_ema_reduce(const void* x, int x_dtype, const int64_t* idx, co
   int* sorted = (int*)(w + L.off_sorted);
   VQB_CUDA_TRY(cudaMemsetAsync(w, 0, L.zero_bytes, st));
   if (N > 0) {
-    if (!absmax_bound2) {
-      VQB_DISPATCH_DTYPE(x_dtype, T,
-        absmax_kernel<T><<<1184, 256, 0, st>>>((const T*)x, H * N * (int64_t)d, (uint32_t*)(scale + 1)));
-      VQB_LAUNCH_CHECK();
-    }
+    if (!absmax_bound2)
+      if (int rc = launch_absmax(x, x_dtype, H * N * (int64_t)d, (uint32_t*)(scale + 1), st)) return rc;
     ema_scale_kernel<<<1, 1, 0, st>>>(absmax_bound2, (const uint32_t*)(scale + 1), N, scale);
     VQB_LAUNCH_CHECK();
     if (int rc = launch_code_sort(idx, mask, H, N, K, counts, cursor, start, sorted,
@@ -951,11 +954,8 @@ static int quantize_ema_impl(const void* x, int x_dtype, const float* codebook, 
   const int two_terms = x_dtype == VQB_F32 ? 1 : 0;
   VQB_CUDA_TRY(cudaMemsetAsync(w, 0, L.E.zero_bytes, st));
   if (N > 0) {
-    if (!absmax_bound2) {
-      VQB_DISPATCH_DTYPE(x_dtype, T,
-        absmax_kernel<T><<<1184, 256, 0, st>>>((const T*)x, H * N * (int64_t)d, (uint32_t*)(scale + 1)));
-      VQB_LAUNCH_CHECK();
-    }
+    if (!absmax_bound2)
+      if (int rc = launch_absmax(x, x_dtype, H * N * (int64_t)d, (uint32_t*)(scale + 1), st)) return rc;
     fused_scale_kernel<<<1, 1, 0, st>>>(absmax_bound2, (const uint32_t*)(scale + 1), N, two_terms, scale);
     VQB_LAUNCH_CHECK();
     // the next level's statistics usually live in the workspace absmax_bound2 points into: zero them only now

@@ -531,6 +531,20 @@ __global__ void rescan_finalize_kernel(const int* __restrict__ flag_list, const 
   }
 }
 
+// In-kernel conversion: scal[0] bounds only the rows within the sampled bound; the search kernel gave the others a
+// negative xinv (they are rescanned exactly).  Their norm bound xn2 (>= |x|^2) goes into scal[1], which nothing reads on
+// this route once make_bias has run, so that scal[0] + scal[1] >= max|x_j| over the batch, as the EMA kernels read it
+// (vqb.h, vqb_ema_reduce).
+__global__ void __launch_bounds__(256)
+conv_outlier_bound_kernel(const float* __restrict__ xinv, const float* __restrict__ xn2, int64_t rows,
+                          uint32_t* __restrict__ scal) {
+  float m = 0.f;
+  for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (int64_t)gridDim.x * blockDim.x)
+    if (xinv[r] < 0.f) m = fmaxf(m, sqrtf(xn2[r]));
+  m = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m)));   // non-negative: bit order = float order
+  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(scal + 1, __float_as_uint(m));
+}
+
 static int g_num_sms = 0;
 static int num_sms() {
   if (!g_num_sms) {
@@ -582,6 +596,8 @@ extern "C" int vqb_search(const void* x, int x_dtype, const float* codebook, con
 
   const int grid_scan = (int)((N + kER - 1) / kER < 4 * (int64_t)num_sms() ? (N + kER - 1) / kER : 4 * num_sms());
   if (!tc) {
+    // nothing on this route writes the row statistics: scal[0] = max|x_j| for the EMA kernels (vqb.h, vqb_ema_reduce)
+    if (int rc = launch_absmax(x, x_dtype, H * N * (int64_t)d, scal, st)) return rc;
     VQB_DISPATCH_DTYPE(x_dtype, T,
       exact_scan_kernel<T, false><<<dim3((unsigned)grid_scan, (unsigned)H), 256, 0, st>>>(
           (const T*)x, codebook, nullptr, nullptr, N, K, d, metric, idx_offset, idx_out, score_out, scal, 0, nullptr));
@@ -625,6 +641,11 @@ extern "C" int vqb_search(const void* x, int x_dtype, const float* codebook, con
                         bias, aug, H, N, K, SL.dp, w + SL.off_cand, scal, (flags & VQB_SEARCH_TIMING) != 0, st, conv);
   if (rc) return rc;
   const int64_t total = H * N;
+  if (conv_mode == 1) {
+    const int64_t want = (total + 255) / 256, cap = 4 * (int64_t)num_sms();
+    conv_outlier_bound_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(xinv, xn2, total, scal);
+    VQB_LAUNCH_CHECK();
+  }
   int* rr_list = (int*)(w + SL.off_rr);
   if (score_out) {
     VQB_DISPATCH_DTYPE(x_dtype, T,

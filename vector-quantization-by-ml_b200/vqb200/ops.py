@@ -209,7 +209,10 @@ def quantize_ema_supported(d: int) -> bool:
 @_on_device
 def quantize_ema(x: torch.Tensor, embeddings: torch.Tensor, idx: torch.Tensor, training: bool, want_loss: bool,
                  bound_ws: Optional[torch.Tensor] = None):
-    """Fused gather/ST/loss + EMA sums (no mask): returns (q (H,N,d) fp32, loss_buf | None, stats (H,K,d+1))."""
+    """Fused gather/ST/loss + EMA sums (no mask): returns (q (H,N,d) fp32, loss_buf | None, stats (H,K,d+1)).
+    `bound_ws`: the workspace `search` returned for this same `x`, with no other search in between (its first 8 bytes
+    bound max|x_j|, which sizes the fixed-point sums; a stale or foreign bound can make them wrap around); None: one
+    extra pass over x computes the bound."""
     L.require_cuda(x, "x")
     H, N, d = x.shape
     K = embeddings.shape[1]
@@ -344,7 +347,10 @@ def quantize_training(x, embeddings, idx, mask_u8, want_loss, ema: bool = False,
 @_on_device
 def ema_reduce(x: torch.Tensor, idx: torch.Tensor, mask_u8: Optional[torch.Tensor], K: int,
                bound_ws: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """stats (H,K,d+1): per-code sums of assigned rows and counts.  Bitwise reproducible."""
+    """stats (H,K,d+1): per-code sums of assigned rows and counts.  Bitwise reproducible.
+    `bound_ws`: the workspace `search` returned for this same `x`, with no other search in between (its first 8 bytes
+    bound max|x_j|, which sizes the fixed-point sums; a stale or foreign bound can make them wrap around); None: one
+    extra pass over x computes the bound."""
     L.require_cuda(x, "x")
     H, N, d = x.shape
     dev = x.device
@@ -507,7 +513,8 @@ def rvq_level_ema_supported(d: int) -> bool:
 def rvq_level_ema(residual: torch.Tensor, residual_next: torch.Tensor, embeddings: torch.Tensor, idx: torch.Tensor,
                   training: bool, first_level: bool, quantized_out: torch.Tensor, next_cache: Optional[torch.Tensor],
                   bound_ws: Optional[torch.Tensor] = None, q_out: Optional[torch.Tensor] = None):
-    """rvq_level + ema_reduce of an un-masked level in one pass: returns (loss_buf, stats (1,K,d+1))."""
+    """rvq_level + ema_reduce of an un-masked level in one pass: returns (loss_buf, stats (1,K,d+1)).
+    `bound_ws` as in `ema_reduce`: the workspace of the search on this `residual`."""
     L.require_cuda(residual, "residual")
     L.require_cuda(residual_next, "residual_next")
     assert residual.dtype == torch.float32 and residual.ndim == 2 and residual_next.shape == residual.shape
