@@ -76,10 +76,23 @@ inline CacheLayout cache_layout(int64_t H, int K, int d) {
   return L;
 }
 
+// Slots of the u32[64] block at the head of a search workspace (SearchLayout::off_scal).  Float bounds are stored as
+// their bits: non-negative floats order like unsigned ints, so atomicMax raises them.
+constexpr int kScalXMax = 0;         // bound of max |x_b| over the batch (x_b = fp16(x s_row) / s_row)
+constexpr int kScalDxMax = 1;        // bound of max |x - x_b| over the batch
+constexpr int kScalRescanned = 2;    // rows resolved by a scan of every code
+constexpr int kScalReranked = 3;     // rows queued for the warp-per-row re-rank
+constexpr int kScalTcUsed = 4;       // 1: the tensor-core pass ran
+constexpr int kScalMisaligned = 5;   // 1: the search kernel's dynamic shared memory was not 1024 B aligned
+constexpr int kScalEmax = 6;         // max_k E_k
+constexpr int kScalTwoQ = 7;         // 2^q of bias operands prepared outside the search (0: prepared by this search)
+constexpr int kScalUnlowered = 8;    // 1: keys not pre-lowered by E_k (window 2 Emax)
+constexpr int kScalPairs = 9;        // (row, code) pairs queued for exact scoring
+
 // Search workspace layout (one caller-owned buffer).
 struct SearchLayout {
   int dp;
-  size_t off_scal;    // u32[64]: [0]=max|x_b| bits, [1]=max|x-x_b| bits, [2]=#rescanned, [3]=#reranked, [4]=tc used, [5]=smem misalign flag, [6]=max E_k bits, [7]=2^q bits of operands prepared by vqb_rvq_level (0: prepared by this search), [8]=1: keys not pre-lowered by E_k (window 2 Emax), [9]=#pairs
+  size_t off_scal;    // u32[64]: slots kScal* above
   size_t off_cnt;     // u32[3][H]: flagged rows per codebook | left to the tiled rescan | pair plan (after scal: zeroed together)
   size_t off_xb;      // fp16 [H][N][dp]  = fp16(x * s_row), zero padded
   size_t off_xinv;    // f32  [H][N]      = 1 / s_row (exact power of two); NEGATIVE marks a row whose bias operand
@@ -89,10 +102,10 @@ struct SearchLayout {
   size_t off_keys;    // u64  [H][N]      packed (score, index) min-keys of rows being rescanned
   size_t off_cand;    // {f32 key, i32 code} [H][N][kNumCand]
   size_t off_flag;    // i32 [H*N] flagged row list
-  size_t off_rr;      // i32 [H*N] rows queued for the warp-per-row re-rank (length in scal[3])
+  size_t off_rr;      // i32 [H*N] rows queued for the warp-per-row re-rank (length in scal[kScalReranked])
   size_t off_bias;    // f32 [H][Kp]  lower-bound bias  |c|^2/2 - E_k  (needs the row stats, so per search)
   size_t off_err;     // f32 [H][Kp]  E_k: bound on |exact score - fp16 tensor-core score| for code k
-  size_t off_pairs;   // {u32 row, u32 code} [pair_cap]  (row, code) pairs scored exactly in resolve phase 2 (count in scal[9])
+  size_t off_pairs;   // {u32 row, u32 code} [pair_cap]  (row, code) pairs scored exactly in resolve phase 2 (count in scal[kScalPairs])
   size_t pair_cap;
   size_t off_caug;    // fp16 [H][Kp][8]  three fp16 pieces of s_c 2^q bias_k (+inf for padded codes), then zeros:
                       //                  the bias term of the score as one extra MMA k-step (search_tc.cu)
@@ -119,6 +132,37 @@ inline SearchLayout search_layout(int64_t H, int64_t N, int K, int d) {
   L.off_pairs = o; o += align_up(L.pair_cap * 8);
   L.total = o;
   return L;
+}
+
+// The latent operand of the tensor-core search inside a search workspace (fields as in SearchLayout), and the header
+// of the codebook cache whose 2^q the bias operand is built with.  make_bias and resolve rely on exactly these values
+// (search_resolve.cu), the EMA kernels on scal[kScalXMax] + scal[kScalDxMax] (vqb.h).  The preparation kernels take
+// its fields as separate parameters: passed as one struct, they compile to up to 8 more registers each (sm_100a).
+struct LatentOperand {
+  __half* xb;
+  float* xinv;
+  float* xn2;
+  __half* xaug;
+  uint32_t* scal;
+  const float* chdr;
+  int dp;
+};
+inline LatentOperand latent_operand(void* search_ws, int64_t H, int64_t N, int K, int d, const void* cache) {
+  const SearchLayout SL = search_layout(H, N, K, d);
+  char* w = (char*)search_ws;
+  return {(__half*)(w + SL.off_xb), (float*)(w + SL.off_xinv), (float*)(w + SL.off_xn2), (__half*)(w + SL.off_xaug),
+          (uint32_t*)(w + SL.off_scal), (const float*)((const char*)cache + cache_layout(H, K, d).off_hdr), SL.dp};
+}
+
+// SM count of the device that is current at the first call (persistent grids are sized from it)
+inline int num_sms() {
+  static const int n = [] {
+    int dev = 0, v = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
+    return v > 0 ? v : 148;
+  }();
+  return n;
 }
 
 // ---- device helpers -----------------------------------------------------------------------
@@ -236,19 +280,18 @@ __device__ __forceinline__ double warp_sum(double v) {
 inline int dtype_size(int dt) { return dt == VQB_F32 ? 4 : 2; }
 
 // ---- internal launchers (defined across the .cu files) --------------------------------------
-// chdr: per-codebook cache header (nullable: no bias operand is written then); rows_per_head maps a row to its header
-int launch_prepare_latents(const void* x, int x_dtype, int64_t rows, int64_t rows_per_head, int d, int dp,
-                           const float* chdr, __half* xb, float* xinv, float* xn2, __half* xaug, uint32_t* scal,
-                           cudaStream_t st);
-// derive_dx_dp > 0: the residual bound |x - x~| is not in scal[1] but derived from scal[0] by dx_bound_16bit()
+// rows_per_head maps a row to its codebook's header in op.chdr
+int launch_prepare_latents(const void* x, int x_dtype, int64_t rows, int64_t rows_per_head, int d,
+                           const LatentOperand& op, cudaStream_t st);
+// derive_dx_dp > 0: the residual bound |x - x~| is not in scal[kScalDxMax] but derived from scal[kScalXMax] by dx_bound_16bit()
 // (16-bit latents converted inside the search kernel: search_tc.cu, CONV)
 int launch_make_bias(const void* cache, const CacheLayout& CL, int64_t H, int K, int metric,
                      uint32_t* scal, float* bias, float* err, __half* caug, cudaStream_t st, int derive_dx_dp = 0);
-// In-kernel conversion of 16-bit latents (search_tc.cu, CONV): scal[0] = bound of the row norms from a strided sample
+// In-kernel conversion of 16-bit latents (search_tc.cu, CONV): scal[kScalXMax] = bound of the row norms from a strided sample
 // (times kSampleGuard); the search kernel converts every row itself and sends rows that exceed the bound to the exact
 // rescan (negative xinv), so the bound only has to be right for the rows that keep their tensor-core candidates.
-// conv_outlier_bound_kernel (search_resolve.cu) then raises scal[1] to the norm bound of those rows, so that
-// scal[0] + scal[1] bounds max|x_j| over the whole batch, as a search workspace promises the EMA kernels (vqb.h).
+// conv_outlier_bound_kernel (search_resolve.cu) then raises scal[kScalDxMax] to the norm bound of those rows, so that
+// scal[kScalXMax] + scal[kScalDxMax] bounds max|x_j| over the whole batch, as a search workspace promises the EMA kernels (vqb.h).
 int launch_sample_bound(const void* x, int x_dtype, int64_t rows, int d, uint32_t* scal, cudaStream_t st);
 // *out = max|x_i| over n elements, exactly (atomicMax of the float bits; *out must be 0 or a smaller bound before)
 int launch_absmax(const void* x, int x_dtype, int64_t n, uint32_t* out, cudaStream_t st);
@@ -323,6 +366,14 @@ __host__ __device__ inline float pow2_scale(float m) {
   if (sh > 100) sh = 100;
   if (sh < -100) sh = -100;
   return ldexpf(1.f, sh);
+}
+
+// Bits of the bound of sqrt(max2), max2 the largest of a batch's fp32 sums of squares over dp terms (|x~|^2 or
+// |x - x~|^2): the sum is inflated by (1 + dp 2.4e-7) for its roundings before the square root.  Non-negative floats
+// order like their bits, so atomicMax of these raises scal[kScalXMax] / scal[kScalDxMax].
+__device__ __forceinline__ uint32_t batch_bound_bits(float max2, int dp) {
+  const float infl = 1.f + (float)dp * 2.4e-7f;
+  return __float_as_uint(sqrtf(max2 * infl) * 1.00001f);
 }
 
 }  // namespace vqb

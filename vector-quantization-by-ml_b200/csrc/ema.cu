@@ -427,14 +427,8 @@ struct RvqExtra {
   float* out;             // (N,d) running sum of the levels' outputs, updated in place
   float* res_out;         // (N,d) next residual
   float* q_level;         // (N,d) this level's output, nullable
-  __half* next_xb;        // nullable: no next level
-  float* next_xinv;
-  float* next_xn2;
-  __half* next_xaug;
-  uint32_t* next_scal;
-  const float* next_chdr;
+  LatentOperand next;     // next.xb null: no next level
   int first;
-  int dp;
 };
 
 template <typename T, int NB, int TERMS, bool RVQ>
@@ -594,16 +588,16 @@ quantize_ema_kernel(const T* __restrict__ x, const float* __restrict__ cb, const
           }
         }
       }
-      if (RVQ && R.next_xb) {                   // next level's operand (shuffles: every lane takes part)
+      if (RVQ && R.next.xb) {                   // next level's operand (shuffles: every lane takes part)
         const bool live = kk[u] >= 0;
         for (int o2 = lpr >> 1; o2 > 0; o2 >>= 1) mabs = fmaxf(mabs, __shfl_xor_sync(0xffffffffu, mabs, o2));
         float s = pow2_scale_bits(mabs);
-        const float a = clamp_row_scale(s, R.next_chdr[4], R.next_chdr[5]);
+        const float a = clamp_row_scale(s, R.next.chdr[4], R.next.chdr[5]);
         const float is = pow2_recip(s);
         if (gl == 0 && live) {
-          R.next_xinv[rr[u]] = a > 0.f ? is : -is;
+          R.next.xinv[rr[u]] = a > 0.f ? is : -is;
           const uint32_t aa = (uint32_t)__half_as_ushort(__float2half_rn(a));
-          *reinterpret_cast<uint4*>(R.next_xaug + (int64_t)rr[u] * 8) = make_uint4(aa | (aa << 16), aa, 0u, 0u);
+          *reinterpret_cast<uint4*>(R.next.xaug + (int64_t)rr[u] * 8) = make_uint4(aa | (aa << 16), aa, 0u, 0u);
         }
         float n2 = 0.f, r2 = 0.f;
 #pragma unroll
@@ -621,13 +615,13 @@ quantize_ema_kernel(const T* __restrict__ x, const float* __restrict__ cb, const
             r2 += e0 * e0 + e1 * e1;
           }
           if (live)
-            *reinterpret_cast<uint4*>(R.next_xb + (int64_t)rr[u] * R.dp + b * 256 + j) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+            *reinterpret_cast<uint4*>(R.next.xb + (int64_t)rr[u] * R.next.dp + b * 256 + j) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
         }
         for (int o2 = lpr >> 1; o2 > 0; o2 >>= 1) {
           n2 += __shfl_xor_sync(0xffffffffu, n2, o2);
           r2 += __shfl_xor_sync(0xffffffffu, r2, o2);
         }
-        if (gl == 0 && live) R.next_xn2[rr[u]] = row_norm2_bound(n2, r2);
+        if (gl == 0 && live) R.next.xn2[rr[u]] = row_norm2_bound(n2, r2);
         max_n2 = fmaxf(max_n2, n2);
         max_r2 = fmaxf(max_r2, r2);
       }
@@ -638,17 +632,16 @@ quantize_ema_kernel(const T* __restrict__ x, const float* __restrict__ cb, const
     }
   }
   flush();
-  if (RVQ && R.next_xb) {
+  if (RVQ && R.next.xb) {
 #pragma unroll
     for (int o2 = 16; o2 > 0; o2 >>= 1) {
       max_n2 = fmaxf(max_n2, __shfl_xor_sync(0xffffffffu, max_n2, o2));
       max_r2 = fmaxf(max_r2, __shfl_xor_sync(0xffffffffu, max_r2, o2));
     }
     if (lane == 0) {
-      const float infl = 1.f + (float)R.dp * 2.4e-7f;
-      atomicMax(R.next_scal + 0, __float_as_uint(sqrtf(max_n2 * infl) * 1.00001f));
-      atomicMax(R.next_scal + 1, __float_as_uint(sqrtf(max_r2 * infl) * 1.00001f));
-      if (blockIdx.x == 0 && threadIdx.x == 0) R.next_scal[7] = __float_as_uint(R.next_chdr[4]);
+      atomicMax(R.next.scal + kScalXMax, batch_bound_bits(max_n2, R.next.dp));
+      atomicMax(R.next.scal + kScalDxMax, batch_bound_bits(max_r2, R.next.dp));
+      if (blockIdx.x == 0 && threadIdx.x == 0) R.next.scal[kScalTwoQ] = __float_as_uint(R.next.chdr[4]);
     }
   }
 }
@@ -959,7 +952,7 @@ static int quantize_ema_impl(const void* x, int x_dtype, const float* codebook, 
     fused_scale_kernel<<<1, 1, 0, st>>>(absmax_bound2, (const uint32_t*)(scale + 1), N, two_terms, scale);
     VQB_LAUNCH_CHECK();
     // the next level's statistics usually live in the workspace absmax_bound2 points into: zero them only now
-    if (rvq && rvq->next_scal) VQB_CUDA_TRY(cudaMemsetAsync(rvq->next_scal, 0, 8, st));
+    if (rvq && rvq->next.xb) VQB_CUDA_TRY(cudaMemsetAsync(rvq->next.scal, 0, (kScalDxMax + 1) * 4, st));
     if (int rc = launch_code_sort(idx, nullptr, H, N, K, counts, cursor, start, sorted,
                                   K <= kSortMaxK ? (uint32_t*)(w + L.E.off_table) : nullptr, st)) return rc;
     const int64_t chunks = (N + kFusedChunkRows - 1) / kFusedChunkRows;
@@ -1029,17 +1022,12 @@ extern "C" int vqb_rvq_level_ema(const float* residual_in, float* residual_out, 
   VQB_REQUIRE(residual_in != residual_out, VQB_ERR_INVALID, "vqb_rvq_level_ema: rows are visited in code order, the "
               "residual cannot be updated in place");
   RvqExtra R = {};
-  R.out = quantized_out; R.res_out = residual_out; R.q_level = q_out; R.first = first_level; R.dp = d_pad(d);
+  R.out = quantized_out; R.res_out = residual_out; R.q_level = q_out; R.first = first_level;
   if (next_ws) {
     VQB_REQUIRE(next_cache != nullptr, VQB_ERR_INVALID, "vqb_rvq_level_ema: next_ws needs next_cache");
-    SearchLayout SL = search_layout(1, N, K, d);
-    VQB_REQUIRE(next_ws_bytes >= SL.total, VQB_ERR_WORKSPACE, "next-level search workspace too small");
-    R.next_xb = (__half*)((char*)next_ws + SL.off_xb);
-    R.next_xaug = (__half*)((char*)next_ws + SL.off_xaug);
-    R.next_xinv = (float*)((char*)next_ws + SL.off_xinv);
-    R.next_xn2 = (float*)((char*)next_ws + SL.off_xn2);
-    R.next_scal = (uint32_t*)((char*)next_ws + SL.off_scal);
-    R.next_chdr = (const float*)((const char*)next_cache + cache_layout(1, K, d).off_hdr);
+    VQB_REQUIRE(next_ws_bytes >= search_layout(1, N, K, d).total, VQB_ERR_WORKSPACE,
+                "next-level search workspace too small");
+    R.next = latent_operand(next_ws, 1, N, K, d, next_cache);
   }
   return quantize_ema_impl(residual_in, VQB_F32, codebook, idx, absmax_bound2, training, 1, nullptr, loss_out, stats, 1,
                            N, K, d, ws, ws_bytes, &R, stream);

@@ -22,15 +22,8 @@ struct GatherLayout {
   size_t total;
 };
 static int gather_grid(int64_t rows) {
-  static int sms = 0;
-  if (!sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
-  }
   int64_t need = (rows + (kGatherThreads / 32) - 1) / (kGatherThreads / 32);
-  int64_t cap = (int64_t)sms * 8;
+  int64_t cap = (int64_t)num_sms() * 8;
   return (int)(need < cap ? (need > 0 ? need : 1) : cap);
 }
 static GatherLayout gather_layout() {
@@ -429,10 +422,9 @@ rvq_level_kernel(const float* res_in, float* res_out, const float* __restrict__ 
     part[blockIdx.x] = t;
     cntp[blockIdx.x] = c;
     if (next_scal) {
-      const float infl = 1.f + (float)dp * 2.4e-7f;
-      atomicMax(next_scal + 0, __float_as_uint(sqrtf(a * infl) * 1.00001f));
-      atomicMax(next_scal + 1, __float_as_uint(sqrtf(b * infl) * 1.00001f));
-      if (blockIdx.x == 0) next_scal[7] = __float_as_uint(next_chdr[4]);   // the 2^q these operands were built with
+      atomicMax(next_scal + kScalXMax, batch_bound_bits(a, dp));
+      atomicMax(next_scal + kScalDxMax, batch_bound_bits(b, dp));
+      if (blockIdx.x == 0) next_scal[kScalTwoQ] = __float_as_uint(next_chdr[4]);   // the 2^q these operands were built with
     }
   }
 }
@@ -745,26 +737,16 @@ extern "C" int vqb_rvq_level(const float* residual_in, float* residual_out, cons
   GatherLayout L = gather_layout();
   VQB_REQUIRE(gather_ws_bytes >= L.total, VQB_ERR_WORKSPACE, "gather workspace too small");
   cudaStream_t st = (cudaStream_t)stream;
-  __half* nxb = nullptr;
-  __half* nxaug = nullptr;
-  float* nxinv = nullptr;
-  float* nxn2 = nullptr;
-  uint32_t* nscal = nullptr;
-  const float* nchdr = nullptr;
+  LatentOperand next = {};   // all null: no next level to prepare
   const int dp = d_pad(d);
   if (next_ws && dp > 512) next_ws = nullptr;   // no tensor-core pass for this width: nothing to prepare
   if (next_ws) {
     VQB_REQUIRE(next_cache != nullptr, VQB_ERR_INVALID,
                 "vqb_rvq_level: next_ws needs next_cache (the codebook cache of the level that will search it)");
-    SearchLayout SL = search_layout(1, N, K, d);
-    VQB_REQUIRE(next_ws_bytes >= SL.total, VQB_ERR_WORKSPACE, "next-level search workspace too small");
-    nxb = (__half*)((char*)next_ws + SL.off_xb);
-    nxaug = (__half*)((char*)next_ws + SL.off_xaug);
-    nxinv = (float*)((char*)next_ws + SL.off_xinv);
-    nxn2 = (float*)((char*)next_ws + SL.off_xn2);
-    nscal = (uint32_t*)((char*)next_ws + SL.off_scal);
-    nchdr = (const float*)((const char*)next_cache + cache_layout(1, K, d).off_hdr);
-    VQB_CUDA_TRY(cudaMemsetAsync(nscal, 0, 8, st));
+    VQB_REQUIRE(next_ws_bytes >= search_layout(1, N, K, d).total, VQB_ERR_WORKSPACE,
+                "next-level search workspace too small");
+    next = latent_operand(next_ws, 1, N, K, d, next_cache);
+    VQB_CUDA_TRY(cudaMemsetAsync(next.scal, 0, (kScalDxMax + 1) * 4, st));
   }
   const int grid = gather_grid(N);
   double* part = (double*)((char*)gather_ws + L.off_part);
@@ -772,7 +754,7 @@ extern "C" int vqb_rvq_level(const float* residual_in, float* residual_out, cons
   if (N > 0) {
     rvq_level_kernel<<<grid, kGatherThreads, 0, st>>>(residual_in, residual_out, codebook, idx, mask, training, first_level,
                                                       quantized_out, q_out, N, K, d, dp, part, cntp,
-                                                      nxb, nxinv, nscal, nxaug, nchdr, nxn2);
+                                                      next.xb, next.xinv, next.scal, next.xaug, next.chdr, next.xn2);
     VQB_LAUNCH_CHECK();
   }
   loss_finalize_kernel<<<1, 256, 0, st>>>(part, cntp, N > 0 ? grid : 0, d, loss_out);

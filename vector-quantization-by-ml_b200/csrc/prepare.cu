@@ -7,8 +7,6 @@
 //     power-of-two scales remove fp16's range problem and are undone exactly in the epilogue.
 //   * per-search lower-bound bias  L_k = |c_k|^2/2 - E_k  (see search_resolve.cu for the proof sketch)
 //   * l2norm of rows (reference utils/losses.py:19)
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace vqb {
@@ -86,9 +84,9 @@ __global__ void codebook_aug_scale_kernel(int64_t H, float* __restrict__ hdr) {
 
 // Fast variant for d % 8 == 0, d <= 256 (one 8-element group per lane): a warp converts 4 (fp32) or 8 (16-bit) rows per
 // iteration with all loads issued up front -- with one 512 B row per warp in flight the kernel is latency bound (Little's law:
-// ~19 KB per SM in flight ~ 3.5 TB/s).
-template <typename T, int MINB>
-__global__ void __launch_bounds__(256, MINB)
+// ~19 KB per SM in flight ~ 3.5 TB/s).  Three blocks per SM: the register cap that measured fastest, without spills.
+template <typename T>
+__global__ void __launch_bounds__(256, 3)
 prepare_latents4_kernel(const T* __restrict__ x, int64_t rows, int64_t rows_per_head, bool single_head, int d, int dp,
                         const float* __restrict__ chdr, __half* __restrict__ xb, float* __restrict__ xinv,
                         float* __restrict__ xn2, __half* __restrict__ xaug, uint32_t* __restrict__ scal) {
@@ -188,9 +186,8 @@ prepare_latents4_kernel(const T* __restrict__ x, int64_t rows, int64_t rows_per_
   if (threadIdx.x == 0) {
     float mn = 0.f, mr = 0.f;
     for (int i = 0; i < wpb; ++i) { mn = fmaxf(mn, s_n[i]); mr = fmaxf(mr, s_r[i]); }
-    const float infl = 1.f + (float)dp * 2.4e-7f;
-    atomicMax(scal + 0, __float_as_uint(sqrtf(mn * infl) * 1.00001f));
-    atomicMax(scal + 1, __float_as_uint(sqrtf(mr * infl) * 1.00001f));
+    atomicMax(scal + kScalXMax, batch_bound_bits(mn, dp));
+    atomicMax(scal + kScalDxMax, batch_bound_bits(mr, dp));
   }
 }
 
@@ -282,9 +279,8 @@ prepare_latents_narrow_kernel(const T* __restrict__ x, int64_t rows, int64_t row
   if (threadIdx.x == 0) {
     float mn = 0.f, mr = 0.f;
     for (int i = 0; i < wpb; ++i) { mn = fmaxf(mn, s_n[i]); mr = fmaxf(mr, s_r[i]); }
-    const float infl = 1.f + (float)dp * 2.4e-7f;
-    atomicMax(scal + 0, __float_as_uint(sqrtf(mn * infl) * 1.00001f));
-    atomicMax(scal + 1, __float_as_uint(sqrtf(mr * infl) * 1.00001f));
+    atomicMax(scal + kScalXMax, batch_bound_bits(mn, dp));
+    atomicMax(scal + kScalDxMax, batch_bound_bits(mr, dp));
   }
 }
 
@@ -380,28 +376,23 @@ __global__ void prepare_latents_kernel(const T* __restrict__ x, int64_t rows, in
   if (threadIdx.x == 0) {
     float mn = 0.f, mr = 0.f;
     for (int i = 0; i < wpb; ++i) { mn = fmaxf(mn, s_n[i]); mr = fmaxf(mr, s_r[i]); }
-    // fp32 accumulation of a sum of squares: inflate by (1 + dp * 2^-23) before the square root
-    float infl = 1.f + (float)dp * 2.4e-7f;
-    float a = sqrtf(mn * infl) * 1.00001f, b = sqrtf(mr * infl) * 1.00001f;
-    atomicMax(scal + 0, __float_as_uint(a));   // non-negative floats order like their bit patterns
-    atomicMax(scal + 1, __float_as_uint(b));
+    atomicMax(scal + kScalXMax, batch_bound_bits(mn, dp));
+    atomicMax(scal + kScalDxMax, batch_bound_bits(mr, dp));
   }
 }
 
-int launch_prepare_latents(const void* x, int x_dtype, int64_t rows, int64_t rows_per_head, int d, int dp,
-                           const float* chdr, __half* xb, float* xinv, float* xn2, __half* xaug, uint32_t* scal,
-                           cudaStream_t st) {
+int launch_prepare_latents(const void* x, int x_dtype, int64_t rows, int64_t rows_per_head, int d,
+                           const LatentOperand& op, cudaStream_t st) {
   if (rows_per_head < 1) rows_per_head = 1;
+  const int dp = op.dp;
+  const float* chdr = op.chdr;
+  __half *xb = op.xb, *xaug = op.xaug;
+  float *xinv = op.xinv, *xn2 = op.xn2;
+  uint32_t* scal = op.scal;
   VQB_REQUIRE(dp <= 512, VQB_ERR_UNSUPPORTED, "prepare_latents: d_pad %d > 512", dp);
   const int warps = 8;
   int64_t blocks = (rows + warps - 1) / warps;
-  static int sms = 0;
-  if (!sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
-  }
+  const int sms = num_sms();
   if (blocks > (int64_t)sms * 8) blocks = (int64_t)sms * 8;     // persistent: rows strided over the grid
   if (blocks < 1) blocks = 1;
   if ((d & 7) == 0 && dp <= 128 && rows < (1ll << 32)) {
@@ -410,21 +401,11 @@ int launch_prepare_latents(const void* x, int x_dtype, int64_t rows, int64_t row
                                                                                 rows_per_head >= rows, d, dp, chdr,
                                                                                 xb, xinv, xn2, xaug, scal));
   } else if ((d & 7) == 0 && d <= 256 && (rows_per_head >= rows || (rows_per_head % 8 == 0 && rows < (1ll << 32)))) {
-    static int minb = -1;     // env VQB_PREP_MINB: resident blocks per SM the kernel is compiled for (register cap)
-    if (minb < 0) { const char* e = getenv("VQB_PREP_MINB"); minb = e ? atoi(e) : 3; }
-    const int64_t want = (rows + warps - 1) / warps, cap = (int64_t)sms * 4 * (minb >= 4 ? 4 : (minb == 3 ? 3 : 2));
+    const int64_t want = (rows + warps - 1) / warps, cap = (int64_t)sms * 4 * 3;
     blocks = want < cap ? want : cap;      // persistent: as many blocks as fit at this register cap
     if (blocks < 1) blocks = 1;
-    if (minb >= 4) {
-      VQB_DISPATCH_DTYPE(x_dtype, T, (prepare_latents4_kernel<T, 4><<<(unsigned)blocks, warps * 32, 0, st>>>(
-          (const T*)x, rows, rows_per_head, rows_per_head >= rows, d, dp, chdr, xb, xinv, xn2, xaug, scal)));
-    } else if (minb == 3) {
-      VQB_DISPATCH_DTYPE(x_dtype, T, (prepare_latents4_kernel<T, 3><<<(unsigned)blocks, warps * 32, 0, st>>>(
-          (const T*)x, rows, rows_per_head, rows_per_head >= rows, d, dp, chdr, xb, xinv, xn2, xaug, scal)));
-    } else {
-      VQB_DISPATCH_DTYPE(x_dtype, T, (prepare_latents4_kernel<T, 2><<<(unsigned)blocks, warps * 32, 0, st>>>(
-          (const T*)x, rows, rows_per_head, rows_per_head >= rows, d, dp, chdr, xb, xinv, xn2, xaug, scal)));
-    }
+    VQB_DISPATCH_DTYPE(x_dtype, T, (prepare_latents4_kernel<T><<<(unsigned)blocks, warps * 32, 0, st>>>(
+        (const T*)x, rows, rows_per_head, rows_per_head >= rows, d, dp, chdr, xb, xinv, xn2, xaug, scal)));
   } else {
     VQB_DISPATCH_DTYPE(x_dtype, T,
       prepare_latents_kernel<T><<<(unsigned)blocks, warps * 32, 0, st>>>((const T*)x, rows, rows_per_head, d, dp, chdr,
@@ -434,7 +415,7 @@ int launch_prepare_latents(const void* x, int x_dtype, int64_t rows, int64_t row
   return VQB_OK;
 }
 
-// Strided sample of the rows: scal[0] = kSampleGuard * max |x_row| over the sample (in-kernel conversion, search_tc.cu).
+// Strided sample of the rows: scal[kScalXMax] = kSampleGuard * max |x_row| over the sample (in-kernel conversion, search_tc.cu).
 // One warp per sampled row, d % 8 == 0, d <= 256.
 template <typename T>
 __global__ void __launch_bounds__(256)
@@ -459,7 +440,7 @@ sample_bound_kernel(const T* __restrict__ x, int64_t rows, int64_t stride, int64
   if (threadIdx.x == 0) {
     float mn = 0.f;
     for (int k = 0; k < 8; ++k) mn = fmaxf(mn, s_n[k]);
-    if (mn > 0.f && mn < 3.0e38f) atomicMax(scal + 0, __float_as_uint(sqrtf(mn) * kSampleGuard));
+    if (mn > 0.f && mn < 3.0e38f) atomicMax(scal + kScalXMax, __float_as_uint(sqrtf(mn) * kSampleGuard));
   }
 }
 
@@ -490,9 +471,9 @@ __global__ void make_bias_kernel(const float* __restrict__ cn2h, const float* __
       bias[i] = kPadBias;
       err[i] = 0.f;
     } else {
-      const float xmax = __uint_as_float(scal[0]);
+      const float xmax = __uint_as_float(scal[kScalXMax]);
       const float dxmax = derive_dx_dp > 0 ? dx_bound_16bit(xmax, derive_dx_dp, hdr[(i / Kp) * kHdrFloats + 5])
-                                           : __uint_as_float(scal[1]);
+                                           : __uint_as_float(scal[kScalDxMax]);
       const float c = cn[i], h = cn2h[i];
       // products are exact in the tensor core (fp16 x fp16 = 22 bits, fits fp32); accumulation is fp32-ish:
       // allow 2^-16 of the largest possible |sum| plus the fp32 rounding of |c|^2/2.
@@ -504,15 +485,15 @@ __global__ void make_bias_kernel(const float* __restrict__ cn2h, const float* __
       bias[i] = h - e;
     }
   }
-  // scal[6] = max_k E_k: the search epilogue's skip test needs a bound that holds for whichever code wins
+  // scal[kScalEmax] = max_k E_k: the search epilogue's skip test needs a bound that holds for whichever code wins
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) e = fmaxf(e, __shfl_xor_sync(0xffffffffu, e, o));
-  if ((threadIdx.x & 31) == 0 && e > 0.f) atomicMax(scal + 6, __float_as_uint(e));
+  if ((threadIdx.x & 31) == 0 && e > 0.f) atomicMax(scal + kScalEmax, __float_as_uint(e));
 }
 
 // Bias operand of the codebook for this search: three fp16 pieces (33 bits) of b_k = s_c 2^q bias_k, +inf for padded
 // codes (they can never become candidates).  bias_k = |c_k|^2/2 - E_k (keys pre-lowered, window L_min + 2 E_j) whenever
-// every b_k is an fp16 number; otherwise (E_k far above max |c|^2/2) bias_k = |c_k|^2/2 and scal[8] = 1 tells resolve
+// every b_k is an fp16 number; otherwise (E_k far above max |c|^2/2) bias_k = |c_k|^2/2 and scal[kScalUnlowered] = 1 tells resolve
 // to use the symmetric window min + 2 Emax.
 __global__ void make_bias_operand_kernel(const float* __restrict__ cn2h, const float* __restrict__ err,
                                          const float* __restrict__ hdr, int64_t total, int Kp, int K,
@@ -522,11 +503,11 @@ __global__ void make_bias_operand_kernel(const float* __restrict__ cn2h, const f
   const int64_t h = i / Kp;
   const int k = (int)(i - h * Kp);
   const float* hd = hdr + h * kHdrFloats;
-  const float emax = __uint_as_float(scal[6]);
+  const float emax = __uint_as_float(scal[kScalEmax]);
   const float scq = hd[0] * hd[4];                       // s_c 2^q (power of two)
   // per codebook; one head falling back switches resolve to the (always valid, wider) 2 Emax window for all heads
   const bool lowered = (hd[3] + emax) * scq < 60000.f;
-  if (k == 0 && !lowered) scal[8] = 1u;
+  if (k == 0 && !lowered) scal[kScalUnlowered] = 1u;
   __half p[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) p[j] = __float2half(0.f);
@@ -676,10 +657,9 @@ l2norm_prepare_kernel(const T* __restrict__ x, float* __restrict__ out, int64_t 
   if (threadIdx.x == 0) {
     float mn = 0.f, mr = 0.f;
     for (int i = 0; i < wpb; ++i) { mn = fmaxf(mn, s_n[i]); mr = fmaxf(mr, s_r[i]); }
-    const float infl = 1.f + (float)dp * 2.4e-7f;
-    atomicMax(scal + 0, __float_as_uint(sqrtf(mn * infl) * 1.00001f));
-    atomicMax(scal + 1, __float_as_uint(sqrtf(mr * infl) * 1.00001f));
-    if (blockIdx.x == 0 && chdr && single_head) scal[7] = __float_as_uint(chdr[4]);   // the 2^q these operands use
+    atomicMax(scal + kScalXMax, batch_bound_bits(mn, dp));
+    atomicMax(scal + kScalDxMax, batch_bound_bits(mr, dp));
+    if (blockIdx.x == 0 && chdr && single_head) scal[kScalTwoQ] = __float_as_uint(chdr[4]);   // the 2^q these operands use
   }
 }
 
@@ -729,24 +709,15 @@ extern "C" int vqb_l2norm_prepare(const void* x, int x_dtype, float* out, int64_
   VQB_REQUIRE(ws_bytes >= SL.total, VQB_ERR_WORKSPACE, "search workspace too small: %zu < %zu", ws_bytes, SL.total);
   if (N == 0) return VQB_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  char* w = (char*)search_ws;
-  uint32_t* scal = (uint32_t*)(w + SL.off_scal);
-  VQB_CUDA_TRY(cudaMemsetAsync(scal, 0, 32, st));      // [0..1] statistics, [7] is written below (H = 1) or stays 0
-  const float* chdr = (const float*)((const char*)cache + cache_layout(H, K, d).off_hdr);
+  const LatentOperand op = latent_operand(search_ws, H, N, K, d, cache);
+  // the batch bounds, and scal[kScalTwoQ]: written below when H = 1, else it stays 0
+  VQB_CUDA_TRY(cudaMemsetAsync(op.scal, 0, (kScalTwoQ + 1) * 4, st));
   const int64_t rows = H * N;
-  static int sms = 0;
-  if (!sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
-  }
   int64_t blocks = (rows + 7) / 8;
-  if (blocks > (int64_t)sms * 8) blocks = (int64_t)sms * 8;
+  if (blocks > (int64_t)num_sms() * 8) blocks = (int64_t)num_sms() * 8;
   VQB_DISPATCH_DTYPE(x_dtype, T,
-    l2norm_prepare_kernel<T><<<(unsigned)blocks, 256, 0, st>>>((const T*)x, out, rows, N, H == 1, d, SL.dp, chdr,
-                                                               (__half*)(w + SL.off_xb), (float*)(w + SL.off_xinv),
-                                                               (float*)(w + SL.off_xn2), (__half*)(w + SL.off_xaug), scal));
+    l2norm_prepare_kernel<T><<<(unsigned)blocks, 256, 0, st>>>((const T*)x, out, rows, N, H == 1, d, op.dp, op.chdr,
+                                                               op.xb, op.xinv, op.xn2, op.xaug, op.scal));
   VQB_LAUNCH_CHECK();
   return VQB_OK;
 }

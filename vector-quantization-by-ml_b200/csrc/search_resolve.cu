@@ -171,10 +171,10 @@ resolve_classify_kernel(const uint2* __restrict__ cand, const float* __restrict_
   if (gid < H * N) {
     const int64_t h = gid / N;
     RowCands R;
-    load_cands(cand, gid, K, Kp, h, err, (aug == 2 || scal[8]) ? __uint_as_float(scal[6]) : 0.f, tie * xn2[gid], R);
+    load_cands(cand, gid, K, Kp, h, err, (aug == 2 || scal[kScalUnlowered]) ? __uint_as_float(scal[kScalEmax]) : 0.f, tie * xn2[gid], R);
     // no fp16 bias operand for this row (prepare.cu), or operands prepared by vqb_rvq_level against a cache that
-    // has been rebuilt with another 2^q since (scal[7] records the one used): rescan exactly
-    if (aug && (xinv[gid] < 0.f || (scal[7] != 0u && scal[7] != __float_as_uint(chdr[h * kHdrFloats + 4]))))
+    // has been rebuilt with another 2^q since (scal[kScalTwoQ] records the one used): rescan exactly
+    if (aug && (xinv[gid] < 0.f || (scal[kScalTwoQ] != 0u && scal[kScalTwoQ] != __float_as_uint(chdr[h * kHdrFloats + 4]))))
       R.full_rescan = true;
     if (R.full_rescan) {
       const uint32_t pos = atomicAdd(flag_cnt + h, 1u);
@@ -236,12 +236,12 @@ resolve_classify_kernel(const uint2* __restrict__ cand, const float* __restrict_
     if (direct_code >= 0)
       score_out[gid] = metric == VQB_DOT ? (float)(-dot) : sqrtf(fmaxf((float)(n2 + cn2 - 2.0 * dot), 0.f));
   }
-  // warp-aggregated append to the re-rank list (scal[3] is its length)
+  // warp-aggregated append to the re-rank list (scal[kScalReranked] is its length)
   const uint32_t m = __ballot_sync(0xffffffffu, queue);
   if (m) {
     const int lane = threadIdx.x & 31;
     uint32_t base = 0;
-    if (lane == __ffs(m) - 1) base = atomicAdd(scal + 3, (uint32_t)__popc(m));
+    if (lane == __ffs(m) - 1) base = atomicAdd(scal + kScalReranked, (uint32_t)__popc(m));
     base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
     if (queue) rr_list[base + __popc(m & ((1u << lane) - 1u))] = (int)gid;
   }
@@ -265,7 +265,7 @@ rerank_emit_kernel(const uint2* __restrict__ cand, const float* __restrict__ err
                    const float* __restrict__ xn2, float tie) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
-  const int64_t count = scal[3];
+  const int64_t count = scal[kScalReranked];
   // the pair slots of the 8 rows a block handles per iteration are reserved with ONE atomic (a row at a time, 250 k
   // queued rows of a d = 64 search serialised on that one counter for 0.24 ms)
   __shared__ uint32_t s_n[8], s_base;
@@ -289,7 +289,7 @@ rerank_emit_kernel(const uint2* __restrict__ cand, const float* __restrict__ err
       const int oc = __shfl_xor_sync(0xffffffffu, c1, o);
       if (om < m1 || (om == m1 && oc > c1)) { m1 = om; c1 = oc; }   // any consistent tie rule: only E(c1) is used
     }
-    const float E1 = (aug == 2 || scal[8]) ? __uint_as_float(scal[6]) : (c1 >= 0 ? err[h * Kp + c1] : 0.f);
+    const float E1 = (aug == 2 || scal[kScalUnlowered]) ? __uint_as_float(scal[kScalEmax]) : (c1 >= 0 ? err[h * Kp + c1] : 0.f);
     const float thr = m1 + 2.f * E1 + (fabsf(m1) + E1) * kPackSlack + tie * xn2[gid];
     const bool act = code >= 0 && key <= thr;
     // hazard (ii): entries 3g and 3g+1 both within thr and from the same pair of N tiles -> that 64-column group
@@ -305,7 +305,7 @@ rerank_emit_kernel(const uint2* __restrict__ cand, const float* __restrict__ err
     if (threadIdx.x == 0) {
       uint32_t t = 0;
       for (int w2 = 0; w2 < (int)(blockDim.x >> 5); ++w2) t += s_n[w2];
-      s_base = t ? atomicAdd(scal + 9, t) : 0u;
+      s_base = t ? atomicAdd(scal + kScalPairs, t) : 0u;
     }
     __syncthreads();
     uint32_t base = s_base;
@@ -350,11 +350,11 @@ __global__ void flag_plan_kernel(const uint32_t* __restrict__ flag_cnt, int H, i
   plan[h] = 0xffffffffu;
   if (n == 0 || (uint64_t)n * (uint64_t)K > kFlagPairBudget) return;
   const uint32_t need = n * (uint32_t)K;
-  const uint32_t base = atomicAdd(scal + 9, need);
+  const uint32_t base = atomicAdd(scal + kScalPairs, need);
   if ((uint64_t)base + need > pair_cap) return;     // (the over-reservation is clamped away by pair_score_kernel)
   plan[h] = base;
   scan_cnt[h] = 0;
-  atomicAdd(scal + 2, n);                           // statistics: rows resolved by a scan of every code
+  atomicAdd(scal + kScalRescanned, n);                           // statistics: rows resolved by a scan of every code
 }
 __global__ void __launch_bounds__(256)
 flag_emit_kernel(const int* __restrict__ flag_list, const uint32_t* __restrict__ flag_cnt,
@@ -374,7 +374,7 @@ __global__ void __launch_bounds__(256)
 pair_score_kernel(const T* __restrict__ x, const float* __restrict__ cb, const uint2* __restrict__ pairs,
                   const uint32_t* __restrict__ scal, uint32_t pair_cap, int64_t total_rows, int64_t N, int K, int d,
                   int metric, unsigned long long* __restrict__ keys) {
-  uint32_t count = scal[9];
+  uint32_t count = scal[kScalPairs];
   if (count > pair_cap) count = pair_cap;      // over-reserved by rows that were diverted to the rescan
   for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < count; p += gridDim.x * blockDim.x) {
     const uint2 pr = pairs[p];
@@ -392,7 +392,7 @@ pair_score_kernel(const T* __restrict__ x, const float* __restrict__ cb, const u
 __global__ void rerank_finalize_kernel(const int* __restrict__ rr_list, const uint32_t* __restrict__ scal,
                                        const unsigned long long* __restrict__ keys, int64_t idx_offset,
                                        int64_t* __restrict__ idx_out, float* __restrict__ score_out) {
-  const int64_t count = scal[3];
+  const int64_t count = scal[kScalReranked];
   for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < count; p += (int64_t)gridDim.x * blockDim.x) {
     const int64_t gid = rr_list[p];
     const unsigned long long key = keys[gid];
@@ -436,7 +436,7 @@ exact_scan_kernel(const T* __restrict__ x, const float* __restrict__ cb, const i
   const T* xh = x + (int64_t)h * N * d;
   const float* cbh = cb + (int64_t)h * K * d;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;   // codes tx+16j (j<4), rows ty+16i (i<2)
-  if (flag_list && blockIdx.x == 0 && blockIdx.z == 0 && threadIdx.x == 0 && count) atomicAdd(scal + 2, (uint32_t)count);
+  if (flag_list && blockIdx.x == 0 && blockIdx.z == 0 && threadIdx.x == 0 && count) atomicAdd(scal + kScalRescanned, (uint32_t)count);
   const int kbeg = kSplit ? (int)blockIdx.z * ksplit_codes : 0;
   const int kend = kSplit ? (kbeg + ksplit_codes < K ? kbeg + ksplit_codes : K) : K;
   if (kbeg >= kend) return;
@@ -531,9 +531,9 @@ __global__ void rescan_finalize_kernel(const int* __restrict__ flag_list, const 
   }
 }
 
-// In-kernel conversion: scal[0] bounds only the rows within the sampled bound; the search kernel gave the others a
-// negative xinv (they are rescanned exactly).  Their norm bound xn2 (>= |x|^2) goes into scal[1], which nothing reads on
-// this route once make_bias has run, so that scal[0] + scal[1] >= max|x_j| over the batch, as the EMA kernels read it
+// In-kernel conversion: scal[kScalXMax] bounds only the rows within the sampled bound; the search kernel gave the others a
+// negative xinv (they are rescanned exactly).  Their norm bound xn2 (>= |x|^2) goes into scal[kScalDxMax], which nothing reads on
+// this route once make_bias has run, so that scal[kScalXMax] + scal[kScalDxMax] >= max|x_j| over the batch, as the EMA kernels read it
 // (vqb.h, vqb_ema_reduce).
 __global__ void __launch_bounds__(256)
 conv_outlier_bound_kernel(const float* __restrict__ xinv, const float* __restrict__ xn2, int64_t rows,
@@ -542,18 +542,7 @@ conv_outlier_bound_kernel(const float* __restrict__ xinv, const float* __restric
   for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (int64_t)gridDim.x * blockDim.x)
     if (xinv[r] < 0.f) m = fmaxf(m, sqrtf(xn2[r]));
   m = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m)));   // non-negative: bit order = float order
-  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(scal + 1, __float_as_uint(m));
-}
-
-static int g_num_sms = 0;
-static int num_sms() {
-  if (!g_num_sms) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-    if (g_num_sms <= 0) g_num_sms = 148;
-  }
-  return g_num_sms;
+  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(scal + kScalDxMax, __float_as_uint(m));
 }
 
 }  // namespace vqb
@@ -586,18 +575,21 @@ extern "C" int vqb_search(const void* x, int x_dtype, const float* codebook, con
   int* flag_list = (int*)(w + SL.off_flag);
   const bool prepared = (flags & VQB_SEARCH_LATENTS_PREPARED) != 0;
   const bool tc = !(flags & VQB_SEARCH_FORCE_EXACT) && SL.dp <= 512 && cache != nullptr;
-  // scal[0..1] hold the row statistics: keep them when the caller prepared the latents
-  if (prepared) {   // keep [0..1] (row statistics) and [7] (2^q of the prepared bias operands)
-    VQB_CUDA_TRY(cudaMemsetAsync((char*)scal + 8, 0, 20, st));
-    VQB_CUDA_TRY(cudaMemsetAsync((char*)scal + 32, 0, (SL.off_cnt - SL.off_scal) + (size_t)H * 12 - 32, st));
+  // keep the batch bounds and the 2^q of latents the caller prepared: zero the slots between and after them
+  if (prepared) {
+    static_assert(kScalXMax == 0 && kScalDxMax == 1 && kScalTwoQ == 7, "slots kept for prepared latents");
+    VQB_CUDA_TRY(cudaMemsetAsync(scal + kScalDxMax + 1, 0, (kScalTwoQ - kScalDxMax - 1) * 4, st));
+    VQB_CUDA_TRY(cudaMemsetAsync(scal + kScalTwoQ + 1, 0,
+                                 (SL.off_cnt - SL.off_scal) + (size_t)H * 12 - (kScalTwoQ + 1) * 4, st));
   } else {
     VQB_CUDA_TRY(cudaMemsetAsync((char*)scal, 0, (SL.off_cnt - SL.off_scal) + (size_t)H * 12, st));
   }
 
   const int grid_scan = (int)((N + kER - 1) / kER < 4 * (int64_t)num_sms() ? (N + kER - 1) / kER : 4 * num_sms());
   if (!tc) {
-    // nothing on this route writes the row statistics: scal[0] = max|x_j| for the EMA kernels (vqb.h, vqb_ema_reduce)
-    if (int rc = launch_absmax(x, x_dtype, H * N * (int64_t)d, scal, st)) return rc;
+    // nothing on this route writes the row statistics: scal[kScalXMax] = max|x_j| for the EMA kernels (vqb.h,
+    // vqb_ema_reduce)
+    if (int rc = launch_absmax(x, x_dtype, H * N * (int64_t)d, scal + kScalXMax, st)) return rc;
     VQB_DISPATCH_DTYPE(x_dtype, T,
       exact_scan_kernel<T, false><<<dim3((unsigned)grid_scan, (unsigned)H), 256, 0, st>>>(
           (const T*)x, codebook, nullptr, nullptr, N, K, d, metric, idx_offset, idx_out, score_out, scal, 0, nullptr));
@@ -607,23 +599,19 @@ extern "C" int vqb_search(const void* x, int x_dtype, const float* codebook, con
 
   CacheLayout CL = cache_layout(H, K, d);
   const char* cbase = (const char*)cache;
-  __half* xb = (__half*)(w + SL.off_xb);
-  float* xinv = (float*)(w + SL.off_xinv);
-  float* xn2 = (float*)(w + SL.off_xn2);
+  const LatentOperand op = latent_operand(ws, H, N, K, d, cache);
   const float tie = metric == VQB_EUCLID ? kTieSlack : 0.f;
   unsigned long long* keys = (unsigned long long*)(w + SL.off_keys);
   float* bias = (float*)(w + SL.off_bias);
   float* err = (float*)(w + SL.off_err);
   int rc;
-  __half* xaug = (__half*)(w + SL.off_xaug);
-  const float* chdr = (const float*)(cbase + CL.off_hdr);
   const int aug = search_tc_aug_mode(N, K, metric);
   // 16-bit latents and enough tensor work per row tile: the search kernel converts the rows itself, overlapped with
   // its MMAs (search_tc.cu, CONV); all that runs ahead of it is a strided sample that bounds the row norms
   ConvArgs conv;
   const int conv_mode = prepared ? 0 : search_tc_conv_ok(N, K, d, x_dtype, aug, (flags & VQB_SEARCH_FUSED_PREP) != 0);
   if (conv_mode == 2) {
-    rc = launch_prepare_latents(x, x_dtype, H * N, N, d, SL.dp, chdr, xb, xinv, xn2, xaug, scal, st);
+    rc = launch_prepare_latents(x, x_dtype, H * N, N, d, op, st);
     if (rc) return rc;
     conv.x = x; conv.x_dtype = -1; conv.d = d;
   } else if (conv_mode == 1) {
@@ -631,19 +619,19 @@ extern "C" int vqb_search(const void* x, int x_dtype, const float* codebook, con
     rc = launch_sample_bound(x, x_dtype, H * N, d, scal, st);
     if (rc) return rc;
   } else if (!prepared) {
-    rc = launch_prepare_latents(x, x_dtype, H * N, N, d, SL.dp, chdr, xb, xinv, xn2, xaug, scal, st);
+    rc = launch_prepare_latents(x, x_dtype, H * N, N, d, op, st);
     if (rc) return rc;
   }
   __half* caug = (__half*)(w + SL.off_caug);
   rc = launch_make_bias(cache, CL, H, K, metric, scal, bias, err, aug == 1 ? caug : nullptr, st, conv_mode == 1 ? SL.dp : 0);
   if (rc) return rc;
-  rc = launch_search_tc(xb, xinv, xn2, tie, xaug, (const __half*)(cbase + CL.off_cb), caug, chdr,
+  rc = launch_search_tc(op.xb, op.xinv, op.xn2, tie, op.xaug, (const __half*)(cbase + CL.off_cb), caug, op.chdr,
                         bias, aug, H, N, K, SL.dp, w + SL.off_cand, scal, (flags & VQB_SEARCH_TIMING) != 0, st, conv);
   if (rc) return rc;
   const int64_t total = H * N;
   if (conv_mode == 1) {
     const int64_t want = (total + 255) / 256, cap = 4 * (int64_t)num_sms();
-    conv_outlier_bound_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(xinv, xn2, total, scal);
+    conv_outlier_bound_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, st>>>(op.xinv, op.xn2, total, scal);
     VQB_LAUNCH_CHECK();
   }
   int* rr_list = (int*)(w + SL.off_rr);
@@ -651,11 +639,11 @@ extern "C" int vqb_search(const void* x, int x_dtype, const float* codebook, con
     VQB_DISPATCH_DTYPE(x_dtype, T,
       (resolve_classify_kernel<T, true><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(
           (const uint2*)(w + SL.off_cand), err, H, N, K, CL.Kp, idx_offset, idx_out, rr_list, flag_list, cnt, keys, scal,
-          xinv, chdr, aug, xn2, tie, (const T*)x, codebook, d, metric, score_out)));
+          op.xinv, op.chdr, aug, op.xn2, tie, (const T*)x, codebook, d, metric, score_out)));
   } else {
     resolve_classify_kernel<float, false><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(
         (const uint2*)(w + SL.off_cand), err, H, N, K, CL.Kp, idx_offset, idx_out, rr_list, flag_list, cnt, keys, scal,
-        xinv, chdr, aug, xn2, tie, nullptr, codebook, d, metric, nullptr);
+        op.xinv, op.chdr, aug, op.xn2, tie, nullptr, codebook, d, metric, nullptr);
   }
   VQB_LAUNCH_CHECK();
   {
@@ -665,7 +653,7 @@ extern "C" int vqb_search(const void* x, int x_dtype, const float* codebook, con
     const int64_t cap = (int64_t)num_sms() * 8;
     const int grid_rr = (int)(want < cap ? want : cap);
     rerank_emit_kernel<<<grid_rr, 256, 0, st>>>((const uint2*)(w + SL.off_cand), err, N, K, CL.Kp, rr_list, scal, aug,
-                                                pairs, pair_cap, flag_list, cnt, xn2, tie);
+                                                pairs, pair_cap, flag_list, cnt, op.xn2, tie);
     VQB_LAUNCH_CHECK();
     flag_plan_kernel<<<(unsigned)((H + 63) / 64), 64, 0, st>>>(cnt, (int)H, K, pair_cap, scal, scan_cnt, plan);
     VQB_LAUNCH_CHECK();
@@ -703,9 +691,9 @@ extern "C" int vqb_search_stats(const void* ws, int64_t* host_out3, void* stream
   uint32_t hbuf[8];
   VQB_CUDA_TRY(cudaMemcpyAsync(hbuf, ws, sizeof(hbuf), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
   VQB_CUDA_TRY(cudaStreamSynchronize((cudaStream_t)stream));
-  host_out3[0] = hbuf[3];
-  host_out3[1] = hbuf[2];
-  host_out3[2] = hbuf[4];
-  if (hbuf[5]) { set_error("search_tc: dynamic shared memory base was not 1024B aligned"); return VQB_ERR_CUDA; }
+  host_out3[0] = hbuf[kScalReranked];
+  host_out3[1] = hbuf[kScalRescanned];
+  host_out3[2] = hbuf[kScalTcUsed];
+  if (hbuf[kScalMisaligned]) { set_error("search_tc: dynamic shared memory base was not 1024B aligned"); return VQB_ERR_CUDA; }
   return VQB_OK;
 }

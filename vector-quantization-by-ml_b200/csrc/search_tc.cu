@@ -351,9 +351,9 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
   const int G = P.H * P.MT;                    // (codebook, row tile) work items
 
   if (threadIdx.x == 0 && (smem_base & 1023u)) {   // the swizzle pattern assumes 1024B-aligned tiles
-    atomicExch(P.scal + 5, 1u);
+    atomicExch(P.scal + kScalMisaligned, 1u);
   }
-  if (blockIdx.x == 0 && threadIdx.x == 0) P.scal[4] = 1u;   // "tensor-core pass ran" marker for vqb_search_stats
+  if (blockIdx.x == 0 && threadIdx.x == 0) P.scal[kScalTcUsed] = 1u;   // "tensor-core pass ran" marker for vqb_search_stats
   if (warp == kWarpTma && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_x) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_c) : "memory");
@@ -488,7 +488,7 @@ search_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
     const float INF = __int_as_float(0x7f800000);
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16) + quarter * 64;
     // Emax * (2 + slack): the part of the candidate threshold that does not depend on the row minimum
-    const float tconst = __uint_as_float(P.scal[6]) * (2.f + kPackSlackTC);
+    const float tconst = __uint_as_float(P.scal[kScalEmax]) * (2.f + kPackSlackTC);
     uint32_t r[16];
     uint32_t tile_it = 0;                           // row tiles processed by this CTA so far
     if (cta < G) {   // pipeline prologue: first chunk of the very first tile (later ones are prefetched in the loop)
@@ -656,7 +656,7 @@ struct AugBarriers {
 
 // One warp converts rows [r0, r1) of codebook `h` exactly as prepare_latents4_kernel does for 16-bit latents (same
 // scale, same fp16 values, same bounds), 8 rows in flight.  A row whose statistics exceed the bounds the bias
-// operand was built with (scal[0] from the strided sample, the residual bound derived from it) gets a NEGATIVE xinv:
+// operand was built with (scal[kScalXMax] from the strided sample, the residual bound derived from it) gets a NEGATIVE xinv:
 // resolve rescans it exactly.
 template <typename T>
 __device__ __forceinline__ void convert_rows16(const T* __restrict__ x, int64_t base, int64_t r0, int64_t r1, int d,
@@ -761,8 +761,8 @@ search_aug_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_consta
   const int G = P.H * P.GPH;
   const bool aug = P.aug != 0;
 
-  if (threadIdx.x == 0 && (smem_base & 1023u)) atomicExch(P.scal + 5, 1u);
-  if (blockIdx.x == 0 && threadIdx.x == 0) P.scal[4] = 1u;
+  if (threadIdx.x == 0 && (smem_base & 1023u)) atomicExch(P.scal + kScalMisaligned, 1u);
+  if (blockIdx.x == 0 && threadIdx.x == 0) P.scal[kScalTcUsed] = 1u;
   if (warp == kWarpTma && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_x) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_c) : "memory");
@@ -938,7 +938,7 @@ search_aug_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_consta
     // ahead of the producer: the fp16 rows are still in L2 when the TMA load comes for them.  The tensor pipe is the
     // bound of this kernel and HBM nearly idle, so the conversion pass costs nothing on the step's critical path.
     const int cw = warp - 18;
-    const float x0 = __uint_as_float(P.scal[0]);
+    const float x0 = __uint_as_float(P.scal[kScalXMax]);
     const float x0sq = x0 * x0 * 0.99999f;
     uint32_t c_it = 0;
     for (int g = cid; g < G; g += num_clusters, ++c_it) {
@@ -983,7 +983,7 @@ search_aug_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_consta
     uint32_t acc = 0, acc_ph = 0;
     const float INF = __int_as_float(0x7f800000);
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16) + quarter * 64;
-    const float tconst = __uint_as_float(P.scal[6]) * (2.f + kPackSlackTC);
+    const float tconst = __uint_as_float(P.scal[kScalEmax]) * (2.f + kPackSlackTC);
     uint32_t rD[4][16];                      // the whole 64-column quarter
     uint32_t tile_it = 0;
     for (int g = cid; g < G; g += num_clusters) {
@@ -1141,7 +1141,6 @@ static cudaEvent_t g_ev0[kTimingSlots], g_ev1[kTimingSlots];
 static bool g_ev_made = false;
 static int g_ev_dev = -1;              // the events belong to the device of the first timed search
 static int g_ev_count = 0;
-static int g_num_sms = 0;              // SMs of the device of the first search: one CTA per SM
 
 // Launches a persistent search kernel: clusters of `cluster` CTAs, one CTA per SM but no more clusters than the G
 // work items, 227 KB of dynamic shared memory allowed; `timing` brackets the launch with an event pair of the ring.
@@ -1155,8 +1154,7 @@ static int launch_search_kernel(int cluster, int G, int threads, size_t smem_byt
     VQB_CUDA_TRY(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     if (dev >= 0 && dev < 64) configured[dev] = true;
   }
-  if (!g_num_sms) VQB_CUDA_TRY(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
-  int nclusters = g_num_sms / cluster;
+  int nclusters = num_sms() / cluster;   // one CTA per SM
   if (nclusters > G) nclusters = G;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)(nclusters * cluster));
