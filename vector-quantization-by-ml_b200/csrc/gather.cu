@@ -656,7 +656,8 @@ extern "C" size_t vqb_gather_workspace_bytes(int64_t H, int64_t N, int d) {
 extern "C" int vqb_gather_st_loss(const void* x, int x_dtype, const float* codebook, const int64_t* idx,
                                   const uint8_t* mask, int training, int want_loss, float* q_out, float* loss_out,
                                   int64_t H, int64_t N, int K, int d, void* ws, size_t ws_bytes, void* stream) {
-  VQB_REQUIRE(x && codebook && idx && q_out, VQB_ERR_INVALID, "vqb_gather_st_loss: null pointer");
+  // an empty batch has no rows to read or write (torch hands out null data pointers for it); its loss is NaN, 0
+  VQB_REQUIRE(codebook && (H * N == 0 || (x && idx && q_out)), VQB_ERR_INVALID, "vqb_gather_st_loss: null pointer");
   VQB_REQUIRE(H > 0 && N >= 0 && K > 0 && d > 0, VQB_ERR_INVALID, "vqb_gather_st_loss: bad shape");
   GatherLayout L = gather_layout();
   if (want_loss) {
@@ -702,9 +703,9 @@ extern "C" int vqb_gather_st_loss(const void* x, int x_dtype, const float* codeb
 extern "C" int vqb_st_commit_backward(const float* grad_q, const float* grad_loss, const void* x, int x_dtype,
                                       const float* codebook, const int64_t* idx, const uint8_t* mask, float coef,
                                       float* grad_x, int64_t H, int64_t N, int K, int d, void* stream) {
+  if (H * N == 0) return VQB_OK;
   VQB_REQUIRE(grad_q && grad_loss && x && codebook && idx && grad_x, VQB_ERR_INVALID,
               "vqb_st_commit_backward: null pointer");
-  if (H * N == 0) return VQB_OK;
   const int grid = gather_grid(H * N);
   VQB_DISPATCH_DTYPE(x_dtype, T,
     st_commit_backward_kernel<T, false><<<grid, kGatherThreads, 0, (cudaStream_t)stream>>>(
@@ -716,9 +717,9 @@ extern "C" int vqb_st_commit_backward(const float* grad_q, const float* grad_los
 extern "C" int vqb_rot_commit_backward(const float* grad_q, const float* grad_loss, const void* x, int x_dtype,
                                        const float* codebook, const int64_t* idx, const uint8_t* mask, float coef,
                                        float* grad_x, int64_t H, int64_t N, int K, int d, void* stream) {
+  if (H * N == 0) return VQB_OK;
   VQB_REQUIRE(grad_q && grad_loss && x && codebook && idx && grad_x, VQB_ERR_INVALID,
               "vqb_rot_commit_backward: null pointer");
-  if (H * N == 0) return VQB_OK;
   const int grid = gather_grid(H * N);
   VQB_DISPATCH_DTYPE(x_dtype, T,
     st_commit_backward_kernel<T, true><<<grid, kGatherThreads, 0, (cudaStream_t)stream>>>(

@@ -132,6 +132,7 @@ def search_stats(ws: torch.Tensor) -> Dict[str, int]:
 @_on_device
 def l2norm_rows(x: torch.Tensor) -> torch.Tensor:
     L.require_cuda(x, "x")
+    x = L.aligned(x)     # the kernel reads 4 elements at a time (16-byte loads for fp32)
     d = x.shape[-1]
     out = torch.empty(x.shape, dtype=torch.float32, device=x.device)
     rows = x.numel() // d if d else 0
@@ -174,6 +175,7 @@ def l2norm_prepare(x: torch.Tensor, K: int, cache: torch.Tensor) -> torch.Tensor
     """x (H,N,d) -> x / |x| (fp32) and, in the shared search workspace, everything the next
     `search(out, ..., latents_prepared=True)` with this codebook cache needs."""
     L.require_cuda(x, "x")
+    x = L.aligned(x)
     H, N, d = x.shape
     out = torch.empty((H, N, d), dtype=torch.float32, device=x.device)
     ws = workspace("search", L.lib().vqb_search_workspace_bytes(H, N, K, d), x.device)
@@ -293,17 +295,23 @@ class _QuantizeST(torch.autograd.Function):
             grad_q = torch.zeros((H, N, d), dtype=torch.float32, device=x.device)
         grad_q = grad_q.contiguous().float()
         g_emb = None
+        # with no live rows (all masked, or N = 0) the loss is the mean of an empty selection: its gradient reaches no
+        # row and no code, so dividing by max(rows, 1) sends zeros where rows = 0 would make 0 * inf = NaN
+        rows = loss[1].clamp_min(1.0) if ctx.want_loss else None
         if ctx.needs_input_grad[1] and ctx.want_loss and grad_commit is not None:
             # learnable codebook: d mse(C[idx], x) / d C[k] = 2 (n_k C[k] - sum of the rows assigned to k) / (rows * d),
             # from the same deterministic segmented sums as the EMA statistics
-            st = ema_reduce(x, idx, mask_u8 if ctx.has_mask else None, K)
-            g_emb = (grad_commit.float() * (2.0 / d) / loss[1]) * (st[..., d:] * embeddings.detach() - st[..., :d])
+            if H * N == 0:
+                g_emb = torch.zeros_like(embeddings)
+            else:
+                st = ema_reduce(x, idx, mask_u8 if ctx.has_mask else None, K)
+                g_emb = (grad_commit.float() * (2.0 / d) / rows) * (st[..., d:] * embeddings.detach() - st[..., :d])
         none = (g_emb,) + (None,) * 6
         has_commit = ctx.want_loss and grad_commit is not None
         if not has_commit and not ctx.rotation:
             return (grad_q.to(x.dtype),) + none
         # device scalar: grad_commit * 2 / (rows_used * d)   (no host sync)
-        g = (grad_commit.float() * (2.0 / d) / loss[1]).reshape(1).contiguous() if has_commit \
+        g = (grad_commit.float() * (2.0 / d) / rows).reshape(1).contiguous() if has_commit \
             else torch.zeros(1, dtype=torch.float32, device=x.device)
         mask = mask_u8 if ctx.has_mask else None
         gx = (rot_commit_backward if ctx.rotation else st_commit_backward)(grad_q, g, x, embeddings, idx, mask)
