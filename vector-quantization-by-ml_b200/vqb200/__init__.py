@@ -11,7 +11,9 @@ replaces
 from .codebook import Codebook, CosineSimCodebook, EuclideanCodebook
 from .params import AffineParameters, CodebookParams, GumbelParams, KmeansParameters
 from .rvq import GroupedResidualVQ, ResidualVQ
+from .simvq import ResidualSimVQ, SimVQ
 from .vq import LossBreakdown, VectorQuantize
 
 __all__ = ["Codebook", "EuclideanCodebook", "CosineSimCodebook", "CodebookParams", "KmeansParameters", "GumbelParams",
-           "AffineParameters", "VectorQuantize", "LossBreakdown", "ResidualVQ", "GroupedResidualVQ"]
+           "AffineParameters", "VectorQuantize", "LossBreakdown", "ResidualVQ", "GroupedResidualVQ", "SimVQ",
+           "ResidualSimVQ"]
